@@ -5,6 +5,7 @@
     python bench.py --impl reference --gpus N --steps K ...    # CPU arm: the reference's step on the host cores
     python bench.py --impl reference-gpu --steps K ...         # the reference's OWN CUDA kernel + its 4 PCIe copies
     python bench.py --config c4 --gpus N --steps 1000          # BASELINE configs[3] as the first-class line
+    python bench.py --steps K --warmup W --dump-outputs DIR    # also write the last timed step's outputs as .npy
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...   # one rank per GPU (the driver does this)
 
 Default workload (BASELINE.json configs[1], SURVEY.md section 8d "C2"): 4096 envs x 128x128 per GPU, env mode --
@@ -52,6 +53,7 @@ BYTES_PER_CELL_LIFE = 0.25
 REPLICAS = 4                               # rotating env batches: 4 x 80 MiB touched round-robin > 126 MB L2
 E2E_GROUPS = 4                             # env groups of the host-driven rollout (measured: 1 -> 40.2, 2 -> 32.8, 4 -> 29.6, 8 -> 33 us per step)
 C4_SIDE, C4_GHOST, C4_KERNEL_K = 65536, 128, 8         # ghost depth measured at 8 GPUs: 64 -> 16.02, 96 -> 16.03, 128 -> 15.81 us per generation
+DUMP_ENVS, DUMP_SEED = 256, 0                          # --dump-outputs: 2 planes x 256 envs x 16384 cells x 4 B = 32 MiB
 
 
 def measured_peak_gbs():
@@ -313,9 +315,18 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="skip the C1/C3/C4/C5 and f-row side measurements")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-e2e", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned to its caller as float32 "
+                         f"DIR/<name>.npy (rank 0): reward [{ENVS_PER_GPU}] of the env batch it stepped, and obs "
+                         f"(int8 stability) and world (cells) [{DUMP_ENVS}, {SIDE * SIDE}] of a fixed sample of "
+                         f"{DUMP_ENVS} of its envs (RandomState({DUMP_SEED}), sorted); C2 GPU run only")
     args = ap.parse_args()
     if args.steps is None:
         args.steps = 1000 if args.config == "c4" else 200
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.config != "c2"):
+        ap.error("--dump-outputs is implemented for the C2 GPU run (--impl ours --config c2) only")
     if args.impl == "reference":
         return run_reference_arm(args)
     if args.impl == "reference-gpu":
@@ -361,6 +372,10 @@ def run_c2_line(c, args):
     issue = seq.prepare(K, events=events)
     issue(); issue()                                        # (both plane orientations of an odd K are cached now)
     dt_eager, regions_eager = repeat_regions(c, issue, args.repeats, events)
+    use_graph = args.launch == "graph"
+    outputs = None
+    if args.dump_outputs and rank == 0 and not use_graph:
+        outputs = last_step_outputs(sims[(K - 1) % R])      # before the L2-resident variant steps sims[0] again
 
     # L2-resident variant (one replica, 80 MiB working set inside the 126 MB L2) -- reported, not the headline
     seq1 = StepSequence(sims[:1], actions)
@@ -385,17 +400,22 @@ def run_c2_line(c, args):
     def issue_graph():
         for _ in range(K // cycle):
             graph.replay()
-        if K % cycle:
+        if K % cycle:               # every call starts at sims[0]: the rest twice steps each sim an even number of times,
+            gseq.run(K % cycle)     # so its planes are back in the captured position (the second call is part of the region)
             gseq.run(K % cycle)
-            gseq.run(cycle - K % cycle)                     # (planes back in the captured position; part of the region)
-    k_graph = K + (cycle - K % cycle if K % cycle else 0)
+    k_graph = K + K % cycle
     dt_graph, regions_graph = repeat_regions(c, issue_graph, min(args.repeats, 5))
     dt_graph = dt_graph * K / k_graph
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0 and use_graph:
+        outputs = last_step_outputs(gsims[(K - 1) % R])     # issue_graph() ends on the same sim as the eager path
+    if outputs is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in outputs.items():
+            np.save(os.path.join(args.dump_outputs, f"{name}.npy"), a)
     del gsims, gseq, graph
     torch.cuda.empty_cache()
 
-    use_graph = args.launch == "graph"
     dt = dt_graph if use_graph else dt_eager
     cells_per_step = B * size * world
     value = cells_per_step * K / dt / 1e9
@@ -441,6 +461,17 @@ def run_c2_line(c, args):
             ("graph_value" if not use_graph else "eager_value"):
                 cells_per_step * K / (dt_eager if use_graph else dt_graph) / 1e9,
             "extras": extras}
+
+
+def last_step_outputs(sim):
+    """What the last step of `sim` returned to its caller (BatchedSim.step: reward, obs) and the world it left, as
+    float32 host arrays; the two planes for a fixed sample of DUMP_ENVS envs (in full they are 2 x 256 MiB)."""
+    import torch
+    envs = np.sort(np.random.RandomState(DUMP_SEED).choice(sim.n_envs, DUMP_ENVS, replace=False))
+    idx = torch.from_numpy(envs).to(sim.device)
+    return {"reward": sim._reward.cpu().numpy().astype(np.float32),
+            "obs": sim.stable[idx].cpu().numpy().astype(np.float32),
+            "world": sim.get_state()[idx].cpu().numpy().astype(np.float32)}
 
 
 def measure_e2e(c, args, sims):
