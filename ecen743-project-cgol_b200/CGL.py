@@ -485,7 +485,7 @@ class sim:
 
     @property
     def _can_defer(self):
-        return self._bs.fused or self.side <= 273           # sides cgl_env_run can keep on chip
+        return self._bs.fused or self.side <= 274           # sides cgl_env_run can keep on chip
 
     # ---- extensions (not in CGL/CGL.py): the reference's own loops around step(), run on the device ----
     def run(self, iters, until_fixed=False):

@@ -409,7 +409,7 @@ env_run_sliced_kernel(const uint32_t *world_in, uint32_t *world_out, int8_t *sta
     }
 }
 
-// Any side whose three byte planes fit in shared memory (side <= 270): one CTA per env, one byte per cell.
+// Any side whose three byte planes fit in 220 KiB of shared memory (side <= 274): one CTA per env, one byte per cell.
 __global__ void __launch_bounds__(256)
 env_run_generic_kernel(const uint32_t *world_in, uint32_t *world_out, int8_t *stable, uint32_t side, uint32_t W,
                        uint32_t max_steps, int stop_when_fixed, int8_t spawn, int8_t stable_max,
@@ -571,7 +571,7 @@ extern "C" int cgl_env_run_rule(const uint32_t *win, uint32_t *wout, int8_t *sta
     }
     const size_t smem = 3ull * side * side;
     CGL_REQUIRE(smem <= 220 * 1024, CGL_E_BADARG,
-                "cgl_env_run: side must be a fused side or small enough for shared memory (side <= 273)");
+                "cgl_env_run: side must be a fused side or small enough for shared memory (side <= 274)");
     static PerDeviceOnce once;                   // opt in to the largest size once per device
     if (once.first())
         CGL_CUDA(cudaFuncSetAttribute(env_run_generic_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024));

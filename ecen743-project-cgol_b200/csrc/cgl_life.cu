@@ -254,6 +254,10 @@ extern "C" int cgl_life_step(const uint32_t *in, uint32_t *out, uint64_t n_envs,
         rows_knob = v ? atoi(v) : 0;
     }
     const uint32_t rpt = rows_knob > 0 ? (uint32_t)rows_knob : pick_rows_per_strip(n_envs, rows, n_cgroups);
+    // A strip reads rows r0 - 1 .. r0 + rpt and load_row_raw wraps a row index once: on a torus with 2 * rows <= rpt
+    // that would read past the env.  Such tiny tori take the generic kernel.
+    if (wrap_rows && 2ull * rows <= rpt)
+        return cgl_life_step_generic(in, out, n_envs, rows, cols, wrap_rows, alive_out, stream);
     const uint32_t n_rblocks = (rows + rpt - 1) / rpt;
     const uint64_t warps = n_envs * n_cgroups * n_rblocks;
     const uint64_t blocks = (warps + (LIFE_ROWS_THREADS / 32) - 1) / (LIFE_ROWS_THREADS / 32);

@@ -195,7 +195,7 @@ life_persist_kernel(uint32_t *buf_a, uint32_t *buf_b, uint32_t rows, uint32_t W,
             span = (uint32_t)(last - rstart - s_lo);
             out_rows = (uint32_t)(g.r1 - g.r0);
             ro0 = (uint32_t)g.r0;
-            rw = rstart < 0 ? rstart + irows : rstart;
+            rw = (rstart % irows + irows) % irows;   // in [0, rows) also when rows < K (see life_tb_kernel)
             ip = in + g.wcol;
             op = out + (g.store_lane ? (uint32_t)g.wi : 0u);
             store_ok = g.store_lane && alive;

@@ -141,7 +141,7 @@ life_tb_kernel(const uint32_t *__restrict__ in, uint32_t *__restrict__ out, uint
     const int r0 = (int)(rb * rpt);
     const int r1 = (r0 + (int)rpt < (int)rows) ? r0 + (int)rpt : (int)rows;
     const int irows = (int)rows;
-    const int rstart = r0 - K;                                  // first gen-0 row fed to level 1 (> -rows)
+    const int rstart = r0 - K;                                  // first gen-0 row fed to level 1 (>= -K)
     const int n_steps = (int)rpt + 3 * K - 1;                   // same trip count for every warp (uniform loop)
     // Step s loads gen-0 row rstart + s.  It is needed (and inside the grid, for open rows) iff
     // s_lo <= s < s_hi; rows from r1 + K on can no longer reach an output row of this strip.
@@ -149,7 +149,9 @@ life_tb_kernel(const uint32_t *__restrict__ in, uint32_t *__restrict__ out, uint
     const int last = (wrap_rows || r1 + K < irows) ? r1 + K : irows;
     const uint32_t span = (uint32_t)(last - rstart - s_lo);
     const uint32_t out_rows = (uint32_t)(r1 - r0);
-    int rw = rstart < 0 ? rstart + irows : rstart;              // row index modulo rows (only used where loads are on)
+    // Row index modulo rows, in [0, rows): the row loop wraps it with one subtraction per trip.  A true modulo,
+    // because a torus with fewer rows than K starts more than one lap above row 0.
+    int rw = (rstart % irows + irows) % irows;
     const uint32_t *ip = in + wcol;
     uint32_t *op = out + (store_ok ? (uint32_t)wi : 0u);
 
@@ -338,7 +340,7 @@ life_tb2_kernel(const uint32_t *__restrict__ in, uint32_t *__restrict__ out, uin
     const int last = (wrap_rows || r1 + K < irows) ? r1 + K : irows;
     const uint32_t span = (uint32_t)(last - rstart - s_lo);
     const uint32_t out_rows = (uint32_t)(r1 - r0);
-    int rw = rstart < 0 ? rstart + irows : rstart;
+    int rw = (rstart % irows + irows) % irows;                  // in [0, rows) also when rows < K (see life_tb_kernel)
     const uint32_t *ip = in + wcol;
     uint32_t *op = out + (store_ok ? (uint32_t)wi : 0u);
     const uint32_t r0W = (uint32_t)r0 * W;

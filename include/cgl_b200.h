@@ -189,7 +189,7 @@ int cgl_env_step_io(uint32_t *world_in_dev, uint32_t *world_out_dev, const int8_
  *   steps_out_dev  int32 [n_envs] or NULL: steps actually executed per env (== max_steps unless
  *                  stop_when_fixed ended the env early; the step that found the fixed point counts).
  *   reward_out_dev / alive_out_dev as in cgl_env_step (of the final state; valid for max_steps == 0 too).
- * Sides: the fused sides (multiples of 32 up to 256) and any side <= 273. */
+ * Sides: the fused sides (multiples of 32 up to 256) and any side <= 274. */
 int cgl_env_run(const uint32_t *world_in_dev, uint32_t *world_out_dev, int8_t *stable_dev, uint64_t n_envs,
                 uint32_t side, uint32_t max_steps, int stop_when_fixed, int spawn, int stable_max,
                 int32_t *steps_out_dev, int32_t *reward_out_dev, uint32_t *alive_out_dev, cgl_stream_t stream);

@@ -128,7 +128,7 @@ def test_decay_rule_equals_fork_cuda_kernel(ref_gpu, B, consts, side):
         assert np.array_equal(obs.cpu().numpy(), rs_), (side, consts, t)
         assert np.array_equal(oc, rw) and np.array_equal(os_, rs_), ("oracle", side, consts, t)
     # plain multi-step runs (cgl_env_run_rule: byte kernel for k < 4, bit-sliced decay kernel from k = 4 on)
-    if side <= 273:
+    if side <= 274:
         for k in (3, 9):
             for _ in range(k):
                 ref.step()

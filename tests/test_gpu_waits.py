@@ -193,7 +193,7 @@ def test_facade_toggle_step_pairs_without_reads(side):
     assert env.get_count() == n_plain + 12
 
 
-@pytest.mark.parametrize("side", [5, 10, 33, 64, 100, 320])
+@pytest.mark.parametrize("side", [5, 10, 33, 64, 100, 320, 448])
 def test_sim_step_one_launch_matches_oracle(side, native):
     """cgl_sim_step through the C ABI: mirror, reward, live count and sequence word, base and fork rules."""
     if not torch.cuda.is_available():
@@ -225,3 +225,18 @@ def test_sim_step_one_launch_matches_oracle(side, native):
             assert np.array_equal(c_d.cpu().numpy(), cells), (side, rule, t)
             assert np.array_equal(s_d.cpu().numpy(), st) and np.array_equal(mirror.numpy(), st), (side, rule, t)
             assert int(res[0]) == int(oracle.reward(st)) and int(res[1]) == int(oracle.alive(cells)) and int(res[2]) == t + 1
+
+
+def test_sim_step_rejects_side_above_limit(native):
+    """448 is the largest side whose byte plane and packed next world fit in shared memory; 449 is refused before any
+    launch."""
+    if not torch.cuda.is_available():
+        pytest.skip("needs a CUDA device")
+    lib = native.load()
+    side = 449
+    wa = torch.zeros(side * ((side + 31) // 32), dtype=torch.int32, device="cuda")
+    wb = torch.zeros_like(wa)
+    s_d = torch.zeros(side * side, dtype=torch.int8, device="cuda")
+    with pytest.raises(native.CglNativeError, match="side must be <= 448"):
+        native.check(lib.cgl_sim_step(native.dptr(wa), native.dptr(wb), native.dptr(s_d), side, side * side, SPAWN, STABLE,
+                                      0, 0, 0, 0, None, None, 1, native.current_stream()))
