@@ -12,26 +12,15 @@ in from the buffer edges advances one row per generation and never reaches an ow
 Horizontal wrap is local.  Message = k * C/8 bytes per neighbour per k generations.
 
 Exchange back ends
-  "persist" ONE cooperative launch per run() call (`cgl_life_band_run`): a warp keeps its strip of
-          rows for all sub-steps of kernel_k generations and waits only for its neighbour strips; every k generations
-          the strips that own a rank's first / last k owned rows store them into the ring neighbours' landing zones
-          over NVLink (CUDA-IPC mapped peer memory, two slots) and bump an arrival counter, and the strips that read
-          ghost rows wait for the counter and copy what they need out of their own landing zone.  No exchange
-          launch, no launch boundary between sub-steps, interior strips never wait for another GPU.  Correct and
-          tested, but measured slower than "p2p" (the persistent kernel's row loop runs at 0.88 us per row step
-          against 0.60: DESIGN.md section 4.6), so it is opt-in.
-  "fused" the halo exchange lives INSIDE the k-generation kernel
-          (`cgl_life_band_block`): the strips that produce a rank's first/last k owned rows store
-          them straight into the neighbours' next input buffers over NVLink (CUDA-IPC mapped peer
-          memory) and bump an arrival counter; only the strips that read ghost rows wait for the
-          neighbours' previous block.  No exchange launches, no host sync, interior strips never wait.
-  "p2p"   (default on GPUs) one exchange launch per block (`cgl_halo_exchange`, 8 CTAs per neighbour): writes the strip
-          straight into the neighbour's landing zone and publishes a sequence flag;
-          `cgl_halo_wait_copy` on the neighbour spins on the flag and moves the strip into its
-          ghost rows.  Two landing slots alternate by block parity, so a rank may run one block
-          ahead of its neighbour without a handshake.  No host synchronisation per exchange.
+  "p2p"   (default on GPUs) one exchange launch per block (`cgl_halo_exchange`, 8 CTAs per neighbour): each side
+          writes its strip straight into the neighbour's landing zone over NVLink (CUDA-IPC mapped peer memory) and
+          publishes a sequence flag, then spins on its own flag and moves the neighbour's strip into its ghost rows.
+          Two landing slots alternate by block parity, so a rank may run one block ahead of its neighbour without a
+          handshake.  No host synchronisation per exchange.  On one GPU, exchange="p2p" makes a ring of one that
+          exchanges with itself (tests the exchange kernel without a second GPU).
   "dist"  torch.distributed batch_isend_irecv (NCCL on GPUs, gloo in the CPU tests).
   "local" all G bands live in this process (one GPU emulating G ranks; tests the ghost-zone math).
+  "single" (default on one rank) no ghost rows: one torus, k-blocked launches of cgl_life_run.
 """
 from __future__ import annotations
 
@@ -83,9 +72,9 @@ class RowBandLife:
         if exchange is None:
             exchange = "single" if world_size == 1 else ("p2p" if self.device.type == "cuda" else "dist")
         self.exchange = exchange
-        # a ring of ONE with exchange="persist" keeps its ghost rows and exchanges with itself (its upper and lower
-        # neighbour are the rank itself: the torus wrap) -- the in-kernel exchange on a single GPU (tests)
-        self._self_ring = self.G == 1 and self.exchange == "persist"
+        # a ring of ONE with exchange="p2p" keeps its ghost rows and exchanges with itself (its upper and lower
+        # neighbour are the rank itself: the torus wrap) -- the exchange kernel on a single GPU (tests)
+        self._self_ring = self.G == 1 and self.exchange == "p2p"
         g = self.k if (self.G > 1 or self._self_ring) else 0
         self.ghost = g
         self.buf_rows = self.band_rows + 2 * g
@@ -94,14 +83,9 @@ class RowBandLife:
         self.block = 0              # exchanges done so far
         self.launches = 0
         self._ipc = None
-        self._fused = None
-        self._ghosts_valid = False
-        if self.exchange == "fused" and self.G > 1:
-            self._setup_fused(n)    # band buffers must be whole cudaMalloc allocations (IPC)
-        else:
-            self._a = torch.zeros(n, dtype=torch.int32, device=self.device)
-            self._b = torch.zeros(n, dtype=torch.int32, device=self.device)
-        if self.exchange in ("p2p", "persist") and (self.G > 1 or self._self_ring):
+        self._a = torch.zeros(n, dtype=torch.int32, device=self.device)
+        self._b = torch.zeros(n, dtype=torch.int32, device=self.device)
+        if self.exchange == "p2p" and (self.G > 1 or self._self_ring):
             self._setup_p2p()
 
     # ---------------------------------------------------------------- state access
@@ -118,7 +102,6 @@ class RowBandLife:
 
     def set_owned(self, words: torch.Tensor) -> None:
         self.owned.copy_(words.view(self.band_rows, self.W))
-        self._ghosts_valid = False
 
     def randomize(self, seed: int = 0) -> None:
         """Synthetic Bernoulli(0.5) start: every packed word uniform, seeded by GLOBAL row so that the
@@ -130,43 +113,6 @@ class RowBandLife:
             g.manual_seed(seed * 1000003 + (r0 + s))
             self.owned[s:s + chunk] = torch.randint(-2 ** 31, 2 ** 31 - 1, (chunk, self.W), dtype=torch.int32,
                                                     device=self.device, generator=g)
-        self._ghosts_valid = False
-
-    # ---------------------------------------------------------------- fused-exchange plumbing
-    def _alloc_shared(self, nbytes):
-        """cudaMalloc'ed (IPC-exportable) memory + its handle."""
-        ptr = ctypes.c_void_p()
-        handle = (ctypes.c_uint8 * 64)()
-        with torch.cuda.device(self.device):
-            native.check(self.lib.cgl_dev_alloc(nbytes, ctypes.byref(ptr)), "cgl_dev_alloc")
-            native.check(self.lib.cgl_ipc_get_handle(ptr, handle), "cgl_ipc_get_handle")
-        return ptr.value, bytes(handle)
-
-    def _as_tensor(self, ptr, n_words):
-        class _Raw:     # zero-copy int32 view of raw device memory
-            __cuda_array_interface__ = {"shape": (n_words,), "typestr": "<i4", "data": (ptr, False), "version": 2}
-        return torch.as_tensor(_Raw(), device=self.device)
-
-    def _setup_fused(self, n_words):
-        import torch.distributed as dist
-        mine = [self._alloc_shared(n_words * 4), self._alloc_shared(n_words * 4), self._alloc_shared(256)]
-        self._a = self._as_tensor(mine[0][0], n_words)
-        self._b = self._as_tensor(mine[1][0], n_words)
-        handles = [None] * self.G
-        dist.all_gather_object(handles, [h for _, h in mine], group=self.group)
-        up, down = (self.rank - 1) % self.G, (self.rank + 1) % self.G
-        peers = {}
-        with torch.cuda.device(self.device):
-            for p in {up, down}:
-                ptrs = []
-                for h in handles[p]:
-                    ptr = ctypes.c_void_p()
-                    native.check(self.lib.cgl_ipc_open_handle((ctypes.c_uint8 * 64).from_buffer_copy(h), ctypes.byref(ptr)),
-                                 "cgl_ipc_open_handle")
-                    ptrs.append(ptr.value)
-                peers[p] = ptrs
-        self._fused = dict(mine=[m[0] for m in mine], up=peers[up], down=peers[down], peers=peers, block_index=0)
-        dist.barrier(group=self.group)
 
     # ---------------------------------------------------------------- P2P plumbing
     def _setup_p2p(self):
@@ -198,20 +144,6 @@ class RowBandLife:
         dist.barrier(group=self.group)
 
     def close(self):
-        if self._fused:
-            import torch.distributed as dist
-            torch.cuda.synchronize(self.device)
-            dist.barrier(group=self.group)
-            f = self._fused
-            self._a = self._b = None
-            with torch.cuda.device(self.device):
-                for ptrs in f["peers"].values():
-                    for p in ptrs:
-                        self.lib.cgl_ipc_close_handle(ctypes.c_void_p(p))
-                dist.barrier(group=self.group)
-                for p in f["mine"]:
-                    self.lib.cgl_dev_free(ctypes.c_void_p(p))
-            self._fused = None
         if self._ipc:
             torch.cuda.synchronize(self.device)
             with torch.cuda.device(self.device):
@@ -241,7 +173,7 @@ class RowBandLife:
     def _exchange(self):
         """Fill the k ghost rows above/below the owned rows of the current buffer."""
         k, W, g = self.k, self.W, self.ghost
-        if self.G == 1:
+        if self.G == 1 and not self._self_ring:
             return
         a = self._a
         top_owned = a[g * W:(g + k) * W]                                     # my first k owned rows
@@ -249,7 +181,7 @@ class RowBandLife:
         ghost_up = a[0:k * W]
         ghost_down = a[(g + self.band_rows) * W:(g + self.band_rows + k) * W]
         self.block += 1
-        if self.exchange in ("dist", "fused"):      # fused: only to (re)fill the ghosts of a fresh grid
+        if self.exchange == "dist":
             import torch.distributed as dist
             up, down = (self.rank - 1) % self.G, (self.rank + 1) % self.G
             send_up, send_down = top_owned.clone(), bot_owned.clone()
@@ -283,7 +215,7 @@ class RowBandLife:
     def run(self, gens: int) -> None:
         """Advance `gens` generations (blocks of k generations between exchanges)."""
         lib, st = self.lib, self._stream()
-        if self.device.type == "cuda" and self.exchange not in ("fused", "persist") and not getattr(self, "_tuned", False):
+        if self.device.type == "cuda" and not getattr(self, "_tuned", False):
             # measure the strip length of the k-blocked kernel for this band shape once (clobbers _b only)
             with torch.cuda.device(self.device):
                 native.check(lib.cgl_life_tune(native.dptr(self._a), native.dptr(self._b),
@@ -297,10 +229,6 @@ class RowBandLife:
             self.launches += -(-gens // self.kernel_k)
             self.generation += gens
             return
-        if self.exchange == "fused":
-            return self._run_fused(gens)
-        if self.exchange == "persist":
-            return self._run_persist(gens)
         done = 0
         while done < gens:
             kb = min(self.k, gens - done)
@@ -309,81 +237,6 @@ class RowBandLife:
                 if not _life_block(lib, self._a, self._b, self.buf_rows, self.cols, 0, kb, min(kb, self.kernel_k), st):
                     self._a, self._b = self._b, self._a
             self.launches += -(-kb // self.kernel_k)
-            done += kb
-            self.generation += kb
-
-    def _run_persist(self, gens: int) -> None:
-        lib, ipc, st, kk = self.lib, self._ipc, self._stream(), self.kernel_k
-
-        def barrier():
-            if self.G > 1:
-                import torch.distributed as dist
-                dist.barrier(group=self.group)
-        if gens % kk:
-            raise ValueError(f"exchange='persist' runs whole sub-steps: gens must be a multiple of kernel_k = {kk}")
-        V = ctypes.c_void_p
-        if not self._ghosts_valid:
-            # fresh grid: zero the arrival counters on every rank, then the first call pushes the edge rows itself
-            torch.cuda.synchronize(self.device)
-            barrier()
-            with torch.cuda.device(self.device):
-                native.check(lib.cgl_dev_memset(V(ipc["base"] + ipc["flags_off"]), 0, 64, st), "cgl_dev_memset")
-            torch.cuda.synchronize(self.device)
-            barrier()
-            self.block = 0
-        strip, base, fo = ipc["strip"], ipc["base"], ipc["flags_off"]
-        up, down = ipc["up"], ipc["down"]
-        arr = V * 2
-        # my first owned rows -> the upper neighbour's "from below" zone; my last owned rows -> the lower one's "from above"
-        peer_up = arr(up + strip, up + 3 * strip)
-        peer_dn = arr(down, down + 2 * strip)
-        mine_up = arr(base, base + 2 * strip)
-        mine_dn = arr(base + strip, base + 3 * strip)
-        n_sub = gens // kk
-        with torch.cuda.device(self.device):
-            native.check(lib.cgl_life_band_run(
-                native.dptr(self._a), native.dptr(self._b), self.buf_rows, self.cols, self.ghost, kk, n_sub, self.block,
-                int(not self._ghosts_valid), peer_up, peer_dn, V(up + fo + 4), V(down + fo), mine_up, mine_dn,
-                V(base + fo), V(base + fo + 4), st), "cgl_life_band_run")
-        self._ghosts_valid = True
-        per_block = self.k // kk
-        self.block += -(-n_sub // per_block)
-        if n_sub & 1:
-            self._a, self._b = self._b, self._a
-        self.launches += 1
-        self.generation += gens
-
-    _BLOCK_SIZES = (16, 12, 8, 6, 4, 3, 2, 1)       # generations one fused launch can do
-
-    def _run_fused(self, gens: int) -> None:
-        import torch.distributed as dist
-        f, lib, st = self._fused, self.lib, self._stream()
-        if not self._ghosts_valid:
-            # fresh grid: fill the ghost rows once with a plain exchange and restart the counters
-            torch.cuda.synchronize(self.device)
-            dist.barrier(group=self.group)
-            self._exchange()
-            torch.cuda.synchronize(self.device)
-            with torch.cuda.device(self.device):
-                native.check(lib.cgl_dev_memset(ctypes.c_void_p(f["mine"][2]), 0, 256, st), "cgl_dev_memset")
-            torch.cuda.synchronize(self.device)
-            dist.barrier(group=self.group)
-            f["block_index"] = 0
-            self._ghosts_valid = True
-        done = 0
-        while done < gens:
-            kb = next(s for s in self._BLOCK_SIZES if s <= min(self.k, gens - done))
-            f["block_index"] += 1
-            cur_is_a = self._a.data_ptr() == f["mine"][0]
-            i_in, i_out = (0, 1) if cur_is_a else (1, 0)
-            with torch.cuda.device(self.device):
-                native.check(lib.cgl_life_band_block(
-                    ctypes.c_void_p(f["mine"][i_in]), ctypes.c_void_p(f["mine"][i_out]), self.buf_rows, self.cols,
-                    self.ghost, kb, ctypes.c_void_p(f["up"][i_out]), ctypes.c_void_p(f["down"][i_out]),
-                    ctypes.c_void_p(f["up"][2]), ctypes.c_void_p(f["down"][2]), ctypes.c_void_p(f["mine"][2]),
-                    f["block_index"], st), "cgl_life_band_block")
-            self._a, self._b = self._b, self._a
-            self.launches += 1
             done += kb
             self.generation += kb
 

@@ -15,6 +15,7 @@ _PKG_DIR = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 LIB_PATH = os.environ.get("CGL_B200_LIB") or os.path.join(_PKG_DIR, "libcgl_b200.so")      # (override: tuning builds)
 
 E_BADARG, E_BADINDEX, E_NOMEM = -1, -2, -3
+ABI_VERSION = 2                         # CGL_B200_ABI_VERSION
 
 
 class CglNativeError(RuntimeError):
@@ -64,14 +65,7 @@ SIGNATURES = {
     "cgl_ipc_get_handle": (_i, [_vp, _vp]),
     "cgl_ipc_open_handle": (_i, [_vp, ctypes.POINTER(_vp)]),
     "cgl_ipc_close_handle": (_i, [_vp]),
-    "cgl_halo_push": (_i, [_vp, _vp, _u64, _vp, _u32, _vp]),
     "cgl_halo_exchange": (_i, [_vp] * 12 + [_u64, _u32, _vp]),
-    "cgl_halo_wait": (_i, [_vp, _u32, _vp]),
-    "cgl_halo_wait_copy": (_i, [_vp, _u32, _vp, _vp, _u64, _vp]),
-    "cgl_life_band_block": (_i, [_vp, _vp, _u32, _u32, _u32, _u32, _vp, _vp, _vp, _vp, _vp, _u32, _vp]),
-    "cgl_life_band_run": (_i, [_vp, _vp, _u32, _u32, _u32, _u32, _u32, _u32, _i, ctypes.POINTER(_vp), ctypes.POINTER(_vp),
-                               _vp, _vp, ctypes.POINTER(_vp), ctypes.POINTER(_vp), _vp, _vp, _vp]),
-    "cgl_life_band_run_supported": (_i, [_u32, _u32, _u32]),
     "cgl_dev_alloc": (_i, [_u64, ctypes.POINTER(_vp)]),
     "cgl_dev_free": (_i, [_vp]),
     "cgl_dev_memset": (_i, [_vp, _i, _u64, _vp]),
@@ -140,7 +134,7 @@ def load(build_if_missing: bool = True) -> ctypes.CDLL:
     for name, (res, args) in SIGNATURES.items():
         fn = getattr(lib, name)          # AttributeError here == header/library mismatch
         fn.restype, fn.argtypes = res, args
-    if lib.cgl_abi_version() != 1:
+    if lib.cgl_abi_version() != ABI_VERSION:
         raise CglNativeError("libcgl_b200.so ABI version mismatch")
     _lib = lib
     return lib
@@ -160,7 +154,7 @@ def ext():
         except ImportError as exc:
             raise CglNativeError(f"cgl_b200/_cgl_ext.so is missing or does not load ({exc}): build it with "
                                  f"`python {_PKG_DIR}/build.py --ext`") from exc
-        if mod.abi_version() != 1:
+        if mod.abi_version() != ABI_VERSION:
             raise CglNativeError("_cgl_ext.so was built against another ABI version")
         _ext = mod
     return _ext

@@ -30,18 +30,6 @@ int sm_count()
     return cached[dev];
 }
 
-// Copy a halo strip into a peer GPU's ghost rows, then publish `seq` (release, system scope).
-__global__ void halo_push_kernel(const uint4 *__restrict__ src, uint4 *__restrict__ dst, uint64_t n_vec,
-                                 uint32_t *flag, uint32_t seq)
-{
-    for (uint64_t i = threadIdx.x; i < n_vec; i += blockDim.x) dst[i] = src[i];
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        __threadfence_system();
-        asm volatile("st.release.sys.global.u32 [%0], %1;" ::"l"(flag), "r"(seq) : "memory");
-    }
-}
-
 // Wait until *flag - seq >= 0 (acquire, system scope).  Bounded: a peer that died or never launched its side of
 // the exchange raises the halo alarm word after g_wait_ns instead of hanging this GPU until a device reset.
 __device__ __forceinline__ bool spin_until(const uint32_t *flag, uint32_t seq)
@@ -56,19 +44,6 @@ __device__ __forceinline__ bool spin_until(const uint32_t *flag, uint32_t seq)
     } while ((++spins & 127u) != 0 || !wait_expired(t0, ALARM_HALO));
     raise_alarm(ALARM_HALO);
     return false;
-}
-
-__global__ void halo_wait_kernel(const uint32_t *flag, uint32_t seq) { spin_until(flag, seq); }
-
-// Wait for the peer's strip (flag >= seq), then move it from the landing zone into the ghost rows.
-__global__ void halo_wait_copy_kernel(const uint32_t *flag, uint32_t seq, const uint4 *__restrict__ src,
-                                      uint4 *__restrict__ dst, uint64_t n_vec)
-{
-    __shared__ int arrived;
-    if (threadIdx.x == 0) arrived = spin_until(flag, seq);
-    __syncthreads();
-    if (!arrived) return;                       // timed out: the ghost rows keep their old contents, alarm raised
-    for (uint64_t i = threadIdx.x; i < n_vec; i += blockDim.x) dst[i] = src[i];
 }
 
 // Whole halo exchange of one rank in ONE launch: CTA 0 talks to the upper neighbour, CTA 1 to the
@@ -122,7 +97,6 @@ static int apply_hooks()
     int rc;
     if ((rc = set_hooks_env(g_alarm_dev, g_wait_ns_host))) return rc;
     if ((rc = set_hooks_life_tb(g_alarm_dev, g_wait_ns_host))) return rc;
-    if ((rc = set_hooks_life_persist(g_alarm_dev, g_wait_ns_host))) return rc;
     return set_hooks_api(g_alarm_dev, g_wait_ns_host);
 }
 
@@ -323,7 +297,7 @@ extern "C" int cgl_stream_wait(cgl_stream_t stream)
 }
 
 
-// ---- IPC + halo ------------------------------------------------------------------------------
+// ---- IPC ------------------------------------------------------------------------------------
 static_assert(sizeof(cudaIpcMemHandle_t) == 64, "IPC handle size");
 
 extern "C" int cgl_ipc_get_handle(void *dev_ptr, uint8_t handle_out[64])
@@ -351,29 +325,6 @@ extern "C" int cgl_ipc_close_handle(void *dev_ptr)
     return 0;
 }
 
-extern "C" int cgl_halo_push(const uint32_t *src, uint32_t *peer_dst, uint64_t n_words,
-                             uint32_t *peer_flag, uint32_t seq, cgl_stream_t stream)
-{
-    CGL_REQUIRE(src && peer_dst && peer_flag && n_words && n_words % 4 == 0, CGL_E_BADARG,
-                "cgl_halo_push: bad argument (n_words must be a multiple of 4)");
-    halo_push_kernel<<<1, 1024, 0, as_stream(stream)>>>(reinterpret_cast<const uint4 *>(src),
-                                                        reinterpret_cast<uint4 *>(peer_dst), n_words / 4,
-                                                        peer_flag, seq);
-    CGL_LAUNCH_CHECK();
-    return 0;
-}
-
-extern "C" int cgl_halo_wait_copy(const uint32_t *flag, uint32_t seq, const uint32_t *src, uint32_t *dst,
-                                  uint64_t n_words, cgl_stream_t stream)
-{
-    CGL_REQUIRE(flag && src && dst && n_words && n_words % 4 == 0, CGL_E_BADARG,
-                "cgl_halo_wait_copy: bad argument (n_words must be a multiple of 4)");
-    halo_wait_copy_kernel<<<1, 1024, 0, as_stream(stream)>>>(flag, seq, reinterpret_cast<const uint4 *>(src),
-                                                             reinterpret_cast<uint4 *>(dst), n_words / 4);
-    CGL_LAUNCH_CHECK();
-    return 0;
-}
-
 extern "C" int cgl_dev_alloc(uint64_t bytes, void **dev_ptr_out)
 {
     CGL_REQUIRE(bytes && dev_ptr_out, CGL_E_BADARG, "cgl_dev_alloc: bad argument");
@@ -392,13 +343,5 @@ extern "C" int cgl_dev_memset(void *dev_ptr, int value, uint64_t bytes, cgl_stre
 extern "C" int cgl_dev_free(void *dev_ptr)
 {
     CGL_CUDA(cudaFree(dev_ptr));
-    return 0;
-}
-
-extern "C" int cgl_halo_wait(const uint32_t *flag, uint32_t seq, cgl_stream_t stream)
-{
-    CGL_REQUIRE(flag, CGL_E_BADARG, "cgl_halo_wait: null");
-    halo_wait_kernel<<<1, 1, 0, as_stream(stream)>>>(flag, seq);
-    CGL_LAUNCH_CHECK();
     return 0;
 }

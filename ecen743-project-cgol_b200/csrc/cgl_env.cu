@@ -1024,32 +1024,6 @@ extern "C" int cgl_init_stable_rule(const uint32_t *world, int8_t *stable, uint6
 
 extern "C" int cgl_life_step(const uint32_t *in, uint32_t *out, uint64_t n_envs, uint32_t rows,
                              uint32_t cols, int wrap_rows, uint32_t *alive_out, cgl_stream_t stream);
-extern "C" int cgl_env_step_tma(uint32_t *win, uint32_t *wout, int8_t *stable, uint64_t n_envs, uint32_t side,
-                                const int32_t *actions, int spawn, int stable_max, int32_t *reward,
-                                uint32_t *alive, int *err, cgl_stream_t stream, int threads);
-
-// Tuning knobs (environment, read once): CGL_ENV_IMPL = "fused" (default) | "tma";
-// CGL_ENV_TMA_THREADS = 128 | 256 (default).  Measured on B200 (tools/sweep_env.py, profiles/):
-// the per-env fused kernel streams at 98-99 % of the HBM roofline once >= ~14 waves of CTAs are
-// in flight; the persistent bulk-copy kernel currently reaches 91 %, so it stays opt-in.
-static int env_impl_is_tma()
-{
-    static int v = -1;
-    if (v < 0) {
-        const char *e = getenv("CGL_ENV_IMPL");
-        v = (e && e[0] == 't') ? 1 : 0;
-    }
-    return v;
-}
-static int env_tma_threads()
-{
-    static int v = 0;
-    if (v == 0) {
-        const char *e = getenv("CGL_ENV_TMA_THREADS");
-        v = (e && atoi(e) == 128) ? 128 : 256;
-    }
-    return v;
-}
 
 // The one implementation behind every env-step entry point (see include/cgl_b200.h, cgl_env_step_ex).
 extern "C" int cgl_env_step_ex(const cgl_env_step_args_t *args, cgl_stream_t stream)
@@ -1076,13 +1050,8 @@ extern "C" int cgl_env_step_ex(const cgl_env_step_args_t *args, cgl_stream_t str
         a.publish = a.want + 1;
     }
     cudaStream_t st = as_stream(stream);
-    const bool ext = a.dead_rule != CGL_DEAD_ZERO || a.masked_toggle;
     int rc = -100;
-    if (!ext && a.stable_out_dev == a.stable_in_dev && a.chain_mode == CGL_CHAIN_NONE && env_impl_is_tma() &&
-        (a.side == 32 || a.side == 64 || a.side == 128))
-        rc = cgl_env_step_tma(a.world_in_dev, a.world_out_dev, a.stable_out_dev, a.n_envs, a.side, a.actions_dev, a.spawn,
-                              a.stable_max, a.reward_out_dev, a.alive_out_dev, a.err_flag_dev, stream, env_tma_threads());
-    if (rc == -100 && fused) {
+    if (fused) {
         switch (a.side) {
         case 32: rc = launch_env_fused<32>(a, st); break;
         case 64: rc = launch_env_fused<64>(a, st); break;

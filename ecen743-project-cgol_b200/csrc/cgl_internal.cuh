@@ -76,11 +76,6 @@ enum { ALARM_BAD_ACTION = 0, ALARM_ENV_TOKEN = 1, ALARM_LIFE_TOKEN = 2, ALARM_HA
 int set_hooks_env(int *alarm_dev, unsigned long long wait_ns);
 int set_hooks_life_tb(int *alarm_dev, unsigned long long wait_ns);
 int set_hooks_api(int *alarm_dev, unsigned long long wait_ns);
-int set_hooks_life_persist(int *alarm_dev, unsigned long long wait_ns);
-
-// cgl_life_persist.cu: n_sub sub-steps of k generations in one cooperative launch; -100 = not applicable.
-int life_persist_run(uint32_t *a, uint32_t *b, uint32_t rows, uint32_t cols, int wrap_rows, uint32_t n_sub, int k,
-                     cudaStream_t st);
 
 #if defined(__CUDACC__)
 __device__ __forceinline__ uint32_t ld_nc_u32(const uint32_t *p) { return __ldg(p); }

@@ -29,22 +29,6 @@ struct Win {            // window of one level: rows (a-1, a) of the level's inp
 // (IMAD / IMAD.HI with opaque multipliers) is 6 % SLOWER although the kernel is ALU-pipe bound, and
 // one-warp CTAs are 12 % slower than 4-warp CTAs, and mapping a whole CTA to one row block (loop
 // bounds in uniform registers) is 7 % slower than the warp-linear mapping below; all removed again.
-// Fused halo exchange (row bands over NVLink, one process per GPU).  With HALO the kernel
-//   * stores locally only the rows this rank owns ([store_lo, store_hi) of its band buffer),
-//   * stores the first / last `depth` owned rows ALSO straight into the ghost rows of the ring
-//     neighbours' output buffers (peer-mapped pointers: plain st.global over NVLink),
-//   * a strip that pushed bumps the neighbour's arrival counter (system-scope release) when it is
-//     done, and a strip that reads ghost rows first waits until its own counters show that BOTH
-//     neighbours finished the previous block (acquire) -- interior strips never wait, so the
-//     exchange overlaps the compute and costs no extra launch.
-struct HaloCtx {
-    uint32_t store_lo, store_hi;          // owned rows of the band buffer
-    uint32_t depth;                       // ghost depth = rows pushed per direction
-    uint32_t *push_up, *push_dn;          // peer: where my row store_lo / my row store_hi - depth lands
-    uint32_t *sig_up, *sig_dn;            // peer arrival counters
-    const uint32_t *wait_up, *wait_dn;    // my arrival counters (filled by the neighbours)
-    uint32_t wait_up_target, wait_dn_target;
-};
 
 // Chained launches of one cgl_life_run: strip (cg, rb) of launch j needs the outputs of -- and must
 // not overwrite the inputs of -- the 3 x 3 neighbouring strips of launch j-1.  Each strip publishes
@@ -52,20 +36,6 @@ struct HaloCtx {
 // reach j; with programmatic dependent launch the first strips of launch j+1 then run while the
 // last strips of launch j finish, which removes the cost of a partly filled last wave.
 struct ChainCtx { uint32_t *tokens; uint32_t want; uint32_t cap; };
-
-// Spin until *ctr - target >= 0 (acquire, system scope); every exit is a warp vote, so the warp stays
-// convergent.  Bounded by g_wait_ns: false = the neighbour never arrived (alarm raised by the caller).
-__device__ __forceinline__ bool wait_counter(const uint32_t *ctr, uint32_t target)
-{
-    uint32_t v, spins = 0;
-    unsigned long long t0 = 0;
-    while (true) {
-        asm volatile("ld.acquire.sys.global.u32 %0, [%1];" : "=r"(v) : "l"(ctr) : "memory");
-        if (!__any_sync(0xffffffffu, (int32_t)(v - target) < 0)) return true;      // warp-uniform exit
-        if (spins == 0) t0 = globaltimer_ns();
-        if ((++spins & 255u) == 0 && __any_sync(0xffffffffu, wait_expired(t0, ALARM_HALO))) return false;
-    }
-}
 
 // Predicated store: `if (ok && a < b) *p = v` as ONE predicated STG.  Written in PTX on purpose: the
 // row-range test is CTA-uniform, and for a uniform condition the compiler emits a branch around the
@@ -87,17 +57,14 @@ constexpr int TB_COLS = 30;             // valid word-columns per warp
 
 constexpr int TB_THREADS = 128;
 
-// (Capping the fused-exchange variant at the plain kernel's 96 registers spills and is slower.)
-template <int K, bool HALO>
+template <int K>
 __global__ void __launch_bounds__(TB_THREADS)
 life_tb_kernel(const uint32_t *__restrict__ in, uint32_t *__restrict__ out, uint32_t rows, uint32_t W,
-               uint32_t rpt, int wrap_rows, uint32_t n_cgroups, uint32_t n_rblocks, const HaloCtx hc,
-               const ChainCtx chain)
+               uint32_t rpt, int wrap_rows, uint32_t n_cgroups, uint32_t n_rblocks, const ChainCtx chain)
 {
     // Warps are numbered along the row first (column group fastest).  No early exit: padding warps
-    // redo the last strip with stores off, the loop trip count is the same for every warp, and the
-    // halo waits are branch-free PTX -- so every shuffle below is provably convergent (plain SHFL;
-    // a divergence fallback path costs ~8 %).
+    // redo the last strip with stores off and the loop trip count is the same for every warp, so
+    // every shuffle below is provably convergent (plain SHFL; a divergence fallback path costs ~8 %).
     const uint32_t lane = threadIdx.x & 31;
     const uint32_t warp = blockIdx.x * (TB_THREADS / 32) + (threadIdx.x >> 5);
     const uint32_t cg = warp % n_cgroups;
@@ -106,7 +73,7 @@ life_tb_kernel(const uint32_t *__restrict__ in, uint32_t *__restrict__ out, uint
     rb = warp_ok ? rb : n_rblocks - 1;
     bool wait_ok = true;                                       // warp-uniform: false once a bounded wait expired
 
-    if (!HALO && chain.tokens != nullptr) {                    // kernel-uniform branch
+    if (chain.tokens != nullptr) {                             // kernel-uniform branch
         cudaTriggerProgrammaticLaunchCompletion();
         // lanes 0..8 watch one neighbour strip each (columns always wrap, rows wrap on the torus)
         const int dj = (int)(lane % 3) - 1, di = (int)(lane / 3) - 1;
@@ -136,7 +103,7 @@ life_tb_kernel(const uint32_t *__restrict__ in, uint32_t *__restrict__ out, uint
 
     const int wi = (int)(cg * TB_COLS + lane) - 1;             // word column of this lane (may be -1 or >= W)
     const uint32_t wcol = wi < 0 ? (uint32_t)(wi + (int)W) : ((uint32_t)wi >= W ? (uint32_t)wi - W : (uint32_t)wi);
-    bool store_ok = warp_ok && wait_ok && lane >= 1 && lane <= TB_COLS && (uint32_t)wi < W;
+    const bool store_ok = warp_ok && wait_ok && lane >= 1 && lane <= TB_COLS && (uint32_t)wi < W;
 
     const int r0 = (int)(rb * rpt);
     const int r1 = (r0 + (int)rpt < (int)rows) ? r0 + (int)rpt : (int)rows;
@@ -155,24 +122,6 @@ life_tb_kernel(const uint32_t *__restrict__ in, uint32_t *__restrict__ out, uint
     const uint32_t *ip = in + wcol;
     uint32_t *op = out + (store_ok ? (uint32_t)wi : 0u);
 
-    // HALO: does this strip push rows to a neighbour / read ghost rows?  (warp-uniform)
-    bool push_up = false, push_dn = false;
-    if (HALO) {
-        push_up = warp_ok && (uint32_t)r0 < hc.store_lo + hc.depth && (uint32_t)r1 > hc.store_lo;
-        push_dn = warp_ok && (uint32_t)r0 < hc.store_hi && (uint32_t)r1 + hc.depth > hc.store_hi;
-        const bool reads_up = r0 - K < (int)hc.store_lo, reads_dn = (uint32_t)(r1 + K) > hc.store_hi;
-        // unconditional (branch-free): strips that need nothing wait for target 0, i.e. not at all
-        const bool up_ok = wait_counter(hc.wait_up, (reads_up || push_up) ? hc.wait_up_target : 0u);
-        const bool dn_ok = wait_counter(hc.wait_dn, (reads_dn || push_dn) ? hc.wait_dn_target : 0u);
-        if (!(up_ok && dn_ok)) {                               // a ring neighbour never arrived: see above
-            wait_ok = false;
-            store_ok = false;
-            push_up = push_dn = false;
-            if (lane == 0) raise_alarm(ALARM_HALO);
-        }
-    }
-
-    const uint32_t owned_rows = HALO ? hc.store_hi - hc.store_lo : 0u;
     Win win[K];
     uint32_t pend[K];                   // pend[g] = output of level g+1 at the previous step
 #pragma unroll
@@ -188,7 +137,7 @@ life_tb_kernel(const uint32_t *__restrict__ in, uint32_t *__restrict__ out, uint
             const uint32_t ru = umin((uint32_t)rw + u, (uint32_t)rw + u - rows);      // (rw + u) mod rows
             raw[u] = 0;
             if ((uint32_t)(s0 + u - s_lo) < span)                                       // rows * W < 2^32
-                raw[u] = HALO ? __ldcg(ip + ru * W) : __ldg(ip + ru * W);               // ghost rows: L2 only
+                raw[u] = __ldg(ip + ru * W);
         }
         rw += TB_UNROLL;
         rw = rw >= irows ? rw - irows : rw;
@@ -210,33 +159,15 @@ life_tb_kernel(const uint32_t *__restrict__ in, uint32_t *__restrict__ out, uint
             // row r0 + so of generation K has just left level K
             const uint32_t so = (uint32_t)(s0 + u - (3 * K - 1));
             const uint32_t ro = (uint32_t)r0 + so;
-            if (!HALO) {
-                st_if_lt(op + ro * W, pend[K - 1], store_ok, so, out_rows);
-            } else {
-                const bool in_strip = store_ok && so < out_rows;
-                const uint32_t rel = ro - hc.store_lo;             // row within the owned range
-                st_if_lt(op + ro * W, pend[K - 1], in_strip, rel, owned_rows);
-                st_if_lt(hc.push_up + rel * W + (uint32_t)wi, pend[K - 1], in_strip, rel, hc.depth);
-                st_if_lt(hc.push_dn + (rel - (owned_rows - hc.depth)) * W + (uint32_t)wi, pend[K - 1],
-                         in_strip && rel < owned_rows, owned_rows - 1 - rel, hc.depth);
-            }
+            st_if_lt(op + ro * W, pend[K - 1], store_ok, so, out_rows);
         }
     }
-    if (!HALO && chain.tokens != nullptr) {
+    if (chain.tokens != nullptr) {
         __threadfence();                             // this strip's rows are visible device-wide ...
         __syncwarp();
         if (lane == 0 && warp_ok && wait_ok)         // ... before its token is published
             asm volatile("st.release.gpu.global.u32 [%0], %1;" ::"l"(chain.tokens + rb * n_cgroups + cg),
                          "r"(chain.want + 1) : "memory");
-    }
-    if (HALO) {
-        __threadfence_system();                      // my peer stores are visible system-wide ...
-        __syncwarp();
-        if (lane == 0 && warp_ok) {                  // ... before the arrival is published
-            __threadfence_system();
-            if (push_up) asm volatile("red.release.sys.global.add.u32 [%0], 1;" ::"l"(hc.sig_up) : "memory");
-            if (push_dn) asm volatile("red.release.sys.global.add.u32 [%0], 1;" ::"l"(hc.sig_dn) : "memory");
-        }
     }
 }
 
@@ -248,18 +179,12 @@ life_tb_kernel(const uint32_t *__restrict__ in, uint32_t *__restrict__ out, uint
 // strips are short: the 8192-row bands of the 8-GPU C4 run (~200-row strips) spend 10 % of every launch in the
 // fill of the skewed pipeline.  Parallelism inside a warp now comes from the wavefront over the unrolled row steps
 // (step u+1 of level g and step u of level g+1 are independent) instead of from K independent levels.
-// Same strip geometry, chaining and ghost-zone contract as life_tb_kernel (non-HALO).
+// Same strip geometry, chaining and ghost-zone contract as life_tb_kernel.
 // Row steps per block and software prefetch of the next block's rows.  Measured on B200 (8320 x 65536 band /
 // 65536^2 torus, us per generation): 6 steps no prefetch 16.18 / 116.5, 8 steps 15.97 / 115.1, 4 steps with the
 // next block's rows requested before the current block is computed 15.76 / 114.1 (96 registers: still 5 CTAs per
 // SM), 3 steps with prefetch 15.88 / 115.2, 4 steps without 21.2 / 151.
-#ifndef CGL_TB2_UNROLL
-#define CGL_TB2_UNROLL 4
-#endif
-#ifndef CGL_TB2_PREFETCH
-#define CGL_TB2_PREFETCH 1
-#endif
-constexpr int TB2_UNROLL = CGL_TB2_UNROLL;
+constexpr int TB2_UNROLL = 4;
 
 template <int K, bool PRO>
 __device__ __forceinline__ void tb2_block(const uint32_t (&raw)[TB2_UNROLL], Win (&win)[K], int s0, uint32_t *op, uint32_t r0W,
@@ -361,7 +286,6 @@ life_tb2_kernel(const uint32_t *__restrict__ in, uint32_t *__restrict__ out, uin
     };
     constexpr int PRO_STEPS = (2 * K + TB2_UNROLL - 1) / TB2_UNROLL * TB2_UNROLL;   // start-up: levels come in one by one
     int s0 = 0;
-#if CGL_TB2_PREFETCH
     // software pipeline: the rows of block i + 1 are requested before block i is computed (two row buffers)
     uint32_t ra[TB2_UNROLL], rbuf[TB2_UNROLL];
     load(ra, 0);
@@ -377,18 +301,6 @@ life_tb2_kernel(const uint32_t *__restrict__ in, uint32_t *__restrict__ out, uin
         load(ra, s0 + 2 * TB2_UNROLL);
         tb2_block<K, false>(rbuf, win, s0 + TB2_UNROLL, op, r0W, W, store_ok, out_rows);
     }
-#else
-    for (; s0 < PRO_STEPS && s0 < n_steps; s0 += TB2_UNROLL) {
-        uint32_t raw[TB2_UNROLL];
-        load(raw, s0);
-        tb2_block<K, true>(raw, win, s0, op, r0W, W, store_ok, out_rows);
-    }
-    for (; s0 < n_steps; s0 += TB2_UNROLL) {
-        uint32_t raw[TB2_UNROLL];
-        load(raw, s0);
-        tb2_block<K, false>(raw, win, s0, op, r0W, W, store_ok, out_rows);
-    }
-#endif
     if (chain.tokens != nullptr) {
         __threadfence();
         __syncwarp();
@@ -398,22 +310,13 @@ life_tb2_kernel(const uint32_t *__restrict__ in, uint32_t *__restrict__ out, uin
     }
 }
 
-// Which pipeline a K-generation launch uses: 1 = direct (life_tb2_kernel), 0 = skewed (life_tb_kernel).  Measured on
+// Which pipeline a K-generation launch uses: true = direct (life_tb2_kernel), false = skewed (life_tb_kernel).  Measured on
 // B200 (profiles/r02_sweeps.md), us per generation direct vs skewed -- one 8-GPU band of C4 (8320 x 65536): K = 2
 // 28.8 / 34.8, 4: 17.8 / 23.7, 6: 17.5 / 23.6, 8: 16.2 / 16.8, 12: 16.8 / 18.2, 16: 18.8 / 18.1; 32768^2: K = 2
 // 41.0 / 65.1, 4: 33.4 / 45.4, 8: 30.5 / 31.2, 16: 34.1 / 35.1.  The direct pipeline wins wherever the K levels fit
 // the register file with room to overlap row steps; at K = 16 (164 registers, 3 CTAs per SM) it is a tie and the
-// skewed one stays.  CGL_TB_MODE=0/1 forces one.
-static int tb_mode(int K)
-{
-    static int forced = -2;
-    if (forced == -2) {
-        const char *e = getenv("CGL_TB_MODE");
-        forced = e ? atoi(e) : -1;
-    }
-    if (forced >= 0) return forced;
-    return K <= 12 ? 1 : 0;
-}
+// skewed one stays.
+constexpr bool tb_direct(int K) { return K <= 12; }
 
 // Strip length for a (rows x cols) grid.  A strip costs rpt + 3K - 1 row steps (pipeline fill), and
 // the grid runs in ceil(CTAs / resident CTAs) waves of equally long CTAs; pick the candidate that
@@ -456,50 +359,30 @@ static uint32_t tuned_rows(uint32_t rows, uint32_t W, int K)
     return 0;
 }
 
-// Strips (per column group) whose output rows intersect [lo, hi).
-static uint32_t strips_touching(uint32_t lo, uint32_t hi, uint32_t rpt, uint32_t rows)
-{
-    if (hi > rows) hi = rows;
-    if (lo >= hi) return 0;
-    return (hi - 1) / rpt - lo / rpt + 1;
-}
-
-// HALO launches: `halo` carries the pointers; *_target are filled in here from `block_index`
-// (1-based count of band blocks since the ghosts were last filled by a plain exchange).
-template <int K, bool HALO>
+template <int K>
 static int launch_tb(const uint32_t *in, uint32_t *out, uint32_t rows, uint32_t cols, int wrap_rows,
-                     cudaStream_t st, HaloCtx halo = HaloCtx(), uint32_t block_index = 0, ChainCtx chain = ChainCtx(),
-                     uint32_t *n_strips_out = nullptr)
+                     cudaStream_t st, ChainCtx chain)
 {
     static int rpt_knob = -1, occ = 0;   // CGL_TB_ROWS overrides the strip length (tuning)
     if (rpt_knob < 0) {
         const char *e = getenv("CGL_TB_ROWS");
         rpt_knob = e ? atoi(e) : 0;
         int n = 0;
-        if (!HALO && tb_mode(K) == 1)
+        if constexpr (tb_direct(K))
             CGL_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, life_tb2_kernel<K>, TB_THREADS, 0));
         else
-            CGL_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, life_tb_kernel<K, HALO>, TB_THREADS, 0));
+            CGL_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, life_tb_kernel<K>, TB_THREADS, 0));
         occ = n > 0 ? n : 1;
     }
     const uint32_t W = cols / 32;
     const uint32_t n_cgroups = (W + TB_COLS - 1) / TB_COLS;
-    uint32_t rpt = rpt_knob > 0 ? (uint32_t)rpt_knob : (HALO ? 0u : tuned_rows(rows, W, K));
+    uint32_t rpt = rpt_knob > 0 ? (uint32_t)rpt_knob : tuned_rows(rows, W, K);
     if (rpt == 0) rpt = tb_pick_rows(rows, n_cgroups, K, (uint64_t)sm_count() * occ);
     if (rpt > rows) rpt = rows;
     const uint32_t n_rblocks = (rows + rpt - 1) / rpt;
     const uint64_t blocks = ((uint64_t)n_cgroups * n_rblocks + TB_THREADS / 32 - 1) / (TB_THREADS / 32);
     CGL_REQUIRE(blocks < (1ull << 31) && rows < (1u << 30) && (uint64_t)rows * W < (1ull << 32), CGL_E_BADARG,
                 "cgl_life_run: grid too large for the k-blocked kernel (rows * cols/32 must be < 2^32)");
-    if (HALO) {
-        // every rank has the same geometry, so my neighbours' strip counts equal mine: the upper
-        // neighbour signals me once per strip that pushed ITS bottom rows, the lower one per top strip
-        const uint32_t top = strips_touching(halo.store_lo, halo.store_lo + halo.depth, rpt, rows) * n_cgroups;
-        const uint32_t bot = strips_touching(halo.store_hi - halo.depth, halo.store_hi, rpt, rows) * n_cgroups;
-        halo.wait_up_target = (block_index - 1) * bot;
-        halo.wait_dn_target = (block_index - 1) * top;
-    }
-    if (n_strips_out) *n_strips_out = n_cgroups * n_rblocks;
     // chaining needs the nine-neighbour footprint (strips at least K rows long) and a large enough token buffer
     if (chain.tokens != nullptr && (rpt < (uint32_t)K || (uint64_t)n_cgroups * n_rblocks > chain.cap)) chain.tokens = nullptr;
     cudaLaunchConfig_t cfg = {};
@@ -511,26 +394,20 @@ static int launch_tb(const uint32_t *in, uint32_t *out, uint32_t rows, uint32_t 
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
     cfg.numAttrs = (chain.tokens != nullptr && chain.want > 0) ? 1 : 0;        // the first launch of a run waits normally
-    if constexpr (!HALO) {
-        if (tb_mode(K) == 1) {
-            CGL_CUDA(cudaLaunchKernelEx(&cfg, life_tb2_kernel<K>, in, out, rows, W, rpt, wrap_rows, n_cgroups, n_rblocks, chain));
-            return 0;
-        }
-    }
-    CGL_CUDA(cudaLaunchKernelEx(&cfg, life_tb_kernel<K, HALO>, in, out, rows, W, rpt, wrap_rows, n_cgroups, n_rblocks,
-                                halo, chain));
+    if constexpr (tb_direct(K))
+        CGL_CUDA(cudaLaunchKernelEx(&cfg, life_tb2_kernel<K>, in, out, rows, W, rpt, wrap_rows, n_cgroups, n_rblocks, chain));
+    else
+        CGL_CUDA(cudaLaunchKernelEx(&cfg, life_tb_kernel<K>, in, out, rows, W, rpt, wrap_rows, n_cgroups, n_rblocks, chain));
     return 0;
 }
 
-template <bool HALO>
 static int tb_dispatch(int k, const uint32_t *in, uint32_t *out, uint32_t rows, uint32_t cols, int wrap_rows,
-                       cudaStream_t st, HaloCtx halo = HaloCtx(), uint32_t block_index = 0, ChainCtx chain = ChainCtx(),
-                       uint32_t *n_strips_out = nullptr)
+                       cudaStream_t st, ChainCtx chain)
 {
 #define CGL_TB_CASE(KK) \
-    case KK: return launch_tb<KK, HALO>(in, out, rows, cols, wrap_rows, st, halo, block_index, chain, n_strips_out)
+    case KK: return launch_tb<KK>(in, out, rows, cols, wrap_rows, st, chain)
     switch (k) {
-        CGL_TB_CASE(1); CGL_TB_CASE(2); CGL_TB_CASE(3); CGL_TB_CASE(4);
+        CGL_TB_CASE(2); CGL_TB_CASE(3); CGL_TB_CASE(4);
         CGL_TB_CASE(6); CGL_TB_CASE(8); CGL_TB_CASE(12); CGL_TB_CASE(16);
     }
 #undef CGL_TB_CASE
@@ -612,30 +489,12 @@ extern "C" int cgl_life_run(uint32_t *buf_a, uint32_t *buf_b, uint32_t rows, uin
     uint32_t chained = 0;                 // launches of the current chain so far
     while (left > 0) {
         int step = 1;
-        if (tiled && (k == 4 || k == 8 || k == 16) && left >= 2 * k && !g_fault_next_chain) {
-            // the bulk of the run in ONE cooperative launch: a warp keeps its strip for all sub-steps and
-            // synchronises with its neighbour strips only (cgl_life_persist.cu)
-            const uint32_t n_sub = left / k;
-            const int rc = life_persist_run(src, dst, rows, cols, wrap_rows, n_sub, (int)k, st);
-            if (rc == 0) {
-                if (n_sub & 1u) { uint32_t *t = src; src = dst; dst = t; }
-                left -= n_sub * k;
-                prev_step = 0;
-                continue;
-            }
-            if (rc != -100) return rc;
-        }
         if (tiled && k > 1) {
             for (int s : sizes)
                 if ((uint32_t)s <= k && (uint32_t)s <= left) { step = s; break; }
         }
         int rc;
-        static int k1_tb = -1;              // CGL_LIFE_K1=tb: single generations through the pipeline kernel too (tuning)
-        if (k1_tb < 0) {
-            const char *e = getenv("CGL_LIFE_K1");
-            k1_tb = (e && e[0] == 't') ? 1 : 0;
-        }
-        if (step == 1 && !(k1_tb && tiled)) {
+        if (step == 1) {
             rc = cgl_life_step(src, dst, 1, rows, cols, wrap_rows, nullptr, stream);
             prev_step = 0;
         } else {
@@ -648,7 +507,7 @@ extern "C" int cgl_life_run(uint32_t *buf_a, uint32_t *buf_b, uint32_t rows, uin
                 }
                 chain = ChainCtx{token_buf, chained, token_cap};
             }
-            rc = tb_dispatch<false>(step, src, dst, rows, cols, wrap_rows, st, HaloCtx(), 0, chain);
+            rc = tb_dispatch(step, src, dst, rows, cols, wrap_rows, st, chain);
             prev_step = step;
             ++chained;
         }
@@ -705,12 +564,11 @@ extern "C" int cgl_life_tune(uint32_t *buf_a, uint32_t *buf_b, uint32_t rows, ui
         // time 4 launches chained like cgl_life_run chains them (all a -> b: every launch writes the same
         // values, so re-running a strip early is harmless); the first one doubles as warm-up
         if (token_buf) CGL_CUDA(cudaMemsetAsync(token_buf, 0, (size_t)token_cap * 4, st));
-        int rc = tb_dispatch<false>(kk, buf_a, buf_b, rows, cols, wrap_rows, st, HaloCtx(), 0, ChainCtx{token_buf, 0, token_cap});
+        int rc = tb_dispatch(kk, buf_a, buf_b, rows, cols, wrap_rows, st, ChainCtx{token_buf, 0, token_cap});
         if (rc) return rc;
         CGL_CUDA(cudaEventRecord(e0, st));
         for (uint32_t rep = 1; rep <= 4; ++rep)
-            if ((rc = tb_dispatch<false>(kk, buf_a, buf_b, rows, cols, wrap_rows, st, HaloCtx(), 0,
-                                         ChainCtx{token_buf, rep, token_cap})))
+            if ((rc = tb_dispatch(kk, buf_a, buf_b, rows, cols, wrap_rows, st, ChainCtx{token_buf, rep, token_cap})))
                 return rc;
         CGL_CUDA(cudaEventRecord(e1, st));
         CGL_CUDA(cudaEventSynchronize(e1));
@@ -723,34 +581,4 @@ extern "C" int cgl_life_tune(uint32_t *buf_a, uint32_t *buf_b, uint32_t rows, ui
     cudaEventDestroy(e1);
     if (best == 0) --g_n_tuned;
     return 0;
-}
-
-// One band block: `gens` generations (a k with a kernel instance: 1,2,3,4,6,8,12,16; gens <= ghost) of a
-// row band that carries `ghost` ghost rows above and below its owned rows, fused with the halo
-// exchange for the NEXT block (see HaloCtx).  in/out: this rank's band buffers (buf_rows x cols);
-// peer_*_out: the ring neighbours' OUTPUT buffers of the same block (peer-mapped); peer_*_sig: their
-// arrival counters {from_above, from_below}; my_ctr: my own two counters; block_index: 1, 2, ...
-extern "C" int cgl_life_band_block(const uint32_t *in, uint32_t *out, uint32_t buf_rows, uint32_t cols,
-                                   uint32_t ghost, uint32_t gens, uint32_t *peer_up_out, uint32_t *peer_dn_out,
-                                   uint32_t *peer_up_ctr, uint32_t *peer_dn_ctr, const uint32_t *my_ctr,
-                                   uint32_t block_index, cgl_stream_t stream)
-{
-    CGL_REQUIRE(in && out && in != out && peer_up_out && peer_dn_out && peer_up_ctr && peer_dn_ctr && my_ctr,
-                CGL_E_BADARG, "cgl_life_band_block: null pointer");
-    CGL_REQUIRE(cols % 32 == 0 && cols >= 32 * TB_COLS && ghost >= 1 && gens >= 1 && gens <= ghost &&
-                buf_rows > 4 * ghost && block_index >= 1, CGL_E_BADARG, "cgl_life_band_block: bad shape");
-    const uint32_t W = cols / 32;
-    HaloCtx hc;
-    hc.store_lo = ghost;
-    hc.store_hi = buf_rows - ghost;
-    hc.depth = ghost;
-    // my first owned rows -> the upper neighbour's bottom ghost rows; my last owned rows -> the lower one's top ghosts
-    hc.push_up = peer_up_out + (uint64_t)(buf_rows - ghost) * W;
-    hc.push_dn = peer_dn_out;
-    hc.sig_up = peer_up_ctr + 1;          // I am the upper neighbour's "from below"
-    hc.sig_dn = peer_dn_ctr + 0;          // and the lower neighbour's "from above"
-    hc.wait_up = my_ctr + 0;
-    hc.wait_dn = my_ctr + 1;
-    hc.wait_up_target = hc.wait_dn_target = 0;
-    return tb_dispatch<true>((int)gens, in, out, buf_rows, cols, 0, as_stream(stream), hc, block_index);
 }

@@ -28,7 +28,7 @@
 extern "C" {
 #endif
 
-#define CGL_B200_ABI_VERSION 1
+#define CGL_B200_ABI_VERSION 2
 
 #define CGL_E_BADARG   (-1)   /* null pointer / zero size / unsupported shape */
 #define CGL_E_BADINDEX (-2)   /* toggle index outside [0, size] (host-buffer entry points only) */
@@ -305,9 +305,8 @@ int cgl_life_step(const uint32_t *world_in_dev, uint32_t *world_out_dev, uint64_
                   cgl_stream_t stream);
 
 /* `gens` generations of ONE (rows x cols) grid, ping-ponging between buf_a (input) and buf_b,
- * `k` generations per HBM pass (temporal blocking in registers; k = 1 streams).  For k = 4, 8, 16 the bulk of the
- * run is ONE cooperative launch in which a warp keeps its strip for all passes and waits only for its neighbour
- * strips (cgl_life_persist.cu); otherwise one launch per pass, chained strip by strip.
+ * `k` generations per HBM pass (temporal blocking in registers; k = 1 streams): one launch per pass, chained strip
+ * by strip.
  * *result_in_a_out = 1 if the final state is in buf_a else 0.  The blocked kernels need cols % 32 == 0 and
  * cols >= 960; other shapes fall back to cgl_life_step per generation. */
 int cgl_life_run(uint32_t *buf_a_dev, uint32_t *buf_b_dev, uint32_t rows, uint32_t cols,
@@ -402,59 +401,15 @@ int cgl_ipc_get_handle(void *dev_ptr, uint8_t handle_out[64]);
 int cgl_ipc_open_handle(const uint8_t handle[64], void **dev_ptr_out);
 int cgl_ipc_close_handle(void *dev_ptr);
 
-/* Push `n_words` from a local buffer into a peer-mapped buffer and then publish `seq` to the
- * peer's flag word (release semantics), in one kernel; the peer waits with cgl_halo_wait. */
-int cgl_halo_push(const uint32_t *src_dev, uint32_t *peer_dst_dev, uint64_t n_words,
-                  uint32_t *peer_flag_dev, uint32_t seq, cgl_stream_t stream);
-/* Block the stream until *flag_dev >= seq (written by a peer GPU). */
-int cgl_halo_wait(const uint32_t *flag_dev, uint32_t seq, cgl_stream_t stream);
-/* The whole exchange of one rank in ONE launch (2 CTAs: one per ring neighbour): push my top rows
+/* The whole exchange of one rank in ONE launch (16 CTAs: 8 per ring neighbour): push my top rows
  * to the upper neighbour's landing slot and my bottom rows to the lower one's, publish `seq`, wait
- * for their strips of the same block and move them into my ghost rows. */
+ * for their strips of the same block and move them into my ghost rows.  A rank may be both of its own
+ * neighbours (a ring of one): its up-side CTAs then wait for the down-side CTAs of the same launch. */
 int cgl_halo_exchange(const uint32_t *top_src_dev, const uint32_t *bot_src_dev, uint32_t *peer_up_landing,
                       uint32_t *peer_dn_landing, uint32_t *peer_up_flag, uint32_t *peer_dn_flag,
                       const uint32_t *my_landing_up, const uint32_t *my_landing_dn, const uint32_t *my_flag_up,
                       const uint32_t *my_flag_dn, uint32_t *ghost_up_dev, uint32_t *ghost_dn_dev,
                       uint64_t n_words, uint32_t seq, cgl_stream_t stream);
-/* Same wait, then copy n_words from the landing zone `src_dev` into the ghost rows `dst_dev`. */
-int cgl_halo_wait_copy(const uint32_t *flag_dev, uint32_t seq, const uint32_t *src_dev, uint32_t *dst_dev,
-                       uint64_t n_words, cgl_stream_t stream);
-/* One row-band block with the halo exchange FUSED into the generation kernel (multi-GPU life mode).
- * The band buffer holds `ghost` ghost rows, the owned rows, `ghost` ghost rows.  Runs `gens`
- * (<= ghost; 1,2,3,4,6,8,12 or 16) generations in -> out in one launch; the kernel writes this
- * rank's first/last `ghost` owned rows straight into the ring neighbours' OUTPUT buffers
- * (peer_up_out / peer_dn_out: CUDA-IPC mapped, same layout) and bumps their arrival counters
- * (peer_*_ctr: uint32[2] = {from_above, from_below}); strips that read ghost rows first wait on
- * my_ctr until both neighbours completed block_index - 1.  block_index = 1 for the first block after
- * the ghosts were filled by a plain exchange (counters zeroed), then 2, 3, ...  No extra launch, no
- * host synchronisation, interior strips never wait. */
-int cgl_life_band_block(const uint32_t *in_dev, uint32_t *out_dev, uint32_t buf_rows, uint32_t cols,
-                        uint32_t ghost, uint32_t gens, uint32_t *peer_up_out, uint32_t *peer_dn_out,
-                        uint32_t *peer_up_ctr, uint32_t *peer_dn_ctr, const uint32_t *my_ctr,
-                        uint32_t block_index, cgl_stream_t stream);
-
-/* Row-band run with the halo exchange INSIDE the kernel (the default multi-GPU path of life mode): n_sub sub-steps
- * of k generations (k = 4, 8 or 16; ghost a multiple of k) over this rank's band buffers (ghost rows, owned rows,
- * ghost rows; buf_a holds the current state, the result is in buf_a if n_sub is even, else in buf_b) in ONE
- * cooperative launch -- a warp keeps its strip of rows for the whole call and waits only for its neighbour strips.
- * Every ghost / k sub-steps (a "block") and after the last sub-step, the strips that own the first / last `ghost`
- * owned rows store them into the ring neighbours' landing zones (peer_*_landing[slot], CUDA-IPC mapped, ghost x
- * cols/32 words each, slot = block & 1) and bump their arrival counters (peer_*_ctr); at the start of a block the
- * strips that read ghost rows wait on my_ctr_* and copy what they will read from my_landing_*[slot] into the
- * band buffer.  Interior strips never wait for another GPU.
- *   block_index   blocks (= pushes) consumed by earlier calls since the counters were zeroed; the caller adds
- *                 ceil(n_sub / (ghost / k)) after each call.
- *   initial_push  1 on a fresh grid (counters zeroed, block_index 0): the edge rows of buf_a are pushed before the
- *                 first sub-step.  With n_sub = 0 the call only pushes.
- * Bounded waits: a neighbour that never delivers raises alarm word 3, the kernel stores nothing further and ends.
- * cgl_life_band_run_supported: 1 if a band of this shape fits a cooperative launch on the current device. */
-int cgl_life_band_run(uint32_t *buf_a_dev, uint32_t *buf_b_dev, uint32_t buf_rows, uint32_t cols, uint32_t ghost,
-                      uint32_t k, uint32_t n_sub, uint32_t block_index, int initial_push,
-                      uint32_t *const peer_up_landing[2], uint32_t *const peer_dn_landing[2], uint32_t *peer_up_ctr,
-                      uint32_t *peer_dn_ctr, const uint32_t *const my_landing_up[2],
-                      const uint32_t *const my_landing_dn[2], const uint32_t *my_ctr_up, const uint32_t *my_ctr_dn,
-                      cgl_stream_t stream);
-int cgl_life_band_run_supported(uint32_t buf_rows, uint32_t cols, uint32_t k);
 
 /* Plain cudaMalloc'ed (zero-filled) device memory: IPC handles need whole allocations, which
  * a caching allocator's sub-blocks are not. */

@@ -18,7 +18,7 @@ def _declared_symbols():
     return sorted(set(re.findall(r"\b(cgl_[a-z0-9_]+)\s*\(", hdr)))
 
 
-def test_header_symbols_are_exported_and_bound():
+def test_header_symbols_are_exported_and_bound_at_abi_version_2():
     from cgl_b200 import native
     lib = native.load()
     syms = _declared_symbols()
@@ -27,7 +27,7 @@ def test_header_symbols_are_exported_and_bound():
         assert hasattr(lib, s), f"{s} declared in include/cgl_b200.h but not exported"
         assert s in native.SIGNATURES, f"{s} has no ctypes signature in native.py"
     assert sorted(native.SIGNATURES) == syms
-    assert lib.cgl_abi_version() == 1
+    assert lib.cgl_abi_version() == 2
     assert lib.cgl_words_per_row(1) == 1 and lib.cgl_words_per_row(32) == 1 and lib.cgl_words_per_row(33) == 2
     assert lib.cgl_env_step_is_fused(128) == 1 and lib.cgl_env_step_is_fused(100) == 0
     assert lib.cgl_env_step_launches(128, 1) == 1 and lib.cgl_env_step_launches(10, 1) == 3

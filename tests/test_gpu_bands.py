@@ -1,5 +1,6 @@
-"""GPU suite: row-band life mode.  One GPU: G emulated bands == plain torus == oracle.  With >= 2 GPUs:
-torchrun over NVLink with both exchange back ends, checked against the single-GPU torus."""
+"""GPU suite: row-band life mode.  One GPU: G emulated bands == plain torus == oracle, and a ring of one through the
+p2p exchange kernel.  With >= 2 GPUs: torchrun over NVLink with both exchange back ends, checked against the
+single-GPU torus."""
 import os
 import subprocess
 import sys
@@ -63,17 +64,17 @@ def test_randomize_is_partition_invariant(bands):
 
 @pytest.mark.parametrize("rows,cols,k,kk,runs", [(4096, 8192, 64, 8, (64, 128, 40)), (2048, 4096, 16, 8, (48, 16)),
                                                  (1024, 2048, 8, 4, (8, 24, 4)), (8192, 2048, 32, 16, (96,))])
-def test_ring_of_one_with_in_kernel_exchange_equals_torus(bands, rows, cols, k, kk, runs):
-    """exchange="persist" on ONE rank: the band keeps ghost rows and exchanges with itself through the landing zones
-    inside the cooperative kernel (cgl_life_band_run) -- every code path of the multi-GPU exchange on one GPU.
-    Several run() calls in a row (block counters carry over); compared with the plain torus and, for the small
-    shapes, the CPU oracle."""
+def test_ring_of_one_with_p2p_exchange_equals_torus(bands, rows, cols, k, kk, runs):
+    """exchange="p2p" on ONE rank: the band keeps ghost rows and exchanges with itself through the landing zones
+    (cgl_halo_exchange, its upper and lower neighbour being the rank itself) -- every code path of the default
+    multi-GPU exchange on one GPU.  Several run() calls in a row (block counters and landing slots carry over);
+    compared with the plain torus and, for the small shapes, the CPU oracle."""
     g = torch.Generator(device="cuda"); g.manual_seed(rows + k)
     words = torch.randint(-2 ** 31, 2 ** 31 - 1, (rows, cols // 32), dtype=torch.int32, device="cuda", generator=g)
     torus = bands.RowBandLife(rows, cols, k=k, kernel_k=kk)
     torus.set_owned(words)
-    with bands.RowBandLife(rows, cols, k=k, kernel_k=kk, exchange="persist") as ring:
-        assert ring.ghost == k and ring.exchange == "persist"
+    with bands.RowBandLife(rows, cols, k=k, kernel_k=kk, exchange="p2p") as ring:
+        assert ring.ghost == k and ring.exchange == "p2p"
         ring.set_owned(words)
         for gens in runs:
             ring.run(gens)
@@ -102,13 +103,13 @@ def test_all_pass_depths_agree(bands):
         assert torch.equal(o, outs[0])
 
 
-@pytest.mark.parametrize("exchange", ["persist", "fused", "p2p", "dist"])
+@pytest.mark.parametrize("exchange", ["p2p", "dist"])
 def test_two_gpu_bands_match_single_gpu(bands, exchange):
     if torch.cuda.device_count() < 2:
         pytest.skip("needs 2 GPUs")
     cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node", "2", "--master-addr",
            "127.0.0.1", "--master-port", "29533", os.path.join(ROOT, "tools", "run_bands.py"), "--rows", "4096", "--cols",
-           "8192", "--k", "8", "--gens", "48" if exchange == "persist" else "43", "--exchange", exchange, "--check"]
+           "8192", "--k", "8", "--gens", "43", "--exchange", exchange, "--check"]
     r = subprocess.run(cmd, capture_output=True, text=True, timeout=600)
     assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-2000:]
     assert '"ok": true' in r.stdout

@@ -372,12 +372,10 @@ print("variant ok")
 """
 
 
-@pytest.mark.parametrize("knobs", [{"CGL_ENV_IMPL": "tma", "CGL_ENV_TMA_THREADS": "256"},
-                                   {"CGL_ENV_IMPL": "tma", "CGL_ENV_TMA_THREADS": "128"},
-                                   {"CGL_ENV_PDL": "0"}, {"CGL_ENV_BYTES": "0"}, {"CGL_ENV_BYTES": "2"}])
+@pytest.mark.parametrize("knobs", [{"CGL_ENV_PDL": "0"}, {"CGL_ENV_BYTES": "0"}, {"CGL_ENV_BYTES": "2"}])
 def test_env_kernel_variants_vs_oracle(cgl, knobs):
-    """The persistent bulk-copy (cp.async.bulk + mbarrier) kernel, the non-PDL launch path, and -- on sides the fused
-    kernel does not take -- the one-launch byte-plane kernel against the three generic kernels it replaced."""
+    """The non-PDL launch path and -- on sides the fused kernel does not take -- the one-launch byte-plane kernel
+    against the three generic kernels it replaced."""
     import subprocess
     import sys
     from conftest import PKG

@@ -6,8 +6,8 @@ the edge of a small grid, bit-exact against the CPU oracle.
     launch), chained launches plus a remainder of smaller blocks; torus and open rows;
   * cgl_life_step at its kernel switch (cols 1920 / 4224 generic, 2048 / 4352 streaming) with 1..25 rows,
     1..200 envs, both row modes, with and without live counts;
-  * the opt-in life kernels, each forced through its environment knob in a subprocess (the knobs are read once per
-    process), a tuned strip length, and RowBandLife on a torus shorter than its kernel_k;
+  * the life kernels' tuning knobs, each forced in a subprocess (the knobs are read once per process), a tuned strip
+    length, and RowBandLife on a torus shorter than its kernel_k;
   * the env step at every side 1..300 (generic, byte-plane, fused and > 256 regimes, every side % 4 class), with
     the byte-plane kernel forced on and off, and both dead-cell rules of the CGL_action+ fork;
   * cgl_env_run on arbitrary int8 planes at parameter corners, fused and generic sides up to its side limit,
@@ -164,11 +164,7 @@ def variant_life_step():
 
 
 @pytest.mark.parametrize("knobs,fn", [
-    ({"CGL_TB_MODE": "0"}, "variant_life_run"),          # the skewed pipeline at K <= 12 (shared with the fused halo exchange)
-    ({"CGL_TB_MODE": "1"}, "variant_life_run"),          # the direct pipeline at K = 16
     ({"CGL_TB_CHAIN": "0"}, "variant_life_run"),
-    ({"CGL_LIFE_PERSIST": "1"}, "variant_life_run"),     # the cooperative kernel for k in {4, 8, 16}
-    ({"CGL_LIFE_K1": "tb"}, "variant_life_run"),
     ({"CGL_TB_ROWS": "19"}, "variant_life_run"),         # strips >= K, not a multiple of either unroll
     ({"CGL_LIFE_PF": "6"}, "variant_life_step"),
     ({"CGL_LIFE_MINB": "5"}, "variant_life_step"),

@@ -21,4 +21,4 @@ for _ in range(5):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record(); run(); e1.record(); torch.cuda.synchronize()
     ts.append(e0.elapsed_time(e1) / 512 * 1e3)
-print(json.dumps({"rpt": os.environ.get("CGL_TB_ROWS"), "k": k, "rows": rows, "persist": os.environ.get("CGL_LIFE_PERSIST", "1"), "us_per_gen": round(statistics.median(ts), 2)}))
+print(json.dumps({"rpt": os.environ.get("CGL_TB_ROWS"), "k": k, "rows": rows, "us_per_gen": round(statistics.median(ts), 2)}))

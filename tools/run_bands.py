@@ -25,7 +25,7 @@ ap.add_argument("--k", type=int, default=8)
 ap.add_argument("--gens", type=int, default=1000)
 ap.add_argument("--kernel-k", type=int, default=0, help="generations per launch (default min(k, 8))")
 ap.add_argument("--warmup", type=int, default=16)
-ap.add_argument("--exchange", default="persist", choices=["persist", "fused", "p2p", "dist"])
+ap.add_argument("--exchange", default="p2p", choices=["p2p", "dist"])
 ap.add_argument("--check", action="store_true")
 ap.add_argument("--seed", type=int, default=1)
 a = ap.parse_args()

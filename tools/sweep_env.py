@@ -46,7 +46,7 @@ for rep in range(3):
     e1.record(); torch.cuda.synchronize()
     gb = min(gb, e0.elapsed_time(e1) / (K // (2 * R) * 2 * R) * 1e3)
 bytes_step = 2.25 * B * side * side
-print(json.dumps({"impl": os.environ.get("CGL_ENV_IMPL", "fused"), "pdl": os.environ.get("CGL_ENV_PDL", "1"), "chained": os.environ.get("CGL_ENV_CHAINED", "1"), "thr": os.environ.get("CGL_ENV_TMA_THREADS"), "side": side,
+print(json.dumps({"pdl": os.environ.get("CGL_ENV_PDL", "1"), "chained": os.environ.get("CGL_ENV_CHAINED", "1"), "side": side,
                   "envs": B, "repl": R, "eager_us": round(best, 2), "host_launch_us": round(host, 2), "graph_us": round(gb, 2),
                   "frac_eager": round(bytes_step / (best * 1e-6) / 1e9 / 6543.4, 4),
                   "frac_graph": round(bytes_step / (gb * 1e-6) / 1e9 / 6543.4, 4)}))
