@@ -41,6 +41,16 @@ def _life_block(lib, a, b, rows, cols, wrap_rows, gens, k, stream) -> bool:
     return res.value == 1
 
 
+def _life_block_pop(lib, a, b, rows, cols, wrap_rows, gens, k, count_row0, count_rows, pop, stream) -> bool:
+    """_life_block that also writes pop (int64 [gens]): the live cells of rows [count_row0, count_row0 + count_rows)
+    after each generation (cgl_life_run_pop: counted in the k-blocked kernels, no extra pass over the grid).
+    Tests monkeypatch this for CPU runs."""
+    res = ctypes.c_int(-1)
+    native.check(lib.cgl_life_run_pop(native.dptr(a), native.dptr(b), rows, cols, wrap_rows, gens, k, count_row0,
+                                      count_rows, native.dptr(pop), ctypes.byref(res), stream), "cgl_life_run_pop")
+    return res.value == 1
+
+
 class _null:
     def __enter__(self):
         return self
@@ -212,9 +222,12 @@ class RowBandLife:
         raise ValueError(f"unknown exchange {self.exchange!r}")
 
     # ---------------------------------------------------------------- stepping
-    def run(self, gens: int) -> None:
-        """Advance `gens` generations (blocks of k generations between exchanges)."""
+    def run(self, gens: int, population: bool = False):
+        """Advance `gens` generations (blocks of k generations between exchanges).  With population=True, return
+        the global population after each generation of this call: int64 [gens] on this rank's device, the same
+        on every rank (one all_reduce per call)."""
         lib, st = self.lib, self._stream()
+        pop = torch.empty(gens, dtype=torch.int64, device=self.device) if population else None
         if self.device.type == "cuda" and not getattr(self, "_tuned", False):
             # measure the strip length of the k-blocked kernel for this band shape once (clobbers _b only)
             with torch.cuda.device(self.device):
@@ -224,21 +237,35 @@ class RowBandLife:
             self._tuned = True
         if self.G == 1 and not self._self_ring:   # plain torus: one call, k generations per launch
             with torch.cuda.device(self.device) if self.device.type == "cuda" else _null():
-                if not _life_block(lib, self._a, self._b, self.band_rows, self.cols, 1, gens, self.kernel_k, st):
+                if population:
+                    in_a = _life_block_pop(lib, self._a, self._b, self.band_rows, self.cols, 1, gens, self.kernel_k,
+                                           0, self.band_rows, pop, st)
+                else:
+                    in_a = _life_block(lib, self._a, self._b, self.band_rows, self.cols, 1, gens, self.kernel_k, st)
+                if not in_a:
                     self._a, self._b = self._b, self._a
             self.launches += -(-gens // self.kernel_k)
             self.generation += gens
-            return
+            return pop
         done = 0
         while done < gens:
             kb = min(self.k, gens - done)
             self._exchange()
             with torch.cuda.device(self.device) if self.device.type == "cuda" else _null():
-                if not _life_block(lib, self._a, self._b, self.buf_rows, self.cols, 0, kb, min(kb, self.kernel_k), st):
+                if population:      # this block's generations, counted over the owned rows of the band buffer
+                    in_a = _life_block_pop(lib, self._a, self._b, self.buf_rows, self.cols, 0, kb, min(kb, self.kernel_k),
+                                           self.ghost, self.band_rows, pop[done:done + kb], st)
+                else:
+                    in_a = _life_block(lib, self._a, self._b, self.buf_rows, self.cols, 0, kb, min(kb, self.kernel_k), st)
+                if not in_a:
                     self._a, self._b = self._b, self._a
             self.launches += -(-kb // self.kernel_k)
             done += kb
             self.generation += kb
+        if population and self.G > 1:
+            import torch.distributed as dist
+            dist.all_reduce(pop, group=self.group)
+        return pop
 
     # ---------------------------------------------------------------- global reductions
     def alive(self) -> int:
@@ -291,7 +318,10 @@ class LocalBands:
     def grid(self) -> torch.Tensor:
         return torch.cat([b.owned for b in self.bands], dim=0)
 
-    def run(self, gens: int) -> None:
+    def run(self, gens: int, population: bool = False):
+        """Advance every band `gens` generations; with population=True return the population of the whole grid
+        after each generation (int64 [gens], the bands' owned-row counts summed)."""
+        pops = [torch.empty(gens, dtype=torch.int64, device=b.device) for b in self.bands] if population else None
         done = 0
         while done < gens:
             kb = min(self.k, gens - done)
@@ -301,8 +331,14 @@ class LocalBands:
                 up, down = (r - 1) % self.G, (r + 1) % self.G
                 b._a[0:b.k * b.W] = bots[up]
                 b._a[(b.ghost + b.band_rows) * b.W:(b.ghost + b.band_rows + b.k) * b.W] = tops[down]
-            for b in self.bands:
-                if not _life_block(b.lib, b._a, b._b, b.buf_rows, b.cols, 0, kb, kb, b._stream()):
+            for r, b in enumerate(self.bands):
+                if population:
+                    in_a = _life_block_pop(b.lib, b._a, b._b, b.buf_rows, b.cols, 0, kb, kb, b.ghost, b.band_rows,
+                                           pops[r][done:done + kb], b._stream())
+                else:
+                    in_a = _life_block(b.lib, b._a, b._b, b.buf_rows, b.cols, 0, kb, kb, b._stream())
+                if not in_a:
                     b._a, b._b = b._b, b._a
                 b.generation += kb
             done += kb
+        return torch.stack(pops).sum(0) if population else None

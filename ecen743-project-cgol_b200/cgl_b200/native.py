@@ -54,6 +54,7 @@ SIGNATURES = {
     "cgl_env_step_launches": (_i, [_u32, _i]),
     "cgl_life_step": (_i, [_vp, _vp, _u64, _u32, _u32, _i, _vp, _vp]),
     "cgl_life_run": (_i, [_vp, _vp, _u32, _u32, _i, _u32, _u32, ctypes.POINTER(_i), _vp]),
+    "cgl_life_run_pop": (_i, [_vp, _vp, _u32, _u32, _i, _u32, _u32, _u32, _u32, _vp, ctypes.POINTER(_i), _vp]),
     "cgl_life_tune": (_i, [_vp, _vp, _u32, _u32, _i, _u32, _vp]),
     "cgl_reward": (_i, [_vp, _u64, _u64, _vp, _vp]),
     "cgl_alive": (_i, [_vp, _u64, _u64, _vp, _vp]),

@@ -57,10 +57,52 @@ constexpr int TB_COLS = 30;             // valid word-columns per warp
 
 constexpr int TB_THREADS = 128;
 
+// Population trace of a counted launch (cgl_life_run_pop): pop[g] += live cells of generation g + 1 of the launch in
+// the rows of [row0, row1) that the strip owns, counted by the lanes that store.  A thread keeps two levels' counts
+// per register as 16-bit halves (K/2 registers instead of K), so a counted launch keeps its strips at most
+// TB_POP_MAX_ROWS rows long: at most 2047 x 32 < 2^16 cells per thread and level.
+struct PopCtx { unsigned long long *pop; uint32_t row0, row1; };
+constexpr uint32_t TB_POP_MAX_ROWS = 2047;
+
+// Add the popcount of level g's output row y to the thread's count if the row lies in the strip's part of the count
+// window: t = row - max(r0, row0) < cn.  CNT 0: no count (the uncounted kernels).
+// Measured alternatives, none kept (ptxas -v, life_tb2_kernel<8>): a separate steady-state loop without the row test
+// for strips inside the window takes 142-148 registers (three loop nests), shared-memory counters 163, and a
+// __launch_bounds__ minimum of 5 CTAs spills; the row test in every step costs 108 registers (4 CTAs per SM).
+template <int CNT, int K>
+__device__ __forceinline__ void tally(uint32_t (&acc)[(K + 1) / 2], int g, uint32_t y, uint32_t t, uint32_t cn)
+{
+    if constexpr (CNT == 1) acc[g >> 1] += (t < cn ? (uint32_t)__popc(y) : 0u) << (16 * (g & 1));
+}
+
+// Strip-uniform set-up of a counted launch: the row test of level g at step s is (uint32_t)(s - m g + cbase) < cn,
+// where level g emits row r0 - K + s - m g - 1 (m = 1 direct, 2 skewed).  Every count of a padding warp or of a strip
+// whose token wait expired is dropped by pop_flush (store_ok).
+struct PopWin { int cbase; uint32_t cn; };
+__device__ __forceinline__ PopWin pop_window(const PopCtx &pc, int r0, int r1, int K)
+{
+    const int lo = r0 > (int)pc.row0 ? r0 : (int)pc.row0;
+    const int hi = r1 < (int)pc.row1 ? r1 : (int)pc.row1;
+    return PopWin{r0 - K - 1 - lo, hi > lo ? (uint32_t)(hi - lo) : 0u};
+}
+
+// End of a counted strip: the storing lanes' counts of each level, summed over the warp, go to pop[g].
 template <int K>
+__device__ __forceinline__ void pop_flush(const uint32_t (&acc)[(K + 1) / 2], const PopCtx &pc, bool store_ok, uint32_t lane)
+{
+#pragma unroll
+    for (int g = 0; g < K; ++g) {
+        uint32_t v = store_ok ? (acc[g >> 1] >> (16 * (g & 1))) & 0xffffu : 0u;
+        v = __reduce_add_sync(0xffffffffu, v);
+        if (lane == 0 && v != 0) atomicAdd(pc.pop + g, (unsigned long long)v);
+    }
+}
+
+template <int K, bool POP>
 __global__ void __launch_bounds__(TB_THREADS)
 life_tb_kernel(const uint32_t *__restrict__ in, uint32_t *__restrict__ out, uint32_t rows, uint32_t W,
-               uint32_t rpt, int wrap_rows, uint32_t n_cgroups, uint32_t n_rblocks, const ChainCtx chain)
+               uint32_t rpt, int wrap_rows, uint32_t n_cgroups, uint32_t n_rblocks, const ChainCtx chain,
+               const PopCtx popc)
 {
     // Warps are numbered along the row first (column group fastest).  No early exit: padding warps
     // redo the last strip with stores off and the loop trip count is the same for every warp, so
@@ -129,6 +171,9 @@ life_tb_kernel(const uint32_t *__restrict__ in, uint32_t *__restrict__ out, uint
         win[g] = Win{0, 0, 0, 0, 0, 0, 0};
         pend[g] = 0;
     }
+    uint32_t acc[(K + 1) / 2] = {};
+    const PopWin pw = POP ? pop_window(popc, r0, r1, K) : PopWin{0, 0};
+    constexpr int CNT = POP ? 1 : 0;
 
     for (int s0 = 0; s0 < n_steps; s0 += TB_UNROLL) {
         uint32_t raw[TB_UNROLL];
@@ -155,6 +200,7 @@ life_tb_kernel(const uint32_t *__restrict__ in, uint32_t *__restrict__ out, uint
                 pend[g] = life_rule(up, mid, d, win[g].mc);
                 win[g].us0 = win[g].ms0; win[g].us1 = win[g].ms1;
                 win[g].ms0 = d.s0; win[g].ms1 = d.s1; win[g].mt0 = d.t0; win[g].mt1 = d.t1; win[g].mc = x;
+                tally<CNT, K>(acc, g, pend[g], (uint32_t)(s0 + u - 2 * g + pw.cbase), pw.cn);     // row r0 - K + s - 2g - 1
             }
             // row r0 + so of generation K has just left level K
             const uint32_t so = (uint32_t)(s0 + u - (3 * K - 1));
@@ -162,6 +208,7 @@ life_tb_kernel(const uint32_t *__restrict__ in, uint32_t *__restrict__ out, uint
             st_if_lt(op + ro * W, pend[K - 1], store_ok, so, out_rows);
         }
     }
+    if constexpr (POP) pop_flush<K>(acc, popc, store_ok, lane);
     if (chain.tokens != nullptr) {
         __threadfence();                             // this strip's rows are visible device-wide ...
         __syncwarp();
@@ -186,9 +233,10 @@ life_tb_kernel(const uint32_t *__restrict__ in, uint32_t *__restrict__ out, uint
 // SM), 3 steps with prefetch 15.88 / 115.2, 4 steps without 21.2 / 151.
 constexpr int TB2_UNROLL = 4;
 
-template <int K, bool PRO>
+template <int K, bool PRO, int CNT>
 __device__ __forceinline__ void tb2_block(const uint32_t (&raw)[TB2_UNROLL], Win (&win)[K], int s0, uint32_t *op, uint32_t r0W,
-                                          uint32_t W, bool store_ok, uint32_t out_rows)
+                                          uint32_t W, bool store_ok, uint32_t out_rows, uint32_t (&acc)[(K + 1) / 2],
+                                          const PopWin &pw)
 {
 #pragma unroll
     for (int u = 0; u < TB2_UNROLL; ++u) {
@@ -208,6 +256,7 @@ __device__ __forceinline__ void tb2_block(const uint32_t (&raw)[TB2_UNROLL], Win
             win[g].us0 = win[g].ms0; win[g].us1 = win[g].ms1;
             win[g].ms0 = d.s0; win[g].ms1 = d.s1; win[g].mt0 = d.t0; win[g].mt1 = d.t1; win[g].mc = x;
             x = y;
+            tally<CNT, K>(acc, g, y, (uint32_t)(s0 + u - g + pw.cbase), pw.cn);     // row r0 - K + s0 + u - g - 1
         }
         // row r0 + so of generation K has just left level K
         const uint32_t so = (uint32_t)(s0 + u - 2 * K);
@@ -215,10 +264,10 @@ __device__ __forceinline__ void tb2_block(const uint32_t (&raw)[TB2_UNROLL], Win
     }
 }
 
-template <int K>
+template <int K, bool POP>
 __global__ void __launch_bounds__(TB_THREADS)
 life_tb2_kernel(const uint32_t *__restrict__ in, uint32_t *__restrict__ out, uint32_t rows, uint32_t W, uint32_t rpt,
-                int wrap_rows, uint32_t n_cgroups, uint32_t n_rblocks, const ChainCtx chain)
+                int wrap_rows, uint32_t n_cgroups, uint32_t n_rblocks, const ChainCtx chain, const PopCtx popc)
 {
     const uint32_t lane = threadIdx.x & 31;
     const uint32_t warp = blockIdx.x * (TB_THREADS / 32) + (threadIdx.x >> 5);
@@ -284,23 +333,28 @@ life_tb2_kernel(const uint32_t *__restrict__ in, uint32_t *__restrict__ out, uin
         rw += TB2_UNROLL;
         rw = rw >= irows ? rw - irows : rw;
     };
+    uint32_t acc[(K + 1) / 2] = {};
+    const PopWin pw = POP ? pop_window(popc, r0, r1, K) : PopWin{0, 0};
+
     constexpr int PRO_STEPS = (2 * K + TB2_UNROLL - 1) / TB2_UNROLL * TB2_UNROLL;   // start-up: levels come in one by one
+    constexpr int CNT = POP ? 1 : 0;
     int s0 = 0;
     // software pipeline: the rows of block i + 1 are requested before block i is computed (two row buffers)
     uint32_t ra[TB2_UNROLL], rbuf[TB2_UNROLL];
     load(ra, 0);
     for (; s0 < PRO_STEPS && s0 < n_steps; s0 += 2 * TB2_UNROLL) {
         load(rbuf, s0 + TB2_UNROLL);
-        tb2_block<K, true>(ra, win, s0, op, r0W, W, store_ok, out_rows);
+        tb2_block<K, true, CNT>(ra, win, s0, op, r0W, W, store_ok, out_rows, acc, pw);
         load(ra, s0 + 2 * TB2_UNROLL);
-        tb2_block<K, true>(rbuf, win, s0 + TB2_UNROLL, op, r0W, W, store_ok, out_rows);
+        tb2_block<K, true, CNT>(rbuf, win, s0 + TB2_UNROLL, op, r0W, W, store_ok, out_rows, acc, pw);
     }
     for (; s0 < n_steps; s0 += 2 * TB2_UNROLL) {
         load(rbuf, s0 + TB2_UNROLL);
-        tb2_block<K, false>(ra, win, s0, op, r0W, W, store_ok, out_rows);
+        tb2_block<K, false, CNT>(ra, win, s0, op, r0W, W, store_ok, out_rows, acc, pw);
         load(ra, s0 + 2 * TB2_UNROLL);
-        tb2_block<K, false>(rbuf, win, s0 + TB2_UNROLL, op, r0W, W, store_ok, out_rows);
+        tb2_block<K, false, CNT>(rbuf, win, s0 + TB2_UNROLL, op, r0W, W, store_ok, out_rows, acc, pw);
     }
+    if constexpr (POP) pop_flush<K>(acc, popc, store_ok, lane);
     if (chain.tokens != nullptr) {
         __threadfence();
         __syncwarp();
@@ -359,25 +413,26 @@ static uint32_t tuned_rows(uint32_t rows, uint32_t W, int K)
     return 0;
 }
 
-template <int K>
+template <int K, bool POP>
 static int launch_tb(const uint32_t *in, uint32_t *out, uint32_t rows, uint32_t cols, int wrap_rows,
-                     cudaStream_t st, ChainCtx chain)
+                     cudaStream_t st, ChainCtx chain, PopCtx popc)
 {
-    static int rpt_knob = -1, occ = 0;   // CGL_TB_ROWS overrides the strip length (tuning)
+    static int rpt_knob = -1, occ = 0;   // per (K, POP): CGL_TB_ROWS overrides the strip length (tuning)
     if (rpt_knob < 0) {
         const char *e = getenv("CGL_TB_ROWS");
         rpt_knob = e ? atoi(e) : 0;
         int n = 0;
         if constexpr (tb_direct(K))
-            CGL_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, life_tb2_kernel<K>, TB_THREADS, 0));
+            CGL_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, life_tb2_kernel<K, POP>, TB_THREADS, 0));
         else
-            CGL_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, life_tb_kernel<K>, TB_THREADS, 0));
+            CGL_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, life_tb_kernel<K, POP>, TB_THREADS, 0));
         occ = n > 0 ? n : 1;
     }
     const uint32_t W = cols / 32;
     const uint32_t n_cgroups = (W + TB_COLS - 1) / TB_COLS;
     uint32_t rpt = rpt_knob > 0 ? (uint32_t)rpt_knob : tuned_rows(rows, W, K);
     if (rpt == 0) rpt = tb_pick_rows(rows, n_cgroups, K, (uint64_t)sm_count() * occ);
+    if (POP && rpt > TB_POP_MAX_ROWS) rpt = TB_POP_MAX_ROWS;     // 16-bit counts per thread (see PopCtx)
     if (rpt > rows) rpt = rows;
     const uint32_t n_rblocks = (rows + rpt - 1) / rpt;
     const uint64_t blocks = ((uint64_t)n_cgroups * n_rblocks + TB_THREADS / 32 - 1) / (TB_THREADS / 32);
@@ -395,17 +450,21 @@ static int launch_tb(const uint32_t *in, uint32_t *out, uint32_t rows, uint32_t 
     cfg.attrs = attr;
     cfg.numAttrs = (chain.tokens != nullptr && chain.want > 0) ? 1 : 0;        // the first launch of a run waits normally
     if constexpr (tb_direct(K))
-        CGL_CUDA(cudaLaunchKernelEx(&cfg, life_tb2_kernel<K>, in, out, rows, W, rpt, wrap_rows, n_cgroups, n_rblocks, chain));
+        CGL_CUDA(cudaLaunchKernelEx(&cfg, life_tb2_kernel<K, POP>, in, out, rows, W, rpt, wrap_rows, n_cgroups, n_rblocks, chain,
+                                    popc));
     else
-        CGL_CUDA(cudaLaunchKernelEx(&cfg, life_tb_kernel<K>, in, out, rows, W, rpt, wrap_rows, n_cgroups, n_rblocks, chain));
+        CGL_CUDA(cudaLaunchKernelEx(&cfg, life_tb_kernel<K, POP>, in, out, rows, W, rpt, wrap_rows, n_cgroups, n_rblocks, chain,
+                                    popc));
     return 0;
 }
 
+// popc.pop == nullptr: the uncounted kernels.
 static int tb_dispatch(int k, const uint32_t *in, uint32_t *out, uint32_t rows, uint32_t cols, int wrap_rows,
-                       cudaStream_t st, ChainCtx chain)
+                       cudaStream_t st, ChainCtx chain, PopCtx popc)
 {
-#define CGL_TB_CASE(KK) \
-    case KK: return launch_tb<KK>(in, out, rows, cols, wrap_rows, st, chain)
+#define CGL_TB_CASE(KK)                                                                     \
+    case KK: return popc.pop ? launch_tb<KK, true>(in, out, rows, cols, wrap_rows, st, chain, popc) \
+                             : launch_tb<KK, false>(in, out, rows, cols, wrap_rows, st, chain, popc)
     switch (k) {
         CGL_TB_CASE(2); CGL_TB_CASE(3); CGL_TB_CASE(4);
         CGL_TB_CASE(6); CGL_TB_CASE(8); CGL_TB_CASE(12); CGL_TB_CASE(16);
@@ -448,6 +507,37 @@ static uint32_t *chain_tokens(cudaStream_t st, uint32_t rows, uint32_t cols, uin
     return tb->p;
 }
 
+// pop += live cells of the n_words words starting at w (rows of W words; the last word of a row keeps the bits of
+// tail_mask): the population of a count window after a generation that ran outside the k-blocked kernels.
+__global__ void window_pop_kernel(const uint32_t *__restrict__ w, uint64_t n_words, uint32_t W, uint32_t tail_mask,
+                                  unsigned long long *__restrict__ pop)
+{
+    unsigned acc = 0;
+    const uint64_t nthr = (uint64_t)gridDim.x * blockDim.x;
+    for (uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x; i < n_words; i += nthr) {
+        uint32_t v = __ldg(w + i);
+        if (i % W == W - 1) v &= tail_mask;
+        acc += __popc(v);
+    }
+    acc = __reduce_add_sync(0xffffffffu, acc);
+    if ((threadIdx.x & 31) == 0 && acc != 0) atomicAdd(pop, (unsigned long long)acc);
+}
+
+static int window_pop(const uint32_t *grid, uint32_t cols, uint32_t row0, uint32_t n_rows, unsigned long long *pop,
+                      cudaStream_t st)
+{
+    const uint32_t W = (cols + 31) / 32;
+    const uint64_t n_words = (uint64_t)n_rows * W;
+    const uint32_t tail_mask = cols % 32 ? (1u << (cols % 32)) - 1u : 0xffffffffu;
+    const unsigned threads = 256;
+    uint64_t bx = (n_words + threads * 4 - 1) / (threads * 4);
+    const uint64_t cap = (uint64_t)sm_count() * 8;
+    bx = bx < 1 ? 1 : (bx > cap ? cap : bx);
+    window_pop_kernel<<<(unsigned)bx, threads, 0, st>>>(grid + (uint64_t)row0 * W, n_words, W, tail_mask, pop);
+    CGL_LAUNCH_CHECK();
+    return 0;
+}
+
 CGL_DEFINE_TU_HOOKS(life_tb)
 
 }  // namespace cgl
@@ -471,13 +561,15 @@ extern "C" int cgl_test_fault(int which)
 // With wrap_rows = 0 the k rows next to each open edge are a ghost zone: their contents after a
 // k-blocked launch are unspecified (they differ from k single steps); every row at least k rows
 // away from an open edge is exact.
-extern "C" int cgl_life_run(uint32_t *buf_a, uint32_t *buf_b, uint32_t rows, uint32_t cols,
-                            int wrap_rows, uint32_t gens, uint32_t k, int *result_in_a_out,
-                            cgl_stream_t stream)
+// pop != nullptr (cgl_life_run_pop): pop[i] += live cells of rows [row0, row0 + n_rows) after generation i + 1.
+static int life_run(uint32_t *buf_a, uint32_t *buf_b, uint32_t rows, uint32_t cols, int wrap_rows, uint32_t gens,
+                    uint32_t k, int *result_in_a_out, cgl_stream_t stream, unsigned long long *pop, uint32_t row0,
+                    uint32_t n_rows)
 {
     CGL_REQUIRE(buf_a && buf_b && rows && cols && buf_a != buf_b, CGL_E_BADARG, "cgl_life_run: bad argument");
     CGL_REQUIRE(k >= 1 && k <= 16, CGL_E_BADARG, "cgl_life_run: k must be in 1..16");
     cudaStream_t st = as_stream(stream);
+    if (pop != nullptr && gens > 0) CGL_CUDA(cudaMemsetAsync(pop, 0, (size_t)gens * sizeof(*pop), st));
     static const int sizes[] = {16, 12, 8, 6, 4, 3, 2, 1};
     uint32_t *src = buf_a, *dst = buf_b;
     uint32_t left = gens;
@@ -496,6 +588,7 @@ extern "C" int cgl_life_run(uint32_t *buf_a, uint32_t *buf_b, uint32_t rows, uin
         int rc;
         if (step == 1) {
             rc = cgl_life_step(src, dst, 1, rows, cols, wrap_rows, nullptr, stream);
+            if (rc == 0 && pop != nullptr) rc = window_pop(dst, cols, row0, n_rows, pop + (gens - left), st);
             prev_step = 0;
         } else {
             ChainCtx chain{nullptr, 0, 0};
@@ -507,7 +600,8 @@ extern "C" int cgl_life_run(uint32_t *buf_a, uint32_t *buf_b, uint32_t rows, uin
                 }
                 chain = ChainCtx{token_buf, chained, token_cap};
             }
-            rc = tb_dispatch(step, src, dst, rows, cols, wrap_rows, st, chain);
+            const PopCtx popc{pop != nullptr ? pop + (gens - left) : nullptr, row0, row0 + n_rows};
+            rc = tb_dispatch(step, src, dst, rows, cols, wrap_rows, st, chain, popc);
             prev_step = step;
             ++chained;
         }
@@ -517,6 +611,27 @@ extern "C" int cgl_life_run(uint32_t *buf_a, uint32_t *buf_b, uint32_t rows, uin
     }
     if (result_in_a_out) *result_in_a_out = (src == buf_a) ? 1 : 0;
     return 0;
+}
+
+extern "C" int cgl_life_run(uint32_t *buf_a, uint32_t *buf_b, uint32_t rows, uint32_t cols,
+                            int wrap_rows, uint32_t gens, uint32_t k, int *result_in_a_out,
+                            cgl_stream_t stream)
+{
+    return life_run(buf_a, buf_b, rows, cols, wrap_rows, gens, k, result_in_a_out, stream, nullptr, 0, 0);
+}
+
+extern "C" int cgl_life_run_pop(uint32_t *buf_a, uint32_t *buf_b, uint32_t rows, uint32_t cols, int wrap_rows,
+                                uint32_t gens, uint32_t k, uint32_t count_row0, uint32_t count_rows, uint64_t *pop_out,
+                                int *result_in_a_out, cgl_stream_t stream)
+{
+    CGL_REQUIRE(pop_out != nullptr, CGL_E_BADARG, "cgl_life_run_pop: pop_out_dev is NULL");
+    CGL_REQUIRE(count_rows > 0, CGL_E_BADARG, "cgl_life_run_pop: count_rows must be at least 1");
+    CGL_REQUIRE((uint64_t)count_row0 + count_rows <= rows, CGL_E_BADARG,
+                "cgl_life_run_pop: count window [%u, %u + %u) is not inside the %u rows", count_row0, count_row0,
+                count_rows, rows);
+    static_assert(sizeof(unsigned long long) == sizeof(uint64_t), "pop_out is uint64");
+    return life_run(buf_a, buf_b, rows, cols, wrap_rows, gens, k, result_in_a_out, stream,
+                    reinterpret_cast<unsigned long long *>(pop_out), count_row0, count_rows);
 }
 
 // Measure the strip length for this shape on the caller's buffers (buf_b is clobbered) and remember
@@ -540,7 +655,7 @@ extern "C" int cgl_life_tune(uint32_t *buf_a, uint32_t *buf_b, uint32_t rows, ui
     int n_cand = 11;
     {
         int occ = 0;
-        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, life_tb2_kernel<8>, TB_THREADS, 0) != cudaSuccess || occ <= 0) {
+        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, life_tb2_kernel<8, false>, TB_THREADS, 0) != cudaSuccess || occ <= 0) {
             cudaGetLastError();
             occ = 5;
         }
@@ -564,11 +679,11 @@ extern "C" int cgl_life_tune(uint32_t *buf_a, uint32_t *buf_b, uint32_t rows, ui
         // time 4 launches chained like cgl_life_run chains them (all a -> b: every launch writes the same
         // values, so re-running a strip early is harmless); the first one doubles as warm-up
         if (token_buf) CGL_CUDA(cudaMemsetAsync(token_buf, 0, (size_t)token_cap * 4, st));
-        int rc = tb_dispatch(kk, buf_a, buf_b, rows, cols, wrap_rows, st, ChainCtx{token_buf, 0, token_cap});
+        int rc = tb_dispatch(kk, buf_a, buf_b, rows, cols, wrap_rows, st, ChainCtx{token_buf, 0, token_cap}, PopCtx{});
         if (rc) return rc;
         CGL_CUDA(cudaEventRecord(e0, st));
         for (uint32_t rep = 1; rep <= 4; ++rep)
-            if ((rc = tb_dispatch(kk, buf_a, buf_b, rows, cols, wrap_rows, st, ChainCtx{token_buf, rep, token_cap})))
+            if ((rc = tb_dispatch(kk, buf_a, buf_b, rows, cols, wrap_rows, st, ChainCtx{token_buf, rep, token_cap}, PopCtx{})))
                 return rc;
         CGL_CUDA(cudaEventRecord(e1, st));
         CGL_CUDA(cudaEventSynchronize(e1));

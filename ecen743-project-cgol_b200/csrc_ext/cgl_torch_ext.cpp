@@ -10,6 +10,7 @@
 //   pack / unpack  uint8 cells <-> bit-packed world at the API boundary                -> cgl_pack / cgl_unpack
 //   reward / alive the reference's reductions (CGL/CGL.py:255-260)                     -> cgl_reward / cgl_alive
 //   life_run       world-only generations (life mode)                                  -> cgl_life_run
+//   life_run_pop   the same, recording the population after every generation           -> cgl_life_run_pop
 // cgl_b200/batched.py uses env_step for BatchedSim.step when the tensors are plain (the struct-cached ctypes path
 // serves the rest), tests/test_gpu_torch_ext.py checks every function against the ctypes binding.
 #include <c10/cuda/CUDAGuard.h>
@@ -178,6 +179,29 @@ bool life_run(const at::Tensor &a, const at::Tensor &b, int64_t rows, int64_t co
     return in_a != 0;
 }
 
+// life_run that also writes pop (int64 [gens]): live cells of rows [count_row0, count_row0 + count_rows) after each
+// generation.  True if the result is in a.
+bool life_run_pop(const at::Tensor &a, const at::Tensor &b, int64_t rows, int64_t cols, bool wrap_rows, int64_t gens,
+                  int64_t k, int64_t count_row0, int64_t count_rows, const at::Tensor &pop)
+{
+    check_cuda(a, at::kInt, "a");
+    check_cuda(b, at::kInt, "b");
+    check_cuda(pop, at::kLong, "pop");
+    const int64_t W = (cols + 31) / 32;
+    TORCH_CHECK(a.numel() == rows * W && b.numel() == rows * W, "buffers must hold rows * ceil(cols/32) words");
+    TORCH_CHECK(a.device() == b.device() && pop.device() == a.device(), "a, b and pop must be on the same device");
+    TORCH_CHECK(pop.numel() == gens, "pop must hold one count per generation");
+    TORCH_CHECK(count_row0 >= 0 && count_rows >= 1 && count_row0 + count_rows <= rows,
+                "count window [count_row0, count_row0 + count_rows) must lie inside the rows");
+    c10::cuda::CUDAGuard guard(a.device());
+    int in_a = 0;
+    check_rc(cgl_life_run_pop(static_cast<uint32_t *>(a.data_ptr()), static_cast<uint32_t *>(b.data_ptr()), (uint32_t)rows,
+                              (uint32_t)cols, wrap_rows ? 1 : 0, (uint32_t)gens, (uint32_t)k, (uint32_t)count_row0,
+                              (uint32_t)count_rows, static_cast<uint64_t *>(pop.data_ptr()), &in_a, stream_of(a)),
+             "cgl_life_run_pop");
+    return in_a != 0;
+}
+
 }  // namespace
 
 PYBIND11_MODULE(TORCH_EXTENSION_NAME, m)
@@ -197,4 +221,6 @@ PYBIND11_MODULE(TORCH_EXTENSION_NAME, m)
     m.def("reward", &reward);
     m.def("alive", &alive);
     m.def("life_run", &life_run);
+    m.def("life_run_pop", &life_run_pop, py::arg("a"), py::arg("b"), py::arg("rows"), py::arg("cols"), py::arg("wrap_rows"),
+          py::arg("gens"), py::arg("k"), py::arg("count_row0"), py::arg("count_rows"), py::arg("pop"));
 }

@@ -313,6 +313,16 @@ int cgl_life_run(uint32_t *buf_a_dev, uint32_t *buf_b_dev, uint32_t rows, uint32
                  int wrap_rows, uint32_t gens, uint32_t k, int *result_in_a_out,
                  cgl_stream_t stream);
 
+/* cgl_life_run that also records the population: pop_out_dev uint64 [gens] (overwritten), pop_out_dev[i] = live
+ * cells in rows [count_row0, count_row0 + count_rows) of the grid after generation i + 1 of this call.  Same
+ * generations, same final grid and same *result_in_a_out as cgl_life_run.  With wrap_rows = 0 a count is exact for
+ * rows the ghost-zone contract keeps exact.  The k-blocked kernels count the rows they emit in registers (no extra
+ * HBM pass); a generation that runs as cgl_life_step adds one read of the window.  CGL_E_BADARG for a NULL
+ * pop_out_dev, count_rows == 0 or a window that does not fit in `rows`, before any device work. */
+int cgl_life_run_pop(uint32_t *buf_a_dev, uint32_t *buf_b_dev, uint32_t rows, uint32_t cols, int wrap_rows,
+                     uint32_t gens, uint32_t k, uint32_t count_row0, uint32_t count_rows, uint64_t *pop_out_dev,
+                     int *result_in_a_out, cgl_stream_t stream);
+
 /* Optional set-up call: time a few strip lengths of the k-blocked kernel for this (rows, cols, k)
  * on the caller's buffers (buf_b is clobbered, buf_a untouched) and remember the fastest for later
  * cgl_life_run calls.  Synchronises the stream. */
