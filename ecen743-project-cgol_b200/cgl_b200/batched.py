@@ -16,6 +16,7 @@ do not depend on the number of GPUs.
 Beyond the single step (SURVEY.md section 8f):
   step(obs_out=, reward_out=)   the new observation goes straight into a caller buffer (replay ring, dqn.py)
   run(k, until_fixed=)          k plain steps / run-until-fixed in one launch, env resident on chip
+  run(k, actions=, reward_trace=, alive_trace=)   k steps following an action schedule, every step's reward recorded
   dead_rule=, empty=, empty_min=, masked_toggle=   the CGL_action+ fork's env
   breakdown_stable / breakdown_state, block_action, save_checkpoint / load_checkpoint, step_host(sync=False)
 """
@@ -274,25 +275,45 @@ class BatchedSim:
                                self._seq.value - (1 << 32 if self._seq.value >= 1 << 31 else 0))
             self._tok = want
 
-    def run(self, max_steps: int, until_fixed: bool = False, want_alive: bool = False):
-        """`max_steps` plain steps (no actions) for every env in ONE launch, the environments resident in
-        shared memory between steps (`cgl_env_run`): the loop of CGL/bench.py:39-40.  With until_fixed
-        an env stops after the first step that leaves its world unchanged -- the convergence loop of
-        CGL_action+/validate.py:133-139 (there: `old = get_state(); step()` then up to LIMIT more
-        compare-and-step rounds, i.e. max_steps = LIMIT + 1) without the per-step host compare.
+    def run(self, max_steps: int, until_fixed: bool = False, want_alive: bool = False,
+            actions: torch.Tensor | None = None, reward_trace: torch.Tensor | None = None,
+            alive_trace: torch.Tensor | None = None):
+        """`max_steps` steps for every env in ONE launch, the environments resident in shared memory between
+        steps (`cgl_env_run_ex`): the loop of CGL/bench.py:39-40.  With until_fixed an env stops after the
+        first step that leaves its world unchanged -- the convergence loop of CGL_action+/validate.py:133-139
+        (there: `old = get_state(); step()` then up to LIMIT more compare-and-step rounds, i.e. max_steps =
+        LIMIT + 1) without the per-step host compare.
+
+        actions (int32 [max_steps, B]): step t first applies actions[t] as step(actions[t]) does (side*side is
+        the no-op; invalid indices are ignored and raise in check_actions()).  reward_trace / alive_trace
+        (caller-owned int32 [max_steps, B]): row t receives every env's reward / live count after step t; with
+        until_fixed the rows from steps[e] on are left as they were.  All three must be contiguous and on the
+        env's device; until_fixed takes no actions.
         Returns (obs, reward, steps): steps = int32 [B] steps executed per env.  `count` advances by
         max_steps, the number of steps the batch was asked for."""
         if not isinstance(max_steps, int) or max_steps < 0:
             raise ValueError("max_steps must be a non-negative integer")
+        for name, t in (("actions", actions), ("reward_trace", reward_trace), ("alive_trace", alive_trace)):
+            if t is not None and (not isinstance(t, torch.Tensor) or t.dtype != torch.int32 or t.device != self.device
+                                  or not t.is_contiguous() or tuple(t.shape) != (max_steps, self.n_envs)):
+                raise TypeError(f"{name} must be a contiguous int32 tensor [max_steps, n_envs] on the env's device")
+        if until_fixed and actions is not None:
+            raise ValueError("until_fixed cannot follow an action schedule: a fixed point is not defined under actions")
         steps = torch.empty(self.n_envs, dtype=torch.int32, device=self.device)
+        a = native.EnvRunArgs()
+        a.world_in = a.world_out = self._wa.data_ptr()
+        a.stable, a.n_envs, a.side, a.max_steps = self.stable.data_ptr(), self.n_envs, self.side, max_steps
+        a.stop_when_fixed, a.spawn, a.stable_max = int(until_fixed), self.spawn, self.stable_max
+        a.dead_rule, a.empty, a.empty_min = DEAD_RULES[self.dead_rule], self.empty, self.empty_min
+        a.masked_toggle = int(self.masked_toggle)
+        a.actions = None if actions is None else actions.data_ptr()
+        a.reward_trace = None if reward_trace is None else reward_trace.data_ptr()
+        a.alive_trace = None if alive_trace is None else alive_trace.data_ptr()
+        a.steps_out, a.reward_out = steps.data_ptr(), self._reward.data_ptr()
+        a.alive_out = self._alive.data_ptr() if want_alive else None
+        a.err_flag = self._err.data_ptr()
         with torch.cuda.device(self.device):
-            native.check(self._lib.cgl_env_run_rule(native.dptr(self._wa), native.dptr(self._wa),
-                                                    native.dptr(self.stable), self.n_envs, self.side, max_steps,
-                                                    int(until_fixed), self.spawn, self.stable_max,
-                                                    DEAD_RULES[self.dead_rule], self.empty, self.empty_min,
-                                                    native.dptr(steps), native.dptr(self._reward),
-                                                    native.dptr(self._alive) if want_alive else None, self._stream()),
-                         "cgl_env_run_rule")
+            native.check(self._lib.cgl_env_run_ex(ctypes.byref(a), self._stream()), "cgl_env_run_ex")
         self.count += max_steps
         self.launches += 1
         return self.stable, self._reward, steps

@@ -82,6 +82,18 @@ class EnvStepArgs(ctypes.Structure):
 
 
 CHAIN_NONE, CHAIN_IDS, CHAIN_SEQ = 0, 1, 2
+
+class EnvRunArgs(ctypes.Structure):
+    """cgl_env_run_args_t (include/cgl_b200.h)."""
+    _fields_ = [("world_in", _vp), ("world_out", _vp), ("stable", _vp), ("n_envs", _u64), ("side", _u32),
+                ("max_steps", _u32), ("stop_when_fixed", ctypes.c_int32), ("spawn", ctypes.c_int32),
+                ("stable_max", ctypes.c_int32), ("dead_rule", ctypes.c_int32), ("empty", ctypes.c_int32),
+                ("empty_min", ctypes.c_int32), ("masked_toggle", ctypes.c_int32), ("actions", _vp),
+                ("reward_trace", _vp), ("alive_trace", _vp), ("steps_out", _vp), ("reward_out", _vp),
+                ("alive_out", _vp), ("err_flag", _vp)]
+
+
+SIGNATURES["cgl_env_run_ex"] = (_i, [ctypes.POINTER(EnvRunArgs), _vp])
 SIGNATURES["cgl_env_step_ex"] = (_i, [ctypes.POINTER(EnvStepArgs), _vp])
 SIGNATURES["cgl_env_step_seq"] = (_i, [ctypes.POINTER(EnvStepArgs), _u32, _u64, _u64, _vp])
 SIGNATURES["cgl_env_step_seq_timed"] = (_i, [ctypes.POINTER(EnvStepArgs), _u32, _u64, _u64, _vp, _vp, _vp])

@@ -356,6 +356,50 @@ CGL_HD void stable_update_sliced_sat(uint32_t (&p)[8], uint32_t surv, uint32_t b
     }
 }
 
+// ---- per-step reward straight from the bit planes (cgl_env_run_ex) -------------------------------------------------
+CGL_HD int popc32(uint32_t x)
+{
+#if defined(__CUDA_ARCH__)
+    return __popc(x);
+#else
+    return __builtin_popcount(x);
+#endif
+}
+
+// The cells of `bit` take the byte value v in every plane (a toggle's stability write).
+CGL_HD void set_cells_sliced(uint32_t (&p)[8], uint32_t bit, int v)
+{
+    for (int b = 0; b < 8; ++b) p[b] = (p[b] & ~bit) | (bit_mask_of(v, b) & bit);
+}
+
+// Cells whose byte, read unsigned, exceeds the constant k (0..255): an MSB-first compare against a uniform operand.
+CGL_HD uint32_t gt_const_sliced(const uint32_t (&p)[8], int k)
+{
+    uint32_t gt = 0, eq = 0xffffffffu;
+    for (int b = 7; b >= 0; --b) {
+        const uint32_t kb = bit_mask_of(k, b);
+        gt |= eq & p[b] & ~kb;
+        eq &= ~(p[b] ^ kb);
+    }
+    return gt;
+}
+
+// The int8 sum of 32 cells after a step of the run kernel, from the planes it carries (cgl_env_run.cu):
+//   CGL_DEAD_SAT    absolute planes: sum_b 2^b popc(plane b) with the sign plane weighing -128;
+//   CGL_DEAD_DECAY  every cell spawn-relative, s = int8(u + SPAWN) = u + SPAWN - 256 [u > 127 - SPAWN];
+//   CGL_DEAD_ZERO   the same over the live cells (`live`): after stable_update_sliced_rel every other cell is u = 0.
+// `wraps` may be false when no reachable u exceeds 127 - SPAWN (the base rule with SPAWN..MAX inside int8): the
+// compare is then skipped.
+CGL_HD int sliced_reward32(int rule, const uint32_t (&p)[8], uint32_t live, int spawn, bool wraps)
+{
+    int s = 0;
+    for (int b = 0; b < 8; ++b) s += popc32(p[b]) << b;
+    if (rule == CGL_DEAD_SAT) return s - (popc32(p[7]) << 8);
+    s += spawn * (rule == CGL_DEAD_DECAY ? 32 : popc32(live));
+    if (wraps) s -= popc32(gt_const_sliced(p, 127 - spawn)) << 8;
+    return s;
+}
+
 // Expand a 4-bit nibble to 4 byte masks (bit i -> byte i = 0xFF).
 CGL_HD uint32_t nibble_to_bytemask(uint32_t nib)
 {

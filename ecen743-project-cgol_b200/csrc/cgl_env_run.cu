@@ -15,6 +15,9 @@
 // way out, so k steps cost 2.25/k bytes per cell-update instead of 2.25 and the loop is bound by the
 // integer pipe.  The per-step logic is the fused env kernel's (cgl_env.cu): bit-sliced rows, (born,
 // surv) nibbles through the lane-private mask tables, byte-SIMD stability update.
+//
+// cgl_env_run_ex adds an action schedule (toggle_state before every step, as in cgl_env_step_rule) and per-step
+// reward / live-count traces to all three kernels, through their TR instantiations (DESIGN.md section 8 f3).
 #include <stdlib.h>
 
 #include "cgl_internal.cuh"
@@ -83,12 +86,25 @@ __device__ __forceinline__ uint32_t lds32(uint32_t shared_addr)
     return v;
 }
 
-template <int S>
+// Action schedules and per-step traces (cgl_env_run_ex) for every kernel of this file: TR = true adds the trailing
+// arguments' work, TR = false compiles to the kernel without them.  Inside, which of actions / reward trace / alive
+// trace are present are uniform run-time tests.  An action is applied as in cgl_env_step_rule: `size` is the no-op,
+// any other index outside [0, size) is ignored and reported; the toggled cell's stability becomes SPAWN (0 under the
+// masked toggle when the cell is dead after it), and the step sees the toggled world.
+struct RunTrace {
+    const int32_t *actions;         // int32 [max_steps][n_envs] or NULL
+    int32_t *reward;                // int32 [max_steps][n_envs] or NULL
+    uint32_t *alive;                // uint32 [max_steps][n_envs] or NULL
+    int *err_flag;
+    int masked;
+};
+
+template <int S, bool TR>
 __global__ void __launch_bounds__(RunCfg<S>::THREADS)
 env_run_kernel(const uint32_t *world_in, uint32_t *world_out, int8_t *stable, uint32_t n_envs,
                uint32_t max_steps, int stop_when_fixed, uint32_t spawn4, uint32_t max4,
                int32_t *__restrict__ steps_out, int32_t *__restrict__ reward_out, uint32_t *__restrict__ alive_out,
-               int rule, uint32_t min4, uint32_t empty4)
+               int rule, uint32_t min4, uint32_t empty4, RunTrace tr)
 {
     using C = RunCfg<S>;
     extern __shared__ __align__(16) unsigned char smem_dyn[];
@@ -104,9 +120,13 @@ env_run_kernel(const uint32_t *world_in, uint32_t *world_out, int8_t *stable, ui
     uint32_t *mix = nxt + C::WPE;
     uint4 *sst = reinterpret_cast<uint4 *>(mix + 2 * C::WPE);
     int *red = reinterpret_cast<int *>(smem_raw + 4096 + C::EPC * C::ENV_BYTES) + g * 2;
+    // TR, one env per CTA: per-step (reward, alive) sums of the warps, double-buffered by step parity
+    int *slot = reinterpret_cast<int *>(smem_raw + 4096 + C::EPC * C::ENV_BYTES) + 2 * C::EPC;
 
     const uint32_t e = blockIdx.x * C::EPC + g;
     const bool active = e < n_envs;
+    if constexpr (TR && C::EPC == 1)
+        if (t == 0) { slot[0] = 0; slot[1] = 0; slot[2] = 0; slot[3] = 0; }
 
     for (int i = threadIdx.x; i < 1024; i += C::THREADS) {
         const uint32_t m = nibble_to_bytemask((uint32_t)i >> 6);
@@ -138,7 +158,23 @@ env_run_kernel(const uint32_t *world_in, uint32_t *world_out, int8_t *stable, ui
     const uint32_t lane_s = (threadIdx.x & 31) * 4, lane_b = lane_s + 128;
     uint32_t steps = 0;
     bool done = !active || max_steps == 0;
+    const bool want_trace = TR && (tr.reward != nullptr || tr.alive != nullptr);
+    int next_act = C::SIZE;                          // the no-op
+    if constexpr (TR)
+        if (!done && tr.actions != nullptr) next_act = tr.actions[e];
     while (!done) {
+        int act = -1;                                // TR: the cell toggled before this step, or -1
+        int racc = 0;
+        uint32_t pacc = 0;
+        if constexpr (TR) {
+            const int a = next_act;
+            if (tr.actions != nullptr && steps + 1 < max_steps) next_act = tr.actions[(size_t)(steps + 1) * n_envs + e];
+            if (a >= 0 && a < C::SIZE) act = a;
+            else if (a != C::SIZE && t == 0) {
+                if (tr.err_flag != nullptr) atomicOr(tr.err_flag, 1);
+                raise_alarm(ALARM_BAD_ACTION);
+            }
+        }
         // ---- next generation: smem plane `cur` -> smem plane `nxt`, (born, surv) nibbles -> mix ----
         uint32_t changed = 0;
         {
@@ -149,6 +185,12 @@ env_run_kernel(const uint32_t *world_in, uint32_t *world_out, int8_t *stable, ui
                 int r = t * C::RPB + j - 1;
                 r = r < 0 ? S - 1 : (r >= S ? 0 : r);
                 lds_words<C::W>(cur + r * C::W, cw[j]);
+                if constexpr (TR) {
+                    // the toggle goes into every loaded copy of its row; `cur` itself stays as it was
+#pragma unroll
+                    for (int w = 0; w < C::W; ++w)
+                        if (act >= 0 && (act >> 5) == r * C::W + w) cw[j][w] ^= 1u << (act & 31);
+                }
 #pragma unroll
                 for (int w = 0; w < C::W; ++w)
                     hs[j][w] = hsum(west_plane(cw[j][(w + C::W - 1) % C::W], cw[j][w]), cw[j][w],
@@ -164,6 +206,7 @@ env_run_kernel(const uint32_t *world_in, uint32_t *world_out, int8_t *stable, ui
                     const uint32_t n = life_rule(hs[j][w], hs[j + 1][w], hs[j + 2][w], c);
                     nx[w] = n;
                     changed |= n ^ c;
+                    if constexpr (TR) pacc += __popc(n);
                     mix_nibbles(n & ~c, n & c, mx[2 * w], mx[2 * w + 1]);
                 }
                 sts_words<C::W>(nxt + r * C::W, nx);
@@ -171,6 +214,13 @@ env_run_kernel(const uint32_t *world_in, uint32_t *world_out, int8_t *stable, ui
             }
         }
         const bool any_changed = env_vote(changed != 0);
+        if constexpr (TR) {
+            // stable[act] = SPAWN (masked: 0 if the toggled cell is dead), written by the thread that updates its chunk
+            if (act >= 0 && t == (act >> 4) % C::TPE) {
+                const bool live = ((cur[act >> 5] >> (act & 31)) & 1u) == 0u;      // cur holds the untoggled plane
+                reinterpret_cast<int8_t *>(sst)[act] = (tr.masked && !live) ? (int8_t)0 : (int8_t)spawn4;
+            }
+        }
         // ---- stability plane in shared memory -------------------------------------------------------
 #pragma unroll 2
         for (int j = 0; j < C::CPT; ++j) {
@@ -190,13 +240,35 @@ env_run_kernel(const uint32_t *world_in, uint32_t *world_out, int8_t *stable, ui
                     const uint32_t born_mask = lds32(__byte_perm(bn, lane_s, 0x5504 + 16 * k));
                     s[k] = stable_update4_rule(rule, s[k], surv_mask, born_mask, spawn4, max4, min4, empty4);
                 }
+                if constexpr (TR) racc = __dp4a((int)s[k], 0x01010101, racc);
             }
             sst[c] = make_uint4(s[0], s[1], s[2], s[3]);
+        }
+        if (TR && want_trace) {
+            racc = __reduce_add_sync(0xffffffffu, racc);
+            pacc = __reduce_add_sync(0xffffffffu, pacc);
+            if ((threadIdx.x & 31) == 0) {
+                if constexpr (C::EPC == 1) {
+                    atomicAdd(&slot[2 * (steps & 1)], racc);
+                    atomicAdd(reinterpret_cast<unsigned *>(&slot[2 * (steps & 1) + 1]), pacc);
+                } else {
+                    if (tr.reward != nullptr) tr.reward[(size_t)steps * n_envs + e] = racc;
+                    if (tr.alive != nullptr) tr.alive[(size_t)steps * n_envs + e] = pacc;
+                }
+            }
         }
         uint32_t *tmp = cur; cur = nxt; nxt = tmp;
         ++steps;
         done = steps >= max_steps || (stop_when_fixed && !any_changed);
         env_sync();                                  // mix and the old plane are free again
+        if constexpr (TR && C::EPC == 1) {
+            if (want_trace && t == 0) {              // the barrier above completed this step's sums
+                int *sl = slot + 2 * ((steps - 1) & 1);
+                if (tr.reward != nullptr) tr.reward[(size_t)(steps - 1) * n_envs + e] = sl[0];
+                if (tr.alive != nullptr) tr.alive[(size_t)(steps - 1) * n_envs + e] = (uint32_t)sl[1];
+                sl[0] = 0; sl[1] = 0;
+            }
+        }
     }
 
     // ---- write back: world, stability, reward, alive, steps ----------------------------------------
@@ -262,12 +334,19 @@ struct SlicedCfg {
 // RULE = CGL_DEAD_ZERO: the base env (dead cells are 0; "don't care" planes, spawn-relative).  CGL_DEAD_DECAY: the
 // CGL_action+ fork's CUDA-kernel rule (dead cells fall by one per step to EMPTY_MIN), all cells carried
 // spawn-relative.  CGL_DEAD_SAT: the fork's CPU rule (dead cells become min(s + EMPTY, EMPTY_MIN)) on absolute planes.
-template <int S, int RULE>
+//
+// TR (cgl_env_run_ex): the owner of the toggled cell's row flips the bit in its registers before it computes the
+// row's sums -- the neighbours see the toggle through the published sums -- and writes the cell's planes.  Each step's
+// reward comes from the planes (sliced_reward32), its live count from popc of the new rows.  One env per CTA: every
+// warp adds its sums to a shared slot of the step's parity; thread 0 stores step t's after the barrier of step t+1
+// (the one that publishes the sums) and clears the slot; the last step's values are the final reward and live count.
+// Several envs per CTA (one warp each): lane 0 stores every step's sums.
+template <int S, int RULE, bool TR>
 __global__ void __launch_bounds__(SlicedCfg<S>::THREADS)
 env_run_sliced_kernel(const uint32_t *world_in, uint32_t *world_out, int8_t *stable, uint32_t n_envs,
                       uint32_t max_steps, int stop_when_fixed, int spawn, int stable_max, int empty_min,
                       int32_t *__restrict__ steps_out, int32_t *__restrict__ reward_out,
-                      uint32_t *__restrict__ alive_out, int empty)
+                      uint32_t *__restrict__ alive_out, int empty, RunTrace tr)
 {
     constexpr bool DECAY = RULE == CGL_DEAD_DECAY, SAT = RULE == CGL_DEAD_SAT;
     using C = SlicedCfg<S>;
@@ -276,12 +355,16 @@ env_run_sliced_kernel(const uint32_t *world_in, uint32_t *world_out, int8_t *sta
     const int t = threadIdx.x % C::TPE;
     uint32_t *hbuf = reinterpret_cast<uint32_t *>(smem_dyn) + g * (4 * C::WPE);     // [buffer][plane][row][w]
     int *red = reinterpret_cast<int *>(smem_dyn + C::EPC * (4 * C::WPE * 4)) + g * 2;
+    int *slot = reinterpret_cast<int *>(smem_dyn + C::EPC * (4 * C::WPE * 4)) + 2 * C::EPC;   // TR, EPC == 1
     const uint32_t e = blockIdx.x * C::EPC + g;
     const bool active = e < n_envs;
 
     uint32_t cw[C::RPB][C::W];                      // this thread's rows of the world
     uint32_t pl[C::RPB][C::W][8];                   // and their stability: 8 bit planes per word
     if (t == 0) { red[0] = 0; red[1] = 0; }
+    if constexpr (TR && C::EPC == 1)
+        if (t == 0) { slot[0] = 0; slot[1] = 0; slot[2] = 0; slot[3] = 0; }
+    uint32_t odd = 0;                               // TR, base rule: live cells loaded with u > STABLE - SPAWN
     if (active) {
         const uint32_t *wp = world_in + (size_t)e * C::WPE;
         const uint4 *sp = reinterpret_cast<const uint4 *>(stable + (size_t)e * C::SIZE);
@@ -295,10 +378,17 @@ env_run_sliced_kernel(const uint32_t *world_in, uint32_t *world_out, int8_t *sta
                 const uint32_t by[8] = {a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w};
                 bytes_to_planes32(by, pl[j][w]);
                 if constexpr (!SAT) add_const_sliced(pl[j][w], -spawn);     // spawn-relative planes (cgl_bits.cuh)
+                if constexpr (TR && !SAT && !DECAY) odd |= gt_const_sliced(pl[j][w], (stable_max - spawn) & 0xff) & cw[j][w];
             }
         }
     }
-    __syncthreads();
+    bool odd_env = false;
+    if constexpr (TR) {
+        if constexpr (C::EPC == 1) odd_env = __syncthreads_or(odd != 0) != 0;
+        else { __syncthreads(); odd_env = __any_sync(0xffffffffu, odd != 0); }
+    } else {
+        __syncthreads();
+    }
     const int max_rel = (stable_max - spawn) & 0xff, min_rel = (empty_min - spawn) & 0xff;
 
     auto env_vote = [&](bool p) -> bool {
@@ -314,8 +404,37 @@ env_run_sliced_kernel(const uint32_t *world_in, uint32_t *world_out, int8_t *sta
     const int r_dn = r_last == S - 1 ? 0 : r_last + 1;
 
     uint32_t steps = 0, changed = 1u, buf = 0;
+    const bool want_trace = TR && (tr.reward != nullptr || tr.alive != nullptr);
+    // The base rule's live cells hold u in [0, STABLE - SPAWN] (a toggle or a birth sets 0, survivors count up to it)
+    // unless the loaded plane had others; u > 127 - SPAWN then needs SPAWN..MAX to wrap int8.
+    const bool wraps = DECAY || max_rel > 127 - spawn || odd_env;
     if (active) {
+        int next_act = C::SIZE;                     // the no-op
+        if constexpr (TR)
+            if (tr.actions != nullptr && max_steps > 0) next_act = tr.actions[e];
         while (steps < max_steps) {
+            if constexpr (TR) {
+                const int a = next_act;             // all threads of the env load the same word: a broadcast
+                if (tr.actions != nullptr && steps + 1 < max_steps) next_act = tr.actions[(size_t)(steps + 1) * n_envs + e];
+                if (a >= 0 && a < C::SIZE) {
+                    if (a / (S * C::RPB) == t) {    // the owner of the cell's row
+                        const int j = (a / S) % C::RPB, w = (a % S) >> 5;
+                        const uint32_t bit = 1u << (a & 31);
+#pragma unroll
+                        for (int jj = 0; jj < C::RPB; ++jj)
+#pragma unroll
+                            for (int ww = 0; ww < C::W; ++ww)
+                                if (jj == j && ww == w) {
+                                    cw[jj][ww] ^= bit;
+                                    const int v = (tr.masked && !(cw[jj][ww] & bit)) ? 0 : spawn;
+                                    set_cells_sliced(pl[jj][ww], bit, SAT ? v : v - spawn);
+                                }
+                    }
+                } else if (a != C::SIZE && t == 0) {
+                    if (tr.err_flag != nullptr) atomicOr(tr.err_flag, 1);
+                    raise_alarm(ALARM_BAD_ACTION);
+                }
+            }
             // horizontal sums of my rows; (s0, s1) go to the shared plane for the rows above and below
             HSum hs[C::RPB][C::W];
             uint32_t *h0 = hbuf + buf * (2 * C::WPE), *h1 = h0 + C::WPE;
@@ -336,6 +455,16 @@ env_run_sliced_kernel(const uint32_t *world_in, uint32_t *world_out, int8_t *sta
             // one barrier: publishes the sums and votes on whether the PREVIOUS step changed the world
             const bool any_changed = env_vote(changed != 0);
             if (stop_when_fixed && !any_changed) break;
+            if constexpr (TR && C::EPC == 1) {
+                if (want_trace && t == 0 && steps > 0) {
+                    int *sl = slot + 2 * ((steps - 1) & 1);
+                    if (tr.reward != nullptr) tr.reward[(size_t)(steps - 1) * n_envs + e] = sl[0];
+                    if (tr.alive != nullptr) tr.alive[(size_t)(steps - 1) * n_envs + e] = (uint32_t)sl[1];
+                    sl[0] = 0; sl[1] = 0;
+                }
+            }
+            int racc = 0;
+            uint32_t pacc = 0;
             uint32_t up0[C::W], up1[C::W], dn0[C::W], dn1[C::W];
             lds_words<C::W>(h0 + r_up * C::W, up0);
             lds_words<C::W>(h1 + r_up * C::W, up1);
@@ -356,7 +485,24 @@ env_run_sliced_kernel(const uint32_t *world_in, uint32_t *world_out, int8_t *sta
                     if constexpr (SAT) stable_update_sliced_sat(pl[j][w], n & c, n & ~c, spawn, stable_max, empty, empty_min);
                     else if constexpr (DECAY) stable_update_sliced_decay(pl[j][w], n & c, n & ~c, max_rel, min_rel);
                     else stable_update_sliced_rel(pl[j][w], n & c, max_rel);
+                    if constexpr (TR) {
+                        racc += sliced_reward32(RULE, pl[j][w], n, spawn, wraps);
+                        pacc += __popc(n);
+                    }
                     cw[j][w] = n;
+                }
+            }
+            if (TR && want_trace) {
+                racc = __reduce_add_sync(0xffffffffu, racc);
+                pacc = __reduce_add_sync(0xffffffffu, pacc);
+                if ((threadIdx.x & 31) == 0) {
+                    if constexpr (C::EPC == 1) {
+                        atomicAdd(&slot[2 * (steps & 1)], racc);
+                        atomicAdd(reinterpret_cast<unsigned *>(&slot[2 * (steps & 1) + 1]), pacc);
+                    } else {
+                        if (tr.reward != nullptr) tr.reward[(size_t)steps * n_envs + e] = racc;
+                        if (tr.alive != nullptr) tr.alive[(size_t)steps * n_envs + e] = pacc;
+                    }
                 }
             }
             ++steps;
@@ -406,26 +552,37 @@ env_run_sliced_kernel(const uint32_t *world_in, uint32_t *world_out, int8_t *sta
         if (reward_out != nullptr) reward_out[e] = acc;
         if (alive_out != nullptr) alive_out[e] = pop;
         if (steps_out != nullptr) steps_out[e] = (int32_t)steps;
+        if constexpr (TR && C::EPC == 1) {
+            if (steps > 0) {                        // the last step: its sums are the final reward and live count
+                if (tr.reward != nullptr) tr.reward[(size_t)(steps - 1) * n_envs + e] = acc;
+                if (tr.alive != nullptr) tr.alive[(size_t)(steps - 1) * n_envs + e] = pop;
+            }
+        }
     }
 }
 
 // Any side whose three byte planes fit in 220 KiB of shared memory (side <= 274): one CTA per env, one byte per cell.
+// TR: thread 0 applies the step's toggle before a barrier; the per-step sums ride on the loop over the cells and are
+// stored by thread 0 after the step's vote.
+template <bool TR>
 __global__ void __launch_bounds__(256)
 env_run_generic_kernel(const uint32_t *world_in, uint32_t *world_out, int8_t *stable, uint32_t side, uint32_t W,
                        uint32_t max_steps, int stop_when_fixed, int8_t spawn, int8_t stable_max,
                        int32_t *__restrict__ steps_out, int32_t *__restrict__ reward_out,
-                       uint32_t *__restrict__ alive_out, int rule, int8_t empty, int8_t empty_min)
+                       uint32_t *__restrict__ alive_out, int rule, int8_t empty, int8_t empty_min, RunTrace tr)
 {
     extern __shared__ __align__(16) unsigned char smem_dyn[];
     const uint32_t size = side * side;
     uint8_t *a = smem_dyn, *b = a + size;
     int8_t *st = reinterpret_cast<int8_t *>(b + size);
-    __shared__ int red[2];
+    __shared__ int red[TR ? 6 : 2];                 // TR: red[2 + 2 * (step & 1)] = the step's (reward, alive)
     const uint64_t e = blockIdx.x;
     const uint32_t *wi = world_in + e * side * W;
     uint32_t *wo = world_out + e * side * W;
     int8_t *sg = stable + e * size;
     if (threadIdx.x == 0) { red[0] = 0; red[1] = 0; }
+    if constexpr (TR)
+        if (threadIdx.x == 0) { red[2] = 0; red[3] = 0; red[4] = 0; red[5] = 0; }
     for (uint32_t i = threadIdx.x; i < size; i += blockDim.x) {
         const uint32_t y = i / side, x = i - y * side;
         a[i] = (wi[y * W + (x >> 5)] >> (x & 31)) & 1u;
@@ -436,6 +593,23 @@ env_run_generic_kernel(const uint32_t *world_in, uint32_t *world_out, int8_t *st
     bool done = max_steps == 0;
     while (!done) {
         int changed = 0;
+        int racc = 0;
+        uint32_t pacc = 0;
+        if constexpr (TR) {
+            if (tr.actions != nullptr) {
+                if (threadIdx.x == 0) {
+                    const int act = tr.actions[(size_t)steps * gridDim.x + e];
+                    if (act >= 0 && (uint32_t)act < size) {
+                        a[act] ^= 1u;
+                        st[act] = (tr.masked && !a[act]) ? (int8_t)0 : spawn;
+                    } else if ((uint32_t)act != size) {
+                        if (tr.err_flag != nullptr) atomicOr(tr.err_flag, 1);
+                        raise_alarm(ALARM_BAD_ACTION);
+                    }
+                }
+                __syncthreads();
+            }
+        }
         for (uint32_t i = threadIdx.x; i < size; i += blockDim.x) {
             const uint32_t y = i / side, x = i - y * side;
             const uint32_t yu = (y == 0 ? side : y) - 1, yd = (y + 1 == side) ? 0 : y + 1;
@@ -447,8 +621,26 @@ env_run_generic_kernel(const uint32_t *world_in, uint32_t *world_out, int8_t *st
             b[i] = q;
             changed |= (p != q);
             st[i] = stable_update1_rule(rule, st[i], p != 0, q != 0, spawn, stable_max, empty, empty_min);
+            if constexpr (TR) { racc += st[i]; pacc += q; }
+        }
+        if constexpr (TR) {
+            racc = __reduce_add_sync(0xffffffffu, racc);
+            pacc = __reduce_add_sync(0xffffffffu, pacc);
+            if ((threadIdx.x & 31) == 0) {
+                atomicAdd(&red[2 + 2 * (steps & 1)], racc);
+                atomicAdd(reinterpret_cast<unsigned *>(&red[3 + 2 * (steps & 1)]), pacc);
+            }
         }
         const bool any_changed = __syncthreads_or(changed) != 0;
+        if constexpr (TR) {
+            // the vote's barrier completed the sums; the slot is added to again two steps later, after the next vote
+            if (threadIdx.x == 0) {
+                int *sl = red + 2 + 2 * (steps & 1);
+                if (tr.reward != nullptr) tr.reward[(size_t)steps * gridDim.x + e] = sl[0];
+                if (tr.alive != nullptr) tr.alive[(size_t)steps * gridDim.x + e] = (uint32_t)sl[1];
+                sl[0] = 0; sl[1] = 0;
+            }
+        }
         uint8_t *tmp = a; a = b; b = tmp;
         ++steps;
         done = steps >= max_steps || (stop_when_fixed && !any_changed);
@@ -494,31 +686,41 @@ static bool run_use_sliced(uint32_t max_steps)
     return max_steps >= 4;
 }
 
-template <int S>
-static int launch_env_run(const uint32_t *win, uint32_t *wout, int8_t *stable, uint64_t n_envs, uint32_t max_steps,
-                          int stop, int spawn, int stable_max, int32_t *steps, int32_t *reward, uint32_t *alive,
-                          cudaStream_t st, int rule, int empty, int empty_min)
+template <int S, bool TR>
+static void launch_env_run_as(const cgl_env_run_args_t &a, const RunTrace &tr, cudaStream_t st)
 {
     using C = RunCfg<S>;
-    static PerDeviceOnce once;
-    if (once.first())
-        CGL_CUDA(cudaFuncSetAttribute(env_run_kernel<S>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM));
-    const unsigned grid = (unsigned)((n_envs + C::EPC - 1) / C::EPC);
-    if (run_use_sliced(max_steps)) {
+    const unsigned grid = (unsigned)((a.n_envs + C::EPC - 1) / C::EPC);
+    if (run_use_sliced(a.max_steps)) {
         using D = SlicedCfg<S>;
+        constexpr int smem = D::SMEM + (TR ? 16 : 0);             // TR: the step sums' slots
 #define CGL_RUN_SLICED(RULE)                                                                                          \
-    env_run_sliced_kernel<S, RULE><<<grid, D::THREADS, D::SMEM, st>>>(win, wout, stable, (uint32_t)n_envs, max_steps, \
-                                                                       stop, spawn, stable_max, empty_min, steps,      \
-                                                                       reward, alive, empty)
-        if (rule == CGL_DEAD_DECAY) CGL_RUN_SLICED(CGL_DEAD_DECAY);
-        else if (rule == CGL_DEAD_SAT) CGL_RUN_SLICED(CGL_DEAD_SAT);
+    env_run_sliced_kernel<S, RULE, TR><<<grid, D::THREADS, smem, st>>>(                                                \
+        a.world_in_dev, a.world_out_dev, a.stable_dev, (uint32_t)a.n_envs, a.max_steps, a.stop_when_fixed, a.spawn,   \
+        a.stable_max, a.empty_min, a.steps_out_dev, a.reward_out_dev, a.alive_out_dev, a.empty, tr)
+        if (a.dead_rule == CGL_DEAD_DECAY) CGL_RUN_SLICED(CGL_DEAD_DECAY);
+        else if (a.dead_rule == CGL_DEAD_SAT) CGL_RUN_SLICED(CGL_DEAD_SAT);
         else CGL_RUN_SLICED(CGL_DEAD_ZERO);
 #undef CGL_RUN_SLICED
     } else {
-        env_run_kernel<S><<<grid, C::THREADS, C::SMEM, st>>>(win, wout, stable, (uint32_t)n_envs, max_steps, stop,
-                                                            rep4(spawn), rep4(stable_max), steps, reward, alive, rule,
-                                                            rep4(empty_min), rep4(empty));
+        env_run_kernel<S, TR><<<grid, C::THREADS, C::SMEM + (TR ? 16 : 0), st>>>(
+            a.world_in_dev, a.world_out_dev, a.stable_dev, (uint32_t)a.n_envs, a.max_steps, a.stop_when_fixed,
+            rep4(a.spawn), rep4(a.stable_max), a.steps_out_dev, a.reward_out_dev, a.alive_out_dev, a.dead_rule,
+            rep4(a.empty_min), rep4(a.empty), tr);
     }
+}
+
+template <int S>
+static int launch_env_run(const cgl_env_run_args_t &a, bool traced, const RunTrace &tr, cudaStream_t st)
+{
+    using C = RunCfg<S>;
+    static PerDeviceOnce once;
+    if (once.first()) {
+        CGL_CUDA(cudaFuncSetAttribute(env_run_kernel<S, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM));
+        CGL_CUDA(cudaFuncSetAttribute(env_run_kernel<S, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM + 16));
+    }
+    if (traced) launch_env_run_as<S, true>(a, tr, st);
+    else launch_env_run_as<S, false>(a, tr, st);
     CGL_LAUNCH_CHECK();
     return 0;
 }
@@ -547,40 +749,68 @@ breakdown_kernel(const int8_t *__restrict__ stable, uint64_t size, uint32_t *__r
 
 using namespace cgl;
 
-extern "C" int cgl_env_run_rule(const uint32_t *win, uint32_t *wout, int8_t *stable, uint64_t n_envs, uint32_t side,
-                                uint32_t max_steps, int stop_when_fixed, int spawn, int stable_max, int dead_rule,
-                                int empty, int empty_min, int32_t *steps, int32_t *reward, uint32_t *alive,
-                                cgl_stream_t stream)
+// The one implementation behind cgl_env_run and cgl_env_run_rule (see include/cgl_b200.h).
+extern "C" int cgl_env_run_ex(const cgl_env_run_args_t *args, cgl_stream_t stream)
 {
-    CGL_REQUIRE(win && wout && stable && n_envs && side, CGL_E_BADARG, "cgl_env_run: bad argument");
-    CGL_REQUIRE(n_envs < (1ull << 31), CGL_E_BADARG, "cgl_env_run: n_envs too large");
-    CGL_REQUIRE(dead_rule >= CGL_DEAD_ZERO && dead_rule <= CGL_DEAD_SAT && empty >= -128 && empty <= 127 &&
-                    empty_min >= -128 && empty_min <= 127,
+    CGL_REQUIRE(args, CGL_E_BADARG, "cgl_env_run_ex: null");
+    const cgl_env_run_args_t &a = *args;
+    CGL_REQUIRE(a.world_in_dev && a.world_out_dev && a.stable_dev && a.n_envs && a.side, CGL_E_BADARG,
+                "cgl_env_run: bad argument");
+    CGL_REQUIRE(a.n_envs < (1ull << 31), CGL_E_BADARG, "cgl_env_run: n_envs too large");
+    CGL_REQUIRE(a.dead_rule >= CGL_DEAD_ZERO && a.dead_rule <= CGL_DEAD_SAT && a.empty >= -128 && a.empty <= 127 &&
+                    a.empty_min >= -128 && a.empty_min <= 127,
                 CGL_E_BADARG, "cgl_env_run_rule: dead_rule must be 0..2, empty / empty_min must fit int8");
+    CGL_REQUIRE(a.masked_toggle == 0 || a.masked_toggle == 1, CGL_E_BADARG, "cgl_env_run_ex: masked_toggle must be 0 or 1");
+    CGL_REQUIRE(!(a.stop_when_fixed && a.actions_dev), CGL_E_BADARG,
+                "cgl_env_run_ex: stop_when_fixed cannot take an action schedule (a fixed point is not defined under actions)");
+    const void *bufs[3] = {a.actions_dev, a.reward_trace_dev, a.alive_trace_dev};
+    for (int i = 0; i < 3; ++i)
+        for (int k = i + 1; k < 3; ++k)
+            CGL_REQUIRE(bufs[i] == nullptr || bufs[i] != bufs[k], CGL_E_BADARG,
+                        "cgl_env_run_ex: the action schedule and the traces must be separate buffers");
+    const bool traced = a.actions_dev || a.reward_trace_dev || a.alive_trace_dev;
+    const RunTrace tr = {a.actions_dev, a.reward_trace_dev, a.alive_trace_dev, a.err_flag_dev, a.masked_toggle};
     cudaStream_t st = as_stream(stream);
-    if (cgl_env_step_is_fused(side)) {
-#define CGL_CASE(S)                                                                                       \
-    case S:                                                                                               \
-        return launch_env_run<S>(win, wout, stable, n_envs, max_steps, stop_when_fixed, spawn, stable_max, \
-                                 steps, reward, alive, st, dead_rule, empty, empty_min)
-        switch (side) {
+    if (cgl_env_step_is_fused(a.side)) {
+#define CGL_CASE(S) \
+    case S: return launch_env_run<S>(a, traced, tr, st)
+        switch (a.side) {
             CGL_CASE(32); CGL_CASE(64); CGL_CASE(96); CGL_CASE(128);
             CGL_CASE(160); CGL_CASE(192); CGL_CASE(224); CGL_CASE(256);
         }
 #undef CGL_CASE
     }
-    const size_t smem = 3ull * side * side;
+    const size_t smem = 3ull * a.side * a.side;
     CGL_REQUIRE(smem <= 220 * 1024, CGL_E_BADARG,
                 "cgl_env_run: side must be a fused side or small enough for shared memory (side <= 274)");
     static PerDeviceOnce once;                   // opt in to the largest size once per device
-    if (once.first())
-        CGL_CUDA(cudaFuncSetAttribute(env_run_generic_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024));
-    env_run_generic_kernel<<<(unsigned)n_envs, 256, smem, st>>>(win, wout, stable, side, cgl_words_per_row(side),
-                                                               max_steps, stop_when_fixed, (int8_t)spawn,
-                                                               (int8_t)stable_max, steps, reward, alive, dead_rule,
-                                                               (int8_t)empty, (int8_t)empty_min);
+    if (once.first()) {
+        CGL_CUDA(cudaFuncSetAttribute(env_run_generic_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024));
+        CGL_CUDA(cudaFuncSetAttribute(env_run_generic_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024));
+    }
+#define CGL_RUN_GENERIC(TR)                                                                                            \
+    env_run_generic_kernel<TR><<<(unsigned)a.n_envs, 256, smem, st>>>(                                                 \
+        a.world_in_dev, a.world_out_dev, a.stable_dev, a.side, cgl_words_per_row(a.side), a.max_steps,                \
+        a.stop_when_fixed, (int8_t)a.spawn, (int8_t)a.stable_max, a.steps_out_dev, a.reward_out_dev, a.alive_out_dev, \
+        a.dead_rule, (int8_t)a.empty, (int8_t)a.empty_min, tr)
+    if (traced) CGL_RUN_GENERIC(true);
+    else CGL_RUN_GENERIC(false);
+#undef CGL_RUN_GENERIC
     CGL_LAUNCH_CHECK();
     return 0;
+}
+
+extern "C" int cgl_env_run_rule(const uint32_t *win, uint32_t *wout, int8_t *stable, uint64_t n_envs, uint32_t side,
+                                uint32_t max_steps, int stop_when_fixed, int spawn, int stable_max, int dead_rule,
+                                int empty, int empty_min, int32_t *steps, int32_t *reward, uint32_t *alive,
+                                cgl_stream_t stream)
+{
+    cgl_env_run_args_t a = {};
+    a.world_in_dev = win; a.world_out_dev = wout; a.stable_dev = stable; a.n_envs = n_envs; a.side = side;
+    a.max_steps = max_steps; a.stop_when_fixed = stop_when_fixed; a.spawn = spawn; a.stable_max = stable_max;
+    a.dead_rule = dead_rule; a.empty = empty; a.empty_min = empty_min;
+    a.steps_out_dev = steps; a.reward_out_dev = reward; a.alive_out_dev = alive;
+    return cgl_env_run_ex(&a, stream);
 }
 
 extern "C" int cgl_env_run(const uint32_t *win, uint32_t *wout, int8_t *stable, uint64_t n_envs, uint32_t side,

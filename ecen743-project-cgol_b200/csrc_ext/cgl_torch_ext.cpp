@@ -7,6 +7,7 @@
 // torch-typed face of it:
 //   env_step       toggle + generation + int8 stability + reward for a batch          -> cgl_env_step_ex
 //   env_run        k plain steps / run-until-fixed in one launch                       -> cgl_env_run_rule
+//   env_run_ex     the same with an action schedule and per-step reward / alive traces -> cgl_env_run_ex
 //   pack / unpack  uint8 cells <-> bit-packed world at the API boundary                -> cgl_pack / cgl_unpack
 //   reward / alive the reference's reductions (CGL/CGL.py:255-260)                     -> cgl_reward / cgl_alive
 //   life_run       world-only generations (life mode)                                  -> cgl_life_run
@@ -107,6 +108,52 @@ at::Tensor env_run(const at::Tensor &world, const at::Tensor &stable, int64_t si
                               static_cast<int32_t *>(steps.data_ptr()), ptr<int32_t>(reward_out), ptr<uint32_t>(alive_out),
                               stream_of(world)),
              "cgl_env_run_rule");
+    return steps;
+}
+
+// env_run with an action schedule (int32 [max_steps, n_envs]) and per-step traces (int32 [max_steps, n_envs], row t
+// = after step t), each optional; masked_toggle and err_flag (int32 [1]) as in env_step.  Returns steps per env.
+at::Tensor env_run_ex(const at::Tensor &world, const at::Tensor &stable, int64_t side, int64_t max_steps,
+                      bool until_fixed, int64_t spawn, int64_t stable_max, int64_t dead_rule, int64_t empty,
+                      int64_t empty_min, bool masked_toggle, const c10::optional<at::Tensor> &actions,
+                      const c10::optional<at::Tensor> &reward_trace, const c10::optional<at::Tensor> &alive_trace,
+                      const c10::optional<at::Tensor> &reward_out, const c10::optional<at::Tensor> &alive_out,
+                      const c10::optional<at::Tensor> &err_flag)
+{
+    check_cuda(world, at::kInt, "world");
+    check_cuda(stable, at::kChar, "stable");
+    const int64_t size = side * side;
+    TORCH_CHECK(side >= 1 && stable.numel() % size == 0 && max_steps >= 0, "bad shape");
+    const int64_t n = stable.numel() / size;
+    const std::pair<const c10::optional<at::Tensor> *, const char *> sched[3] = {
+        {&actions, "actions"}, {&reward_trace, "reward_trace"}, {&alive_trace, "alive_trace"}};
+    for (const auto &p : sched) {
+        if (!p.first->has_value()) continue;
+        check_cuda(**p.first, at::kInt, p.second);
+        TORCH_CHECK((*p.first)->dim() == 2 && (*p.first)->size(0) == max_steps && (*p.first)->size(1) == n, p.second,
+                    " must be [max_steps, n_envs]");
+    }
+    if (reward_out.has_value()) check_cuda(*reward_out, at::kInt, "reward_out");
+    if (alive_out.has_value()) check_cuda(*alive_out, at::kInt, "alive_out");
+    if (err_flag.has_value()) check_cuda(*err_flag, at::kInt, "err_flag");
+    c10::cuda::CUDAGuard guard(world.device());
+    at::Tensor steps = at::empty({n}, world.options().dtype(at::kInt));
+    cgl_env_run_args_t a = {};
+    a.world_in_dev = static_cast<const uint32_t *>(world.data_ptr());
+    a.world_out_dev = static_cast<uint32_t *>(world.data_ptr());
+    a.stable_dev = static_cast<int8_t *>(stable.data_ptr());
+    a.n_envs = (uint64_t)n; a.side = (uint32_t)side; a.max_steps = (uint32_t)max_steps;
+    a.stop_when_fixed = until_fixed ? 1 : 0; a.spawn = (int32_t)spawn; a.stable_max = (int32_t)stable_max;
+    a.dead_rule = (int32_t)dead_rule; a.empty = (int32_t)empty; a.empty_min = (int32_t)empty_min;
+    a.masked_toggle = masked_toggle ? 1 : 0;
+    a.actions_dev = ptr<const int32_t>(actions);
+    a.reward_trace_dev = ptr<int32_t>(reward_trace);
+    a.alive_trace_dev = ptr<uint32_t>(alive_trace);
+    a.steps_out_dev = static_cast<int32_t *>(steps.data_ptr());
+    a.reward_out_dev = ptr<int32_t>(reward_out);
+    a.alive_out_dev = ptr<uint32_t>(alive_out);
+    a.err_flag_dev = ptr<int>(err_flag);
+    check_rc(cgl_env_run_ex(&a, stream_of(world)), "cgl_env_run_ex");
     return steps;
 }
 
@@ -216,6 +263,11 @@ PYBIND11_MODULE(TORCH_EXTENSION_NAME, m)
     m.def("env_run", &env_run, py::arg("world"), py::arg("stable"), py::arg("side"), py::arg("max_steps"),
           py::arg("until_fixed") = false, py::arg("spawn") = -1, py::arg("stable_max") = 1, py::arg("dead_rule") = 0,
           py::arg("empty") = 0, py::arg("empty_min") = 0, py::arg("reward_out") = py::none(), py::arg("alive_out") = py::none());
+    m.def("env_run_ex", &env_run_ex, py::arg("world"), py::arg("stable"), py::arg("side"), py::arg("max_steps"),
+          py::arg("until_fixed") = false, py::arg("spawn") = -1, py::arg("stable_max") = 1, py::arg("dead_rule") = 0,
+          py::arg("empty") = 0, py::arg("empty_min") = -128, py::arg("masked_toggle") = false,
+          py::arg("actions") = py::none(), py::arg("reward_trace") = py::none(), py::arg("alive_trace") = py::none(),
+          py::arg("reward_out") = py::none(), py::arg("alive_out") = py::none(), py::arg("err_flag") = py::none());
     m.def("pack", &pack);
     m.def("unpack", &unpack);
     m.def("reward", &reward);

@@ -201,6 +201,36 @@ int cgl_env_run_rule(const uint32_t *world_in_dev, uint32_t *world_out_dev, int8
                      int dead_rule, int empty, int empty_min, int32_t *steps_out_dev, int32_t *reward_out_dev,
                      uint32_t *alive_out_dev, cgl_stream_t stream);
 
+/* The struct form of cgl_env_run / cgl_env_run_rule (both call it), which adds an action schedule and per-step
+ * traces to the on-chip run.  Zero-initialise it; zero fields keep the meaning they have in cgl_env_run_rule.
+ * For every env e and step t = 0 .. max_steps-1, in order:
+ *   1. if actions_dev != NULL: toggle_state(actions_dev[t * n_envs + e]) exactly as cgl_env_step_rule applies its
+ *      action (side*side is the no-op; any other index outside [0, side*side) is ignored, sets *err_flag_dev |= 1
+ *      and alarm word 0; masked_toggle as there);
+ *   2. one generation and the stability update;
+ *   3. reward_trace_dev[t * n_envs + e] = the reward (int32 sum of the stability plane) and
+ *      alive_trace_dev[t * n_envs + e] = the live count, for each trace that is not NULL.
+ * So a run equals max_steps calls of cgl_env_step_rule with actions_dev + t * n_envs, the reward and live count read
+ * after each, at the cost of the on-chip run (DESIGN.md section 8 f3).  With stop_when_fixed (which takes no actions:
+ * CGL_E_BADARG) the rows t >= steps_out_dev[e] are not written.  Row indices are 64-bit.  Argument errors (NULL
+ * struct or plane, n_envs >= 2^31, dead_rule / empty / empty_min / masked_toggle out of range, a side that does not
+ * fit, a schedule or trace sharing another's buffer) return CGL_E_BADARG before any device work. */
+typedef struct cgl_env_run_args {
+    const uint32_t *world_in_dev;
+    uint32_t *world_out_dev;          /* may alias world_in_dev, as in cgl_env_run */
+    int8_t *stable_dev;
+    uint64_t n_envs;
+    uint32_t side, max_steps;
+    int32_t stop_when_fixed, spawn, stable_max, dead_rule, empty, empty_min, masked_toggle;
+    const int32_t *actions_dev;       /* int32 [max_steps][n_envs] or NULL (plain steps) */
+    int32_t *reward_trace_dev;        /* int32 [max_steps][n_envs] or NULL */
+    uint32_t *alive_trace_dev;        /* uint32 [max_steps][n_envs] or NULL */
+    int32_t *steps_out_dev, *reward_out_dev;
+    uint32_t *alive_out_dev;
+    int *err_flag_dev;                /* or NULL */
+} cgl_env_run_args_t;
+int cgl_env_run_ex(const cgl_env_run_args_t *args, cgl_stream_t stream);
+
 /* Value counts of the stability plane, the device form of breakdown_stable (CGL/CGL_action+/CGL.py:
  * 294-297, np.unique(..., return_counts=True)): hist_out_dev uint32 [n_envs][256],
  * hist[e][v + 128] = number of cells of env e whose stability equals v. */
