@@ -17,6 +17,7 @@ Beyond the single step (SURVEY.md section 8f):
   step(obs_out=, reward_out=)   the new observation goes straight into a caller buffer (replay ring, dqn.py)
   run(k, until_fixed=)          k plain steps / run-until-fixed in one launch, env resident on chip
   run(k, actions=, reward_trace=, alive_trace=)   k steps following an action schedule, every step's reward recorded
+  run(k, ..., obs_trace=)       and every step's observation, written straight into a caller buffer (replay ring)
   dead_rule=, empty=, empty_min=, masked_toggle=   the CGL_action+ fork's env
   breakdown_stable / breakdown_state, block_action, save_checkpoint / load_checkpoint, step_host(sync=False)
 """
@@ -277,7 +278,7 @@ class BatchedSim:
 
     def run(self, max_steps: int, until_fixed: bool = False, want_alive: bool = False,
             actions: torch.Tensor | None = None, reward_trace: torch.Tensor | None = None,
-            alive_trace: torch.Tensor | None = None):
+            alive_trace: torch.Tensor | None = None, obs_trace: torch.Tensor | None = None):
         """`max_steps` steps for every env in ONE launch, the environments resident in shared memory between
         steps (`cgl_env_run_ex`): the loop of CGL/bench.py:39-40.  With until_fixed an env stops after the
         first step that leaves its world unchanged -- the convergence loop of CGL_action+/validate.py:133-139
@@ -289,6 +290,10 @@ class BatchedSim:
         (caller-owned int32 [max_steps, B]): row t receives every env's reward / live count after step t; with
         until_fixed the rows from steps[e] on are left as they were.  All three must be contiguous and on the
         env's device; until_fixed takes no actions.
+        obs_trace (caller-owned int8 [max_steps, B, size], contiguous, on the env's device): row t receives every
+        env's stability plane after step t (`cgl_env_run_obs`).  The run is then out of place like step(obs_out=):
+        the current plane is left untouched and `self.stable` becomes the view obs_trace[max_steps - 1] (with
+        max_steps == 0 nothing is written and `self.stable` stays).  until_fixed takes no obs_trace.
         Returns (obs, reward, steps): steps = int32 [B] steps executed per env.  `count` advances by
         max_steps, the number of steps the batch was asked for."""
         if not isinstance(max_steps, int) or max_steps < 0:
@@ -297,8 +302,14 @@ class BatchedSim:
             if t is not None and (not isinstance(t, torch.Tensor) or t.dtype != torch.int32 or t.device != self.device
                                   or not t.is_contiguous() or tuple(t.shape) != (max_steps, self.n_envs)):
                 raise TypeError(f"{name} must be a contiguous int32 tensor [max_steps, n_envs] on the env's device")
+        if obs_trace is not None and (not isinstance(obs_trace, torch.Tensor) or obs_trace.dtype != torch.int8
+                                      or obs_trace.device != self.device or not obs_trace.is_contiguous()
+                                      or tuple(obs_trace.shape) != (max_steps, self.n_envs, self.size)):
+            raise TypeError("obs_trace must be a contiguous int8 tensor [max_steps, n_envs, size] on the env's device")
         if until_fixed and actions is not None:
             raise ValueError("until_fixed cannot follow an action schedule: a fixed point is not defined under actions")
+        if until_fixed and obs_trace is not None:
+            raise ValueError("until_fixed cannot record an obs_trace: its rows would end at different steps per env")
         steps = torch.empty(self.n_envs, dtype=torch.int32, device=self.device)
         a = native.EnvRunArgs()
         a.world_in = a.world_out = self._wa.data_ptr()
@@ -313,7 +324,13 @@ class BatchedSim:
         a.alive_out = self._alive.data_ptr() if want_alive else None
         a.err_flag = self._err.data_ptr()
         with torch.cuda.device(self.device):
-            native.check(self._lib.cgl_env_run_ex(ctypes.byref(a), self._stream()), "cgl_env_run_ex")
+            if obs_trace is None:
+                native.check(self._lib.cgl_env_run_ex(ctypes.byref(a), self._stream()), "cgl_env_run_ex")
+            else:
+                o = native.EnvRunObsArgs(run=a, obs_trace=obs_trace.data_ptr() or None)
+                native.check(self._lib.cgl_env_run_obs(ctypes.byref(o), self._stream()), "cgl_env_run_obs")
+                if max_steps:
+                    self.stable = obs_trace[max_steps - 1]
         self.count += max_steps
         self.launches += 1
         return self.stable, self._reward, steps

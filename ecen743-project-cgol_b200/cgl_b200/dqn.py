@@ -49,7 +49,8 @@ class TrajectoryReplay:
     """Replay memory laid out as the trajectory of B lock-stepped environments (see the module docstring).
 
     `env` is a BatchedSim (or anything with n_envs, size, device, stable, bind_observation(buf),
-    step(actions, obs_out=, reward_out=) and reset()).  `max_size` counts transitions like the reference's
+    step(actions, obs_out=, reward_out=) and reset(); run() also needs run(k, actions=, reward_trace=, obs_trace=)).
+    `max_size` counts transitions like the reference's
     `max_size` (dqn.py:12); the ring has ceil(max_size / B) + 1 observation slots.
     """
 
@@ -117,6 +118,35 @@ class TrajectoryReplay:
         self.env.step(None if actions is None else act, obs_out=self._obs_v[n], reward_out=self._rew_v[s])
         self.t += 1
         return self._obs_v[n], self._rew_v[s]
+
+    def run(self, actions: torch.Tensor):
+        """k ring steps in on-chip env runs (`env.run(k, actions=, reward_trace=, obs_trace=)`): leaves the ring, `t`
+        and the env exactly as k calls of step(actions[i]) do.  actions: int32 [k, B] with 1 <= k <= slots - 1.
+        The observations go straight into their ring slots, in two runs where the slots wrap the ring end; the
+        rewards and actions, whose rows wrap one step earlier, through a [k, B] scratch and at most two copies each.
+        Returns (next_state, reward) of the last step = views of the ring."""
+        if not isinstance(actions, torch.Tensor) or actions.dim() != 2 or actions.shape[1] != self.B:
+            raise TypeError("actions must be an int32 tensor [k, n_envs]")
+        k = actions.shape[0]
+        if not 1 <= k <= self.slots - 1:
+            raise ValueError(f"k = {k} ring steps: 1 <= k <= slots - 1 = {self.slots - 1} are resident")
+        actions = actions.contiguous()
+        rew = torch.empty((k, self.B), dtype=torch.int32, device=self.device)
+        o = (self.t + 1) % self.slots                         # obs slot of step 0's next observation
+        k1 = min(k, self.slots - o)
+        self.env.run(k1, actions=actions[:k1], reward_trace=rew[:k1], obs_trace=self.obs[o:o + k1])
+        if k1 < k:
+            self.env.run(k - k1, actions=actions[k1:], reward_trace=rew[k1:], obs_trace=self.obs[:k - k1])
+        s = self.t % self.slots                               # action / reward slot of step 0
+        j = min(k, self.slots - s)
+        self.action[s:s + j].copy_(actions[:j])
+        self.reward[s:s + j].copy_(rew[:j])
+        if j < k:
+            self.action[:k - j].copy_(actions[j:])
+            self.reward[:k - j].copy_(rew[j:])
+        self.t += k
+        last = (self.t - 1) % self.slots
+        return self._obs_v[self.t % self.slots], self._rew_v[last]
 
     def reset(self) -> torch.Tensor:
         """env.reset() (main.py:59) into a fresh slot; the jump from the last observation of the old episode

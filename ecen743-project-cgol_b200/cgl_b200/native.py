@@ -93,7 +93,13 @@ class EnvRunArgs(ctypes.Structure):
                 ("alive_out", _vp), ("err_flag", _vp)]
 
 
+class EnvRunObsArgs(ctypes.Structure):
+    """cgl_env_run_obs_args_t (include/cgl_b200.h)."""
+    _fields_ = [("run", EnvRunArgs), ("obs_trace", _vp)]
+
+
 SIGNATURES["cgl_env_run_ex"] = (_i, [ctypes.POINTER(EnvRunArgs), _vp])
+SIGNATURES["cgl_env_run_obs"] = (_i, [ctypes.POINTER(EnvRunObsArgs), _vp])
 SIGNATURES["cgl_env_step_ex"] = (_i, [ctypes.POINTER(EnvStepArgs), _vp])
 SIGNATURES["cgl_env_step_seq"] = (_i, [ctypes.POINTER(EnvStepArgs), _u32, _u64, _u64, _vp])
 SIGNATURES["cgl_env_step_seq_timed"] = (_i, [ctypes.POINTER(EnvStepArgs), _u32, _u64, _u64, _vp, _vp, _vp])

@@ -17,8 +17,12 @@
 // surv) nibbles through the lane-private mask tables, byte-SIMD stability update.
 //
 // cgl_env_run_ex adds an action schedule (toggle_state before every step, as in cgl_env_step_rule) and per-step
-// reward / live-count traces to all three kernels, through their TR instantiations (DESIGN.md section 8 f3).
+// reward / live-count traces to all three kernels, through their TR instantiations (DESIGN.md section 8 f3.1).
+// cgl_env_run_obs adds the observation (the stability plane) after every step, through the OBS instantiations of the
+// byte and generic kernels (DESIGN.md section 8 f3.2).
 #include <stdlib.h>
+
+#include <utility>
 
 #include "cgl_internal.cuh"
 
@@ -99,12 +103,15 @@ struct RunTrace {
     int masked;
 };
 
-template <int S, bool TR>
+// OBS (implies TR): every updated 16-byte chunk of the stability plane is also stored to row (step, e) of `obs`
+// (int8 [max_steps][n_envs][SIZE]), and the plane is not written back: the run is out of place, the last row holds
+// the final plane.  `obs` is a kernel argument of its own because growing RunTrace reschedules the sliced kernels.
+template <int S, bool TR, bool OBS = false>
 __global__ void __launch_bounds__(RunCfg<S>::THREADS)
 env_run_kernel(const uint32_t *world_in, uint32_t *world_out, int8_t *stable, uint32_t n_envs,
                uint32_t max_steps, int stop_when_fixed, uint32_t spawn4, uint32_t max4,
                int32_t *__restrict__ steps_out, int32_t *__restrict__ reward_out, uint32_t *__restrict__ alive_out,
-               int rule, uint32_t min4, uint32_t empty4, RunTrace tr)
+               int rule, uint32_t min4, uint32_t empty4, RunTrace tr, int8_t *obs)
 {
     using C = RunCfg<S>;
     extern __shared__ __align__(16) unsigned char smem_dyn[];
@@ -166,6 +173,8 @@ env_run_kernel(const uint32_t *world_in, uint32_t *world_out, int8_t *stable, ui
         int act = -1;                                // TR: the cell toggled before this step, or -1
         int racc = 0;
         uint32_t pacc = 0;
+        uint4 *orow = nullptr;
+        if constexpr (OBS) orow = reinterpret_cast<uint4 *>(obs + ((size_t)steps * n_envs + e) * C::SIZE);
         if constexpr (TR) {
             const int a = next_act;
             if (tr.actions != nullptr && steps + 1 < max_steps) next_act = tr.actions[(size_t)(steps + 1) * n_envs + e];
@@ -243,6 +252,7 @@ env_run_kernel(const uint32_t *world_in, uint32_t *world_out, int8_t *stable, ui
                 if constexpr (TR) racc = __dp4a((int)s[k], 0x01010101, racc);
             }
             sst[c] = make_uint4(s[0], s[1], s[2], s[3]);
+            if constexpr (OBS) orow[c] = make_uint4(s[0], s[1], s[2], s[3]);     // (evict-first stores: no faster)
         }
         if (TR && want_trace) {
             racc = __reduce_add_sync(0xffffffffu, racc);
@@ -287,7 +297,7 @@ env_run_kernel(const uint32_t *world_in, uint32_t *world_out, int8_t *stable, ui
             const uint4 v = sst[j * C::TPE + t];
             acc = __dp4a((int)v.x, 0x01010101, acc); acc = __dp4a((int)v.y, 0x01010101, acc);
             acc = __dp4a((int)v.z, 0x01010101, acc); acc = __dp4a((int)v.w, 0x01010101, acc);
-            sp[j * C::TPE + t] = v;
+            if constexpr (!OBS) sp[j * C::TPE + t] = v;
         }
     }
     acc = __reduce_add_sync(0xffffffffu, acc);
@@ -563,13 +573,15 @@ env_run_sliced_kernel(const uint32_t *world_in, uint32_t *world_out, int8_t *sta
 
 // Any side whose three byte planes fit in 220 KiB of shared memory (side <= 274): one CTA per env, one byte per cell.
 // TR: thread 0 applies the step's toggle before a barrier; the per-step sums ride on the loop over the cells and are
-// stored by thread 0 after the step's vote.
-template <bool TR>
+// stored by thread 0 after the step's vote.  OBS (implies TR): every cell's new stability byte is also stored to row
+// (step, e) of `obs` (rows need not be 16-byte aligned), and the plane is not written back.
+template <bool TR, bool OBS = false>
 __global__ void __launch_bounds__(256)
 env_run_generic_kernel(const uint32_t *world_in, uint32_t *world_out, int8_t *stable, uint32_t side, uint32_t W,
                        uint32_t max_steps, int stop_when_fixed, int8_t spawn, int8_t stable_max,
                        int32_t *__restrict__ steps_out, int32_t *__restrict__ reward_out,
-                       uint32_t *__restrict__ alive_out, int rule, int8_t empty, int8_t empty_min, RunTrace tr)
+                       uint32_t *__restrict__ alive_out, int rule, int8_t empty, int8_t empty_min, RunTrace tr,
+                       int8_t *obs)
 {
     extern __shared__ __align__(16) unsigned char smem_dyn[];
     const uint32_t size = side * side;
@@ -595,6 +607,8 @@ env_run_generic_kernel(const uint32_t *world_in, uint32_t *world_out, int8_t *st
         int changed = 0;
         int racc = 0;
         uint32_t pacc = 0;
+        int8_t *orow = nullptr;
+        if constexpr (OBS) orow = obs + ((size_t)steps * gridDim.x + e) * size;
         if constexpr (TR) {
             if (tr.actions != nullptr) {
                 if (threadIdx.x == 0) {
@@ -621,6 +635,7 @@ env_run_generic_kernel(const uint32_t *world_in, uint32_t *world_out, int8_t *st
             b[i] = q;
             changed |= (p != q);
             st[i] = stable_update1_rule(rule, st[i], p != 0, q != 0, spawn, stable_max, empty, empty_min);
+            if constexpr (OBS) orow[i] = st[i];
             if constexpr (TR) { racc += st[i]; pacc += q; }
         }
         if constexpr (TR) {
@@ -648,7 +663,7 @@ env_run_generic_kernel(const uint32_t *world_in, uint32_t *world_out, int8_t *st
     int acc = 0;
     uint32_t pop = 0;
     for (uint32_t i = threadIdx.x; i < size; i += blockDim.x) {
-        sg[i] = st[i];
+        if constexpr (!OBS) sg[i] = st[i];
         acc += st[i];
     }
     for (uint32_t wdx = threadIdx.x; wdx < side * W; wdx += blockDim.x) {
@@ -686,12 +701,14 @@ static bool run_use_sliced(uint32_t max_steps)
     return max_steps >= 4;
 }
 
-template <int S, bool TR>
-static void launch_env_run_as(const cgl_env_run_args_t &a, const RunTrace &tr, cudaStream_t st)
+// OBS runs take the byte kernel at every step count: the bit-sliced kernel would need a planes -> bytes transpose
+// per 32 cells in every step to store the observation (DESIGN.md section 8 f3.2).
+template <int S, bool TR, bool OBS>
+static void launch_env_run_as(const cgl_env_run_args_t &a, const RunTrace &tr, int8_t *obs, cudaStream_t st)
 {
     using C = RunCfg<S>;
     const unsigned grid = (unsigned)((a.n_envs + C::EPC - 1) / C::EPC);
-    if (run_use_sliced(a.max_steps)) {
+    if (!OBS && run_use_sliced(a.max_steps)) {
         using D = SlicedCfg<S>;
         constexpr int smem = D::SMEM + (TR ? 16 : 0);             // TR: the step sums' slots
 #define CGL_RUN_SLICED(RULE)                                                                                          \
@@ -703,24 +720,27 @@ static void launch_env_run_as(const cgl_env_run_args_t &a, const RunTrace &tr, c
         else CGL_RUN_SLICED(CGL_DEAD_ZERO);
 #undef CGL_RUN_SLICED
     } else {
-        env_run_kernel<S, TR><<<grid, C::THREADS, C::SMEM + (TR ? 16 : 0), st>>>(
+        env_run_kernel<S, TR, OBS><<<grid, C::THREADS, C::SMEM + (TR ? 16 : 0), st>>>(
             a.world_in_dev, a.world_out_dev, a.stable_dev, (uint32_t)a.n_envs, a.max_steps, a.stop_when_fixed,
             rep4(a.spawn), rep4(a.stable_max), a.steps_out_dev, a.reward_out_dev, a.alive_out_dev, a.dead_rule,
-            rep4(a.empty_min), rep4(a.empty), tr);
+            rep4(a.empty_min), rep4(a.empty), tr, obs);
     }
 }
 
 template <int S>
-static int launch_env_run(const cgl_env_run_args_t &a, bool traced, const RunTrace &tr, cudaStream_t st)
+static int launch_env_run(const cgl_env_run_args_t &a, bool traced, const RunTrace &tr, int8_t *obs, cudaStream_t st)
 {
     using C = RunCfg<S>;
     static PerDeviceOnce once;
     if (once.first()) {
         CGL_CUDA(cudaFuncSetAttribute(env_run_kernel<S, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM));
         CGL_CUDA(cudaFuncSetAttribute(env_run_kernel<S, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM + 16));
+        CGL_CUDA(cudaFuncSetAttribute(env_run_kernel<S, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                      C::SMEM + 16));
     }
-    if (traced) launch_env_run_as<S, true>(a, tr, st);
-    else launch_env_run_as<S, false>(a, tr, st);
+    if (obs != nullptr) launch_env_run_as<S, true, true>(a, tr, obs, st);
+    else if (traced) launch_env_run_as<S, true, false>(a, tr, obs, st);
+    else launch_env_run_as<S, false, false>(a, tr, obs, st);
     CGL_LAUNCH_CHECK();
     return 0;
 }
@@ -749,11 +769,20 @@ breakdown_kernel(const int8_t *__restrict__ stable, uint64_t size, uint32_t *__r
 
 using namespace cgl;
 
-// The one implementation behind cgl_env_run and cgl_env_run_rule (see include/cgl_b200.h).
-extern "C" int cgl_env_run_ex(const cgl_env_run_args_t *args, cgl_stream_t stream)
+// Do the byte ranges [p, p + np) and [q, q + nq) share a byte?  (Lengths up to 2^96: no wrap-around.)
+static bool ranges_overlap(const void *p, unsigned __int128 np, const void *q, unsigned __int128 nq)
 {
-    CGL_REQUIRE(args, CGL_E_BADARG, "cgl_env_run_ex: null");
-    const cgl_env_run_args_t &a = *args;
+    if (p == nullptr || q == nullptr || np == 0 || nq == 0) return false;
+    const unsigned __int128 a = (uintptr_t)p, b = (uintptr_t)q;
+    return a < b + nq && b < a + np;
+}
+
+// The one implementation behind cgl_env_run_ex, cgl_env_run and cgl_env_run_rule (see include/cgl_b200.h).
+extern "C" int cgl_env_run_obs(const cgl_env_run_obs_args_t *args, cgl_stream_t stream)
+{
+    CGL_REQUIRE(args, CGL_E_BADARG, "cgl_env_run_obs: null");
+    const cgl_env_run_args_t &a = args->run;
+    int8_t *const obs = args->obs_trace_dev;
     CGL_REQUIRE(a.world_in_dev && a.world_out_dev && a.stable_dev && a.n_envs && a.side, CGL_E_BADARG,
                 "cgl_env_run: bad argument");
     CGL_REQUIRE(a.n_envs < (1ull << 31), CGL_E_BADARG, "cgl_env_run: n_envs too large");
@@ -768,12 +797,32 @@ extern "C" int cgl_env_run_ex(const cgl_env_run_args_t *args, cgl_stream_t strea
         for (int k = i + 1; k < 3; ++k)
             CGL_REQUIRE(bufs[i] == nullptr || bufs[i] != bufs[k], CGL_E_BADARG,
                         "cgl_env_run_ex: the action schedule and the traces must be separate buffers");
-    const bool traced = a.actions_dev || a.reward_trace_dev || a.alive_trace_dev;
+    if (obs != nullptr) {
+        CGL_REQUIRE(!a.stop_when_fixed, CGL_E_BADARG,
+                    "cgl_env_run_obs: stop_when_fixed cannot take an obs trace (its rows would end at different steps)");
+        CGL_REQUIRE(a.side <= 274, CGL_E_BADARG,
+                    "cgl_env_run: side must be a fused side or small enough for shared memory (side <= 274)");
+        const uint64_t size = (uint64_t)a.side * a.side;
+        const unsigned __int128 rows = (unsigned __int128)a.max_steps * a.n_envs;
+        const unsigned __int128 obs_bytes = rows * size;
+        const unsigned __int128 plane = (unsigned __int128)a.n_envs * size;
+        const unsigned __int128 world = (unsigned __int128)a.n_envs * a.side * cgl_words_per_row(a.side) * 4;
+        const std::pair<const void *, unsigned __int128> other[6] = {
+            {a.stable_dev, plane}, {a.actions_dev, rows * 4}, {a.reward_trace_dev, rows * 4},
+            {a.alive_trace_dev, rows * 4}, {a.world_in_dev, world}, {a.world_out_dev, world}};
+        for (const auto &o : other)
+            CGL_REQUIRE(!ranges_overlap(obs, obs_bytes, o.first, o.second), CGL_E_BADARG,
+                        "cgl_env_run_obs: the obs trace overlaps the stability plane, a world, the action schedule or a "
+                        "trace");
+        CGL_REQUIRE(!cgl_env_step_is_fused(a.side) || ((uintptr_t)obs & 15) == 0, CGL_E_BADARG,
+                    "cgl_env_run_obs: the obs trace must be 16-byte aligned on the fused sides");
+    }
+    const bool traced = a.actions_dev || a.reward_trace_dev || a.alive_trace_dev || obs;
     const RunTrace tr = {a.actions_dev, a.reward_trace_dev, a.alive_trace_dev, a.err_flag_dev, a.masked_toggle};
     cudaStream_t st = as_stream(stream);
     if (cgl_env_step_is_fused(a.side)) {
 #define CGL_CASE(S) \
-    case S: return launch_env_run<S>(a, traced, tr, st)
+    case S: return launch_env_run<S>(a, traced, tr, obs, st)
         switch (a.side) {
             CGL_CASE(32); CGL_CASE(64); CGL_CASE(96); CGL_CASE(128);
             CGL_CASE(160); CGL_CASE(192); CGL_CASE(224); CGL_CASE(256);
@@ -787,17 +836,27 @@ extern "C" int cgl_env_run_ex(const cgl_env_run_args_t *args, cgl_stream_t strea
     if (once.first()) {
         CGL_CUDA(cudaFuncSetAttribute(env_run_generic_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024));
         CGL_CUDA(cudaFuncSetAttribute(env_run_generic_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024));
+        CGL_CUDA(cudaFuncSetAttribute(env_run_generic_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                      220 * 1024));
     }
-#define CGL_RUN_GENERIC(TR)                                                                                            \
-    env_run_generic_kernel<TR><<<(unsigned)a.n_envs, 256, smem, st>>>(                                                 \
+#define CGL_RUN_GENERIC(TR, OBS)                                                                                       \
+    env_run_generic_kernel<TR, OBS><<<(unsigned)a.n_envs, 256, smem, st>>>(                                            \
         a.world_in_dev, a.world_out_dev, a.stable_dev, a.side, cgl_words_per_row(a.side), a.max_steps,                \
         a.stop_when_fixed, (int8_t)a.spawn, (int8_t)a.stable_max, a.steps_out_dev, a.reward_out_dev, a.alive_out_dev, \
-        a.dead_rule, (int8_t)a.empty, (int8_t)a.empty_min, tr)
-    if (traced) CGL_RUN_GENERIC(true);
-    else CGL_RUN_GENERIC(false);
+        a.dead_rule, (int8_t)a.empty, (int8_t)a.empty_min, tr, obs)
+    if (obs != nullptr) CGL_RUN_GENERIC(true, true);
+    else if (traced) CGL_RUN_GENERIC(true, false);
+    else CGL_RUN_GENERIC(false, false);
 #undef CGL_RUN_GENERIC
     CGL_LAUNCH_CHECK();
     return 0;
+}
+
+extern "C" int cgl_env_run_ex(const cgl_env_run_args_t *args, cgl_stream_t stream)
+{
+    CGL_REQUIRE(args, CGL_E_BADARG, "cgl_env_run_ex: null");
+    const cgl_env_run_obs_args_t o = {*args, nullptr};
+    return cgl_env_run_obs(&o, stream);
 }
 
 extern "C" int cgl_env_run_rule(const uint32_t *win, uint32_t *wout, int8_t *stable, uint64_t n_envs, uint32_t side,

@@ -8,6 +8,7 @@
 //   env_step       toggle + generation + int8 stability + reward for a batch          -> cgl_env_step_ex
 //   env_run        k plain steps / run-until-fixed in one launch                       -> cgl_env_run_rule
 //   env_run_ex     the same with an action schedule and per-step reward / alive traces -> cgl_env_run_ex
+//                  and, with obs_trace, the observation after every step               -> cgl_env_run_obs
 //   pack / unpack  uint8 cells <-> bit-packed world at the API boundary                -> cgl_pack / cgl_unpack
 //   reward / alive the reference's reductions (CGL/CGL.py:255-260)                     -> cgl_reward / cgl_alive
 //   life_run       world-only generations (life mode)                                  -> cgl_life_run
@@ -112,13 +113,15 @@ at::Tensor env_run(const at::Tensor &world, const at::Tensor &stable, int64_t si
 }
 
 // env_run with an action schedule (int32 [max_steps, n_envs]) and per-step traces (int32 [max_steps, n_envs], row t
-// = after step t), each optional; masked_toggle and err_flag (int32 [1]) as in env_step.  Returns steps per env.
+// = after step t), each optional; masked_toggle and err_flag (int32 [1]) as in env_step.  obs_trace (int8
+// [max_steps, n_envs, side*side]) receives the stability plane after every step; `stable` is then read only.
+// Returns steps per env.
 at::Tensor env_run_ex(const at::Tensor &world, const at::Tensor &stable, int64_t side, int64_t max_steps,
                       bool until_fixed, int64_t spawn, int64_t stable_max, int64_t dead_rule, int64_t empty,
                       int64_t empty_min, bool masked_toggle, const c10::optional<at::Tensor> &actions,
                       const c10::optional<at::Tensor> &reward_trace, const c10::optional<at::Tensor> &alive_trace,
                       const c10::optional<at::Tensor> &reward_out, const c10::optional<at::Tensor> &alive_out,
-                      const c10::optional<at::Tensor> &err_flag)
+                      const c10::optional<at::Tensor> &err_flag, const c10::optional<at::Tensor> &obs_trace)
 {
     check_cuda(world, at::kInt, "world");
     check_cuda(stable, at::kChar, "stable");
@@ -136,9 +139,17 @@ at::Tensor env_run_ex(const at::Tensor &world, const at::Tensor &stable, int64_t
     if (reward_out.has_value()) check_cuda(*reward_out, at::kInt, "reward_out");
     if (alive_out.has_value()) check_cuda(*alive_out, at::kInt, "alive_out");
     if (err_flag.has_value()) check_cuda(*err_flag, at::kInt, "err_flag");
+    if (obs_trace.has_value()) {
+        check_cuda(*obs_trace, at::kChar, "obs_trace");
+        TORCH_CHECK(obs_trace->dim() == 3 && obs_trace->size(0) == max_steps && obs_trace->size(1) == n &&
+                        obs_trace->size(2) == size,
+                    "obs_trace must be [max_steps, n_envs, side*side]");
+        TORCH_CHECK(obs_trace->device() == world.device(), "obs_trace must be on the world's device");
+    }
     c10::cuda::CUDAGuard guard(world.device());
     at::Tensor steps = at::empty({n}, world.options().dtype(at::kInt));
-    cgl_env_run_args_t a = {};
+    cgl_env_run_obs_args_t o = {};
+    cgl_env_run_args_t &a = o.run;
     a.world_in_dev = static_cast<const uint32_t *>(world.data_ptr());
     a.world_out_dev = static_cast<uint32_t *>(world.data_ptr());
     a.stable_dev = static_cast<int8_t *>(stable.data_ptr());
@@ -153,7 +164,9 @@ at::Tensor env_run_ex(const at::Tensor &world, const at::Tensor &stable, int64_t
     a.reward_out_dev = ptr<int32_t>(reward_out);
     a.alive_out_dev = ptr<uint32_t>(alive_out);
     a.err_flag_dev = ptr<int>(err_flag);
-    check_rc(cgl_env_run_ex(&a, stream_of(world)), "cgl_env_run_ex");
+    o.obs_trace_dev = ptr<int8_t>(obs_trace);
+    if (obs_trace.has_value()) check_rc(cgl_env_run_obs(&o, stream_of(world)), "cgl_env_run_obs");
+    else check_rc(cgl_env_run_ex(&a, stream_of(world)), "cgl_env_run_ex");
     return steps;
 }
 
@@ -267,7 +280,8 @@ PYBIND11_MODULE(TORCH_EXTENSION_NAME, m)
           py::arg("until_fixed") = false, py::arg("spawn") = -1, py::arg("stable_max") = 1, py::arg("dead_rule") = 0,
           py::arg("empty") = 0, py::arg("empty_min") = -128, py::arg("masked_toggle") = false,
           py::arg("actions") = py::none(), py::arg("reward_trace") = py::none(), py::arg("alive_trace") = py::none(),
-          py::arg("reward_out") = py::none(), py::arg("alive_out") = py::none(), py::arg("err_flag") = py::none());
+          py::arg("reward_out") = py::none(), py::arg("alive_out") = py::none(), py::arg("err_flag") = py::none(),
+          py::arg("obs_trace") = py::none());
     m.def("pack", &pack);
     m.def("unpack", &unpack);
     m.def("reward", &reward);

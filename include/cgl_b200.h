@@ -231,6 +231,24 @@ typedef struct cgl_env_run_args {
 } cgl_env_run_args_t;
 int cgl_env_run_ex(const cgl_env_run_args_t *args, cgl_stream_t stream);
 
+/* cgl_env_run_ex that also records the observation after every step.  cgl_env_run_ex is this call with
+ * obs_trace_dev == NULL.  With obs_trace_dev != NULL:
+ *   - after step t, obs_trace_dev[(t * n_envs + e) * side*side ...] holds env e's stability plane, bit-identical to
+ *     the plane cgl_env_step_rule leaves after the same actions (with or without a schedule or the other traces);
+ *   - the run is out of place, like cgl_env_step_io: with max_steps > 0, run.stable_dev is read and never written,
+ *     and the plane after the last step is row max_steps-1.  max_steps == 0 writes no row and leaves the plane as
+ *     it is.  world_out_dev, the reward / alive outputs and steps_out_dev behave as in cgl_env_run_ex;
+ *   - every side runs a one-byte-per-cell shared-memory kernel at every max_steps; CGL_RUN_IMPL does not apply;
+ *   - on the fused sides the trace must be 16-byte aligned; elsewhere any address works.
+ * Trace offsets are 64-bit.  Besides the errors of cgl_env_run_ex, these return CGL_E_BADARG before any device
+ * work: stop_when_fixed with a trace (rows would end at different steps per env), and a trace whose bytes overlap
+ * the stability plane, either world, the action schedule or either per-step trace. */
+typedef struct cgl_env_run_obs_args {
+    cgl_env_run_args_t run;           /* exactly as for cgl_env_run_ex */
+    int8_t *obs_trace_dev;            /* int8 [max_steps][n_envs][side*side] or NULL */
+} cgl_env_run_obs_args_t;
+int cgl_env_run_obs(const cgl_env_run_obs_args_t *args, cgl_stream_t stream);
+
 /* Value counts of the stability plane, the device form of breakdown_stable (CGL/CGL_action+/CGL.py:
  * 294-297, np.unique(..., return_counts=True)): hist_out_dev uint32 [n_envs][256],
  * hist[e][v + 128] = number of cells of env e whose stability equals v. */
