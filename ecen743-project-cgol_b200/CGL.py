@@ -503,6 +503,23 @@ class sim:
         self._changed()
         return n
 
+    def run_until_cycle(self, iters, max_period=2):
+        """`run(iters, until_fixed=True)` that also stops when the world repeats one of its last max_period
+        (1..8) worlds: after the first step t with world_t == world_{t-p}, p <= max_period, the world when the
+        call starts counting as world_0.  Returns (steps executed, p), p = 0 if no step in `iters` matched; a
+        spaceship reports 0 until it has crossed the torus.  `count` advances by the steps."""
+        self._flush()
+        self._wait()
+        with self._torch.cuda.device(self._dev):
+            period = self._torch.zeros(1, dtype=self._torch.int32, device=self._dev)
+            _, rew, steps = self._b.run(int(iters), max_period=int(max_period), period_out=period)
+            n, p = int(steps.item()), int(period.item())
+            self._res[0] = int(rew.item())
+        self.count += n
+        self._reward_valid, self._alive_valid = True, False
+        self._changed()
+        return n, p
+
     def breakdown_stable(self):
         """np.asarray((unique values, counts)) of the stability vector (CGL_action+/CGL.py:294-297)."""
         self._flush()

@@ -18,6 +18,7 @@ Beyond the single step (SURVEY.md section 8f):
   run(k, until_fixed=)          k plain steps / run-until-fixed in one launch, env resident on chip
   run(k, actions=, reward_trace=, alive_trace=)   k steps following an action schedule, every step's reward recorded
   run(k, ..., obs_trace=)       and every step's observation, written straight into a caller buffer (replay ring)
+  run(k, max_period=P)          run until each world repeats one of its last P worlds (its cycle length -> period_out)
   dead_rule=, empty=, empty_min=, masked_toggle=   the CGL_action+ fork's env
   breakdown_stable / breakdown_state, block_action, save_checkpoint / load_checkpoint, step_host(sync=False)
 """
@@ -278,7 +279,8 @@ class BatchedSim:
 
     def run(self, max_steps: int, until_fixed: bool = False, want_alive: bool = False,
             actions: torch.Tensor | None = None, reward_trace: torch.Tensor | None = None,
-            alive_trace: torch.Tensor | None = None, obs_trace: torch.Tensor | None = None):
+            alive_trace: torch.Tensor | None = None, obs_trace: torch.Tensor | None = None,
+            max_period: int = 0, period_out: torch.Tensor | None = None):
         """`max_steps` steps for every env in ONE launch, the environments resident in shared memory between
         steps (`cgl_env_run_ex`): the loop of CGL/bench.py:39-40.  With until_fixed an env stops after the
         first step that leaves its world unchanged -- the convergence loop of CGL_action+/validate.py:133-139
@@ -294,6 +296,10 @@ class BatchedSim:
         env's stability plane after step t (`cgl_env_run_obs`).  The run is then out of place like step(obs_out=):
         the current plane is left untouched and `self.stable` becomes the view obs_trace[max_steps - 1] (with
         max_steps == 0 nothing is written and `self.stable` stays).  until_fixed takes no obs_trace.
+        max_period (1..8, `cgl_env_run_cycle`): an env stops after the first step t whose world equals the world
+        p <= max_period steps earlier (the world when the call started counts as step 0); max_period=1 is
+        until_fixed.  period_out (caller-owned contiguous int32 [B] on the env's device, optional) receives that p,
+        or 0 for an env that ran all max_steps without a repeat.  It takes no until_fixed, actions or obs_trace.
         Returns (obs, reward, steps): steps = int32 [B] steps executed per env.  `count` advances by
         max_steps, the number of steps the batch was asked for."""
         if not isinstance(max_steps, int) or max_steps < 0:
@@ -310,6 +316,16 @@ class BatchedSim:
             raise ValueError("until_fixed cannot follow an action schedule: a fixed point is not defined under actions")
         if until_fixed and obs_trace is not None:
             raise ValueError("until_fixed cannot record an obs_trace: its rows would end at different steps per env")
+        if not isinstance(max_period, int) or not 0 <= max_period <= native.RUN_MAX_PERIOD:
+            raise ValueError(f"max_period must be an integer in 0..{native.RUN_MAX_PERIOD}")
+        if max_period and (until_fixed or actions is not None or obs_trace is not None):
+            raise ValueError("max_period replaces until_fixed and takes no actions or obs_trace")
+        if period_out is not None and (not isinstance(period_out, torch.Tensor) or period_out.dtype != torch.int32
+                                       or period_out.device != self.device or not period_out.is_contiguous()
+                                       or tuple(period_out.shape) != (self.n_envs,)):
+            raise TypeError("period_out must be a contiguous int32 tensor [n_envs] on the env's device")
+        if period_out is not None and not max_period:
+            raise ValueError("period_out needs max_period")
         steps = torch.empty(self.n_envs, dtype=torch.int32, device=self.device)
         a = native.EnvRunArgs()
         a.world_in = a.world_out = self._wa.data_ptr()
@@ -324,7 +340,11 @@ class BatchedSim:
         a.alive_out = self._alive.data_ptr() if want_alive else None
         a.err_flag = self._err.data_ptr()
         with torch.cuda.device(self.device):
-            if obs_trace is None:
+            if max_period:
+                native.check(self._lib.cgl_env_run_cycle(ctypes.byref(a), max_period,
+                                                         None if period_out is None else period_out.data_ptr(),
+                                                         self._stream()), "cgl_env_run_cycle")
+            elif obs_trace is None:
                 native.check(self._lib.cgl_env_run_ex(ctypes.byref(a), self._stream()), "cgl_env_run_ex")
             else:
                 o = native.EnvRunObsArgs(run=a, obs_trace=obs_trace.data_ptr() or None)

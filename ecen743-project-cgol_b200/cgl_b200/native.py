@@ -100,6 +100,8 @@ class EnvRunObsArgs(ctypes.Structure):
 
 SIGNATURES["cgl_env_run_ex"] = (_i, [ctypes.POINTER(EnvRunArgs), _vp])
 SIGNATURES["cgl_env_run_obs"] = (_i, [ctypes.POINTER(EnvRunObsArgs), _vp])
+SIGNATURES["cgl_env_run_cycle"] = (_i, [ctypes.POINTER(EnvRunArgs), _u32, _vp, _vp])
+RUN_MAX_PERIOD = 8                      # CGL_RUN_MAX_PERIOD
 SIGNATURES["cgl_env_step_ex"] = (_i, [ctypes.POINTER(EnvStepArgs), _vp])
 SIGNATURES["cgl_env_step_seq"] = (_i, [ctypes.POINTER(EnvStepArgs), _u32, _u64, _u64, _vp])
 SIGNATURES["cgl_env_step_seq_timed"] = (_i, [ctypes.POINTER(EnvStepArgs), _u32, _u64, _u64, _vp, _vp, _vp])

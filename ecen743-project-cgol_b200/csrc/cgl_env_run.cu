@@ -20,6 +20,8 @@
 // reward / live-count traces to all three kernels, through their TR instantiations (DESIGN.md section 8 f3.1).
 // cgl_env_run_obs adds the observation (the stability plane) after every step, through the OBS instantiations of the
 // byte and generic kernels (DESIGN.md section 8 f3.2).
+// cgl_env_run_cycle stops an env when its world repeats one of its last max_period worlds, through the CYC
+// instantiations of the bit-sliced and generic kernels (DESIGN.md section 8 f3.3).
 #include <stdlib.h>
 
 #include <utility>
@@ -318,6 +320,18 @@ env_run_kernel(const uint32_t *world_in, uint32_t *world_out, int8_t *stable, ui
     }
 }
 
+// CYC (cgl_env_run_cycle): world_j is kept in history slot j % P.  `differs` has bit s set when world_t differs from
+// slot s; the slots filled before step t are those of world_max(0, t-P) .. world_{t-1}.  Returns the lag p in
+// 1..min(P, t) at which world_t repeats, or 0.  At most one filled slot can match (include/cgl_b200.h).
+__device__ __forceinline__ uint32_t cycle_lag(uint32_t differs, uint32_t t, uint32_t P)
+{
+    const uint32_t filled = (1u << (t < P ? t : P)) - 1u;
+    const uint32_t hit = ~differs & filled;
+    if (hit == 0) return 0;
+    const uint32_t p = (t - (uint32_t)(__ffs(hit) - 1)) % P;
+    return p == 0 ? P : p;
+}
+
 // =========================================================================================
 // Bit-sliced variant for longer runs.  Everything a thread owns stays in REGISTERS for the whole call: its
 // rows of the world (bit plane) and their stability as 8 bit planes per 32 cells (cgl_bits.cuh).  The rule
@@ -351,12 +365,21 @@ struct SlicedCfg {
 // warp adds its sums to a shared slot of the step's parity; thread 0 stores step t's after the barrier of step t+1
 // (the one that publishes the sums) and clears the slot; the last step's values are the final reward and live count.
 // Several envs per CTA (one warp each): lane 0 stores every step's sums.
-template <int S, int RULE, bool TR>
+//
+// CYC (cgl_env_run_cycle, stop_when_fixed == 0, no actions): every thread keeps its own rows of the last max_period
+// worlds in a ring in shared memory (world_0 written at load time); no other thread reads them, so no barrier is
+// added.  Each new word is compared with every slot (one LOP3 per slot into a per-slot accumulator) before it
+// replaces the oldest.  The per-slot "differs" bits are OR-reduced over the warp; one env per CTA: warps atomicOr them
+// into a shared slot indexed by step & 3, read after the next step's barrier (the one that carries the vote) and
+// cleared two steps later, and the last step's slot is read after the final barrier.  Several envs per CTA: the warp
+// reduction is the whole env.
+template <int S, int RULE, bool TR, bool CYC = false>
 __global__ void __launch_bounds__(SlicedCfg<S>::THREADS)
 env_run_sliced_kernel(const uint32_t *world_in, uint32_t *world_out, int8_t *stable, uint32_t n_envs,
                       uint32_t max_steps, int stop_when_fixed, int spawn, int stable_max, int empty_min,
                       int32_t *__restrict__ steps_out, int32_t *__restrict__ reward_out,
-                      uint32_t *__restrict__ alive_out, int empty, RunTrace tr)
+                      uint32_t *__restrict__ alive_out, int empty, RunTrace tr, uint32_t max_period,
+                      int32_t *__restrict__ period_out)
 {
     constexpr bool DECAY = RULE == CGL_DEAD_DECAY, SAT = RULE == CGL_DEAD_SAT;
     using C = SlicedCfg<S>;
@@ -366,6 +389,9 @@ env_run_sliced_kernel(const uint32_t *world_in, uint32_t *world_out, int8_t *sta
     uint32_t *hbuf = reinterpret_cast<uint32_t *>(smem_dyn) + g * (4 * C::WPE);     // [buffer][plane][row][w]
     int *red = reinterpret_cast<int *>(smem_dyn + C::EPC * (4 * C::WPE * 4)) + g * 2;
     int *slot = reinterpret_cast<int *>(smem_dyn + C::EPC * (4 * C::WPE * 4)) + 2 * C::EPC;   // TR, EPC == 1
+    // CYC: [after the TR slots] 4 "differs" slots (EPC == 1) | ring [env][max_period][word (j, w)][thread]
+    unsigned *cyc = reinterpret_cast<unsigned *>(slot + 4);
+    uint32_t *ring = reinterpret_cast<uint32_t *>(cyc + 4) + g * max_period * C::WPE + t;
     const uint32_t e = blockIdx.x * C::EPC + g;
     const bool active = e < n_envs;
 
@@ -374,6 +400,8 @@ env_run_sliced_kernel(const uint32_t *world_in, uint32_t *world_out, int8_t *sta
     if (t == 0) { red[0] = 0; red[1] = 0; }
     if constexpr (TR && C::EPC == 1)
         if (t == 0) { slot[0] = 0; slot[1] = 0; slot[2] = 0; slot[3] = 0; }
+    if constexpr (CYC && C::EPC == 1)
+        if (t == 0) { cyc[0] = 0; cyc[1] = 0; cyc[2] = 0; cyc[3] = 0; }
     uint32_t odd = 0;                               // TR, base rule: live cells loaded with u > STABLE - SPAWN
     if (active) {
         const uint32_t *wp = world_in + (size_t)e * C::WPE;
@@ -381,6 +409,10 @@ env_run_sliced_kernel(const uint32_t *world_in, uint32_t *world_out, int8_t *sta
 #pragma unroll
         for (int j = 0; j < C::RPB; ++j) {
             lds_words<C::W>(wp + (t * C::RPB + j) * C::W, cw[j]);       // (plain loads: the helper is address-space agnostic)
+            if constexpr (CYC) {
+#pragma unroll
+                for (int w = 0; w < C::W; ++w) ring[(j * C::W + w) * C::TPE] = cw[j][w];       // world_0 -> slot 0
+            }
 #pragma unroll
             for (int w = 0; w < C::W; ++w) {
                 const uint4 a = sp[((t * C::RPB + j) * S + w * 32) / 16];
@@ -414,6 +446,7 @@ env_run_sliced_kernel(const uint32_t *world_in, uint32_t *world_out, int8_t *sta
     const int r_dn = r_last == S - 1 ? 0 : r_last + 1;
 
     uint32_t steps = 0, changed = 1u, buf = 0;
+    uint32_t period = 0, wslot = CYC ? 1u % max_period : 0u;        // CYC: the ring slot of the next world
     const bool want_trace = TR && (tr.reward != nullptr || tr.alive != nullptr);
     // The base rule's live cells hold u in [0, STABLE - SPAWN] (a toggle or a birth sets 0, survivors count up to it)
     // unless the loaded plane had others; u > 127 - SPAWN then needs SPAWN..MAX to wrap int8.
@@ -465,6 +498,13 @@ env_run_sliced_kernel(const uint32_t *world_in, uint32_t *world_out, int8_t *sta
             // one barrier: publishes the sums and votes on whether the PREVIOUS step changed the world
             const bool any_changed = env_vote(changed != 0);
             if (stop_when_fixed && !any_changed) break;
+            if constexpr (CYC && C::EPC == 1) {
+                if (steps > 0) {                    // the barrier above completed the previous step's "differs" bits
+                    period = cycle_lag(cyc[(steps - 1) & 3], steps, max_period);
+                    if (period != 0) break;
+                }
+                if (t == 0) cyc[(steps + 2) & 3] = 0;       // last read in the previous step, next written two on
+            }
             if constexpr (TR && C::EPC == 1) {
                 if (want_trace && t == 0 && steps > 0) {
                     int *sl = slot + 2 * ((steps - 1) & 1);
@@ -481,6 +521,7 @@ env_run_sliced_kernel(const uint32_t *world_in, uint32_t *world_out, int8_t *sta
             lds_words<C::W>(h0 + r_dn * C::W, dn0);
             lds_words<C::W>(h1 + r_dn * C::W, dn1);
             changed = 0;
+            uint32_t dacc[CGL_RUN_MAX_PERIOD] = {};         // CYC: OR of (new ^ slot s) over my words
 #pragma unroll
             for (int j = 0; j < C::RPB; ++j) {
 #pragma unroll
@@ -499,6 +540,13 @@ env_run_sliced_kernel(const uint32_t *world_in, uint32_t *world_out, int8_t *sta
                         racc += sliced_reward32(RULE, pl[j][w], n, spawn, wraps);
                         pacc += __popc(n);
                     }
+                    if constexpr (CYC) {
+                        uint32_t *rw = ring + (j * C::W + w) * C::TPE;
+#pragma unroll
+                        for (int s = 0; s < CGL_RUN_MAX_PERIOD; ++s)
+                            if (s < (int)max_period) dacc[s] |= n ^ rw[s * C::WPE];
+                        rw[wslot * C::WPE] = n;
+                    }
                     cw[j][w] = n;
                 }
             }
@@ -515,8 +563,20 @@ env_run_sliced_kernel(const uint32_t *world_in, uint32_t *world_out, int8_t *sta
                     }
                 }
             }
+            uint32_t differs = 0;
+            if constexpr (CYC) {
+#pragma unroll
+                for (int s = 0; s < CGL_RUN_MAX_PERIOD; ++s) differs |= (dacc[s] != 0 ? 1u : 0u) << s;
+                differs = __reduce_or_sync(0xffffffffu, differs);
+                if (C::EPC == 1 && (threadIdx.x & 31) == 0 && differs != 0) atomicOr(&cyc[steps & 3], differs);
+                wslot = wslot + 1 == max_period ? 0 : wslot + 1;
+            }
             ++steps;
             buf ^= 1u;                              // the next step writes the other buffer: no reader is overtaken
+            if constexpr (CYC && C::EPC > 1) {
+                period = cycle_lag(differs, steps, max_period);
+                if (period != 0) break;
+            }
         }
     }
 
@@ -557,11 +617,16 @@ env_run_sliced_kernel(const uint32_t *world_in, uint32_t *world_out, int8_t *sta
         __syncthreads();
         acc = red[0];
         pop = (uint32_t)red[1];
+        // a run that used its whole budget: the barrier above completed the last step's "differs" bits
+        if constexpr (CYC)
+            if (period == 0 && steps > 0) period = cycle_lag(cyc[(steps - 1) & 3], steps, max_period);
     }
     if (active && t == 0) {
         if (reward_out != nullptr) reward_out[e] = acc;
         if (alive_out != nullptr) alive_out[e] = pop;
         if (steps_out != nullptr) steps_out[e] = (int32_t)steps;
+        if constexpr (CYC)
+            if (period_out != nullptr) period_out[e] = (int32_t)period;
         if constexpr (TR && C::EPC == 1) {
             if (steps > 0) {                        // the last step: its sums are the final reward and live count
                 if (tr.reward != nullptr) tr.reward[(size_t)(steps - 1) * n_envs + e] = acc;
@@ -575,19 +640,26 @@ env_run_sliced_kernel(const uint32_t *world_in, uint32_t *world_out, int8_t *sta
 // TR: thread 0 applies the step's toggle before a barrier; the per-step sums ride on the loop over the cells and are
 // stored by thread 0 after the step's vote.  OBS (implies TR): every cell's new stability byte is also stored to row
 // (step, e) of `obs` (rows need not be 16-byte aligned), and the plane is not written back.
-template <bool TR, bool OBS = false>
+// CYC (cgl_env_run_cycle): the last max_period worlds are kept as flat bit vectors of ceil(size/32) words after the
+// three planes.  The cell loop runs over whole warps; each warp packs its 32 new cells with one ballot (i is
+// warp-contiguous; the bit order does not matter for equality) and its lane 0 compares the word with every slot and
+// stores it.  Lane 0s atomicOr their "differs" bits into a shared slot indexed by step & 3, read after the vote.
+template <bool TR, bool OBS = false, bool CYC = false>
 __global__ void __launch_bounds__(256)
 env_run_generic_kernel(const uint32_t *world_in, uint32_t *world_out, int8_t *stable, uint32_t side, uint32_t W,
                        uint32_t max_steps, int stop_when_fixed, int8_t spawn, int8_t stable_max,
                        int32_t *__restrict__ steps_out, int32_t *__restrict__ reward_out,
                        uint32_t *__restrict__ alive_out, int rule, int8_t empty, int8_t empty_min, RunTrace tr,
-                       int8_t *obs)
+                       int8_t *obs, uint32_t max_period, int32_t *__restrict__ period_out)
 {
     extern __shared__ __align__(16) unsigned char smem_dyn[];
     const uint32_t size = side * side;
     uint8_t *a = smem_dyn, *b = a + size;
     int8_t *st = reinterpret_cast<int8_t *>(b + size);
-    __shared__ int red[TR ? 6 : 2];                 // TR: red[2 + 2 * (step & 1)] = the step's (reward, alive)
+    const uint32_t nw = (size + 31) / 32;           // CYC: words per world in the history
+    uint32_t *hist = reinterpret_cast<uint32_t *>(smem_dyn + ((3 * size + 3) & ~3u));
+    __shared__ int red[(TR ? 6 : 2) + (CYC ? 4 : 0)];   // TR: red[2 + 2 * (step & 1)] = the step's (reward, alive)
+    unsigned *cyc = reinterpret_cast<unsigned *>(red + (TR ? 6 : 2));      // CYC: "differs" bits by step & 3
     const uint64_t e = blockIdx.x;
     const uint32_t *wi = world_in + e * side * W;
     uint32_t *wo = world_out + e * side * W;
@@ -595,13 +667,23 @@ env_run_generic_kernel(const uint32_t *world_in, uint32_t *world_out, int8_t *st
     if (threadIdx.x == 0) { red[0] = 0; red[1] = 0; }
     if constexpr (TR)
         if (threadIdx.x == 0) { red[2] = 0; red[3] = 0; red[4] = 0; red[5] = 0; }
+    if constexpr (CYC)
+        if (threadIdx.x == 0) { cyc[0] = 0; cyc[1] = 0; cyc[2] = 0; cyc[3] = 0; }
     for (uint32_t i = threadIdx.x; i < size; i += blockDim.x) {
         const uint32_t y = i / side, x = i - y * side;
         a[i] = (wi[y * W + (x >> 5)] >> (x & 31)) & 1u;
         st[i] = sg[i];
     }
     __syncthreads();
-    uint32_t steps = 0;
+    if constexpr (CYC) {                            // world_0 -> slot 0, in the bit order of the step's ballots
+        for (uint32_t w = threadIdx.x; w < nw; w += blockDim.x) {
+            uint32_t word = 0;
+            for (uint32_t j = 0; j < 32 && 32 * w + j < size; ++j) word |= (uint32_t)a[32 * w + j] << j;
+            hist[w] = word;
+        }
+        __syncthreads();
+    }
+    uint32_t steps = 0, period = 0, wslot = CYC ? 1u % max_period : 0u;
     bool done = max_steps == 0;
     while (!done) {
         int changed = 0;
@@ -624,20 +706,36 @@ env_run_generic_kernel(const uint32_t *world_in, uint32_t *world_out, int8_t *st
                 __syncthreads();
             }
         }
-        for (uint32_t i = threadIdx.x; i < size; i += blockDim.x) {
-            const uint32_t y = i / side, x = i - y * side;
-            const uint32_t yu = (y == 0 ? side : y) - 1, yd = (y + 1 == side) ? 0 : y + 1;
-            const uint32_t xl = (x == 0 ? side : x) - 1, xr = (x + 1 == side) ? 0 : x + 1;
-            const uint32_t n = a[yu * side + xl] + a[yu * side + x] + a[yu * side + xr] + a[y * side + xl] +
-                               a[y * side + xr] + a[yd * side + xl] + a[yd * side + x] + a[yd * side + xr];
-            const uint8_t p = a[i];
-            const uint8_t q = (n == 3u) || (n == 2u && p);
-            b[i] = q;
-            changed |= (p != q);
-            st[i] = stable_update1_rule(rule, st[i], p != 0, q != 0, spawn, stable_max, empty, empty_min);
-            if constexpr (OBS) orow[i] = st[i];
-            if constexpr (TR) { racc += st[i]; pacc += q; }
+        uint32_t differs = 0;                        // CYC, lane 0: bit s = a word of mine differs from slot s
+        const uint32_t lim = CYC ? nw * 32 : size;
+        for (uint32_t i = threadIdx.x; i < lim; i += blockDim.x) {
+            bool live = false;
+            if (!CYC || i < size) {
+                const uint32_t y = i / side, x = i - y * side;
+                const uint32_t yu = (y == 0 ? side : y) - 1, yd = (y + 1 == side) ? 0 : y + 1;
+                const uint32_t xl = (x == 0 ? side : x) - 1, xr = (x + 1 == side) ? 0 : x + 1;
+                const uint32_t n = a[yu * side + xl] + a[yu * side + x] + a[yu * side + xr] + a[y * side + xl] +
+                                   a[y * side + xr] + a[yd * side + xl] + a[yd * side + x] + a[yd * side + xr];
+                const uint8_t p = a[i];
+                const uint8_t q = (n == 3u) || (n == 2u && p);
+                b[i] = q;
+                changed |= (p != q);
+                st[i] = stable_update1_rule(rule, st[i], p != 0, q != 0, spawn, stable_max, empty, empty_min);
+                if constexpr (OBS) orow[i] = st[i];
+                if constexpr (TR) { racc += st[i]; pacc += q; }
+                live = q != 0;
+            }
+            if constexpr (CYC) {
+                const uint32_t word = __ballot_sync(0xffffffffu, live);
+                if ((threadIdx.x & 31) == 0) {
+                    uint32_t *hw = hist + (i >> 5);
+                    for (uint32_t s = 0; s < max_period; ++s) differs |= (hw[s * nw] != word ? 1u : 0u) << s;
+                    hw[wslot * nw] = word;
+                }
+            }
         }
+        if constexpr (CYC)
+            if ((threadIdx.x & 31) == 0 && differs != 0) atomicOr(&cyc[steps & 3], differs);
         if constexpr (TR) {
             racc = __reduce_add_sync(0xffffffffu, racc);
             pacc = __reduce_add_sync(0xffffffffu, pacc);
@@ -656,9 +754,15 @@ env_run_generic_kernel(const uint32_t *world_in, uint32_t *world_out, int8_t *st
                 sl[0] = 0; sl[1] = 0;
             }
         }
+        if constexpr (CYC) {
+            // the vote's barrier completed this step's bits; the slot two steps on was last read a step ago
+            period = cycle_lag(cyc[steps & 3], steps + 1, max_period);
+            if (threadIdx.x == 0) cyc[(steps + 2) & 3] = 0;
+            wslot = wslot + 1 == max_period ? 0 : wslot + 1;
+        }
         uint8_t *tmp = a; a = b; b = tmp;
         ++steps;
-        done = steps >= max_steps || (stop_when_fixed && !any_changed);
+        done = steps >= max_steps || (stop_when_fixed && !any_changed) || period != 0;
     }
     int acc = 0;
     uint32_t pop = 0;
@@ -684,6 +788,8 @@ env_run_generic_kernel(const uint32_t *world_in, uint32_t *world_out, int8_t *st
         if (reward_out != nullptr) reward_out[e] = red[0];
         if (alive_out != nullptr) alive_out[e] = (uint32_t)red[1];
         if (steps_out != nullptr) steps_out[e] = (int32_t)steps;
+        if constexpr (CYC)
+            if (period_out != nullptr) period_out[e] = (int32_t)period;
     }
 }
 
@@ -714,7 +820,7 @@ static void launch_env_run_as(const cgl_env_run_args_t &a, const RunTrace &tr, i
 #define CGL_RUN_SLICED(RULE)                                                                                          \
     env_run_sliced_kernel<S, RULE, TR><<<grid, D::THREADS, smem, st>>>(                                                \
         a.world_in_dev, a.world_out_dev, a.stable_dev, (uint32_t)a.n_envs, a.max_steps, a.stop_when_fixed, a.spawn,   \
-        a.stable_max, a.empty_min, a.steps_out_dev, a.reward_out_dev, a.alive_out_dev, a.empty, tr)
+        a.stable_max, a.empty_min, a.steps_out_dev, a.reward_out_dev, a.alive_out_dev, a.empty, tr, 0u, nullptr)
         if (a.dead_rule == CGL_DEAD_DECAY) CGL_RUN_SLICED(CGL_DEAD_DECAY);
         else if (a.dead_rule == CGL_DEAD_SAT) CGL_RUN_SLICED(CGL_DEAD_SAT);
         else CGL_RUN_SLICED(CGL_DEAD_ZERO);
@@ -743,6 +849,51 @@ static int launch_env_run(const cgl_env_run_args_t &a, bool traced, const RunTra
     else launch_env_run_as<S, false, false>(a, tr, obs, st);
     CGL_LAUNCH_CHECK();
     return 0;
+}
+
+// CYC runs take the bit-sliced kernel at every step count: the byte kernel has no CYC instantiation.
+template <int S, bool TR>
+static void launch_env_run_cycle_as(const cgl_env_run_args_t &a, const RunTrace &tr, uint32_t max_period,
+                                    int32_t *period_out, cudaStream_t st)
+{
+    using D = SlicedCfg<S>;
+    const unsigned grid = (unsigned)((a.n_envs + D::EPC - 1) / D::EPC);
+    const size_t smem = D::SMEM + 32 + (size_t)D::EPC * max_period * D::WPE * 4;     // TR slots, cyc slots, ring
+#define CGL_RUN_SLICED(RULE)                                                                                          \
+    env_run_sliced_kernel<S, RULE, TR, true><<<grid, D::THREADS, smem, st>>>(                                          \
+        a.world_in_dev, a.world_out_dev, a.stable_dev, (uint32_t)a.n_envs, a.max_steps, 0, a.spawn, a.stable_max,      \
+        a.empty_min, a.steps_out_dev, a.reward_out_dev, a.alive_out_dev, a.empty, tr, max_period, period_out)
+    if (a.dead_rule == CGL_DEAD_DECAY) CGL_RUN_SLICED(CGL_DEAD_DECAY);
+    else if (a.dead_rule == CGL_DEAD_SAT) CGL_RUN_SLICED(CGL_DEAD_SAT);
+    else CGL_RUN_SLICED(CGL_DEAD_ZERO);
+#undef CGL_RUN_SLICED
+}
+
+template <int S>
+static int launch_env_run_cycle(const cgl_env_run_args_t &a, bool traced, const RunTrace &tr, uint32_t max_period,
+                                int32_t *period_out, cudaStream_t st)
+{
+    using D = SlicedCfg<S>;
+    constexpr size_t smem_max = D::SMEM + 32 + (size_t)D::EPC * CGL_RUN_MAX_PERIOD * D::WPE * 4;
+    static PerDeviceOnce once;
+    if (smem_max > 48 * 1024 && once.first()) {       // 256^2 at max_period 8: 96 KB
+#define CGL_OPT_IN(RULE, TR) \
+    CGL_CUDA(cudaFuncSetAttribute(env_run_sliced_kernel<S, RULE, TR, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max))
+        CGL_OPT_IN(CGL_DEAD_ZERO, false); CGL_OPT_IN(CGL_DEAD_DECAY, false); CGL_OPT_IN(CGL_DEAD_SAT, false);
+        CGL_OPT_IN(CGL_DEAD_ZERO, true); CGL_OPT_IN(CGL_DEAD_DECAY, true); CGL_OPT_IN(CGL_DEAD_SAT, true);
+#undef CGL_OPT_IN
+    }
+    if (traced) launch_env_run_cycle_as<S, true>(a, tr, max_period, period_out, st);
+    else launch_env_run_cycle_as<S, false>(a, tr, max_period, period_out, st);
+    CGL_LAUNCH_CHECK();
+    return 0;
+}
+
+// Shared memory of the generic kernel: three byte planes, and for CYC runs max_period bit-vector worlds after them.
+static uint64_t generic_smem(uint32_t side, uint32_t max_period)
+{
+    const uint64_t size = (uint64_t)side * side;
+    return max_period == 0 ? 3 * size : ((3 * size + 3) & ~3ull) + (uint64_t)max_period * 4 * ((size + 31) / 32);
 }
 
 // Value counts of int8 planes: hist[e][v + 128] = #{i : stable[e][i] == v}.  One CTA per env; equal
@@ -777,12 +928,9 @@ static bool ranges_overlap(const void *p, unsigned __int128 np, const void *q, u
     return a < b + nq && b < a + np;
 }
 
-// The one implementation behind cgl_env_run_ex, cgl_env_run and cgl_env_run_rule (see include/cgl_b200.h).
-extern "C" int cgl_env_run_obs(const cgl_env_run_obs_args_t *args, cgl_stream_t stream)
+// The argument checks of cgl_env_run_obs (obs may be NULL) and cgl_env_run_cycle: 0 or CGL_E_BADARG.
+static int check_env_run_args(const cgl_env_run_args_t &a, const int8_t *obs)
 {
-    CGL_REQUIRE(args, CGL_E_BADARG, "cgl_env_run_obs: null");
-    const cgl_env_run_args_t &a = args->run;
-    int8_t *const obs = args->obs_trace_dev;
     CGL_REQUIRE(a.world_in_dev && a.world_out_dev && a.stable_dev && a.n_envs && a.side, CGL_E_BADARG,
                 "cgl_env_run: bad argument");
     CGL_REQUIRE(a.n_envs < (1ull << 31), CGL_E_BADARG, "cgl_env_run: n_envs too large");
@@ -817,6 +965,18 @@ extern "C" int cgl_env_run_obs(const cgl_env_run_obs_args_t *args, cgl_stream_t 
         CGL_REQUIRE(!cgl_env_step_is_fused(a.side) || ((uintptr_t)obs & 15) == 0, CGL_E_BADARG,
                     "cgl_env_run_obs: the obs trace must be 16-byte aligned on the fused sides");
     }
+    CGL_REQUIRE(cgl_env_step_is_fused(a.side) || generic_smem(a.side, 0) <= 220 * 1024, CGL_E_BADARG,
+                "cgl_env_run: side must be a fused side or small enough for shared memory (side <= 274)");
+    return 0;
+}
+
+// The one implementation behind cgl_env_run_ex, cgl_env_run and cgl_env_run_rule (see include/cgl_b200.h).
+extern "C" int cgl_env_run_obs(const cgl_env_run_obs_args_t *args, cgl_stream_t stream)
+{
+    CGL_REQUIRE(args, CGL_E_BADARG, "cgl_env_run_obs: null");
+    const cgl_env_run_args_t &a = args->run;
+    int8_t *const obs = args->obs_trace_dev;
+    if (const int rc = check_env_run_args(a, obs)) return rc;
     const bool traced = a.actions_dev || a.reward_trace_dev || a.alive_trace_dev || obs;
     const RunTrace tr = {a.actions_dev, a.reward_trace_dev, a.alive_trace_dev, a.err_flag_dev, a.masked_toggle};
     cudaStream_t st = as_stream(stream);
@@ -829,9 +989,7 @@ extern "C" int cgl_env_run_obs(const cgl_env_run_obs_args_t *args, cgl_stream_t 
         }
 #undef CGL_CASE
     }
-    const size_t smem = 3ull * a.side * a.side;
-    CGL_REQUIRE(smem <= 220 * 1024, CGL_E_BADARG,
-                "cgl_env_run: side must be a fused side or small enough for shared memory (side <= 274)");
+    const size_t smem = generic_smem(a.side, 0);
     static PerDeviceOnce once;                   // opt in to the largest size once per device
     if (once.first()) {
         CGL_CUDA(cudaFuncSetAttribute(env_run_generic_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024));
@@ -843,10 +1001,57 @@ extern "C" int cgl_env_run_obs(const cgl_env_run_obs_args_t *args, cgl_stream_t 
     env_run_generic_kernel<TR, OBS><<<(unsigned)a.n_envs, 256, smem, st>>>(                                            \
         a.world_in_dev, a.world_out_dev, a.stable_dev, a.side, cgl_words_per_row(a.side), a.max_steps,                \
         a.stop_when_fixed, (int8_t)a.spawn, (int8_t)a.stable_max, a.steps_out_dev, a.reward_out_dev, a.alive_out_dev, \
-        a.dead_rule, (int8_t)a.empty, (int8_t)a.empty_min, tr, obs)
+        a.dead_rule, (int8_t)a.empty, (int8_t)a.empty_min, tr, obs, 0u, nullptr)
     if (obs != nullptr) CGL_RUN_GENERIC(true, true);
     else if (traced) CGL_RUN_GENERIC(true, false);
     else CGL_RUN_GENERIC(false, false);
+#undef CGL_RUN_GENERIC
+    CGL_LAUNCH_CHECK();
+    return 0;
+}
+
+extern "C" int cgl_env_run_cycle(const cgl_env_run_args_t *args, uint32_t max_period, int32_t *period_out,
+                                 cgl_stream_t stream)
+{
+    CGL_REQUIRE(args, CGL_E_BADARG, "cgl_env_run_cycle: null");
+    const cgl_env_run_args_t &a = *args;
+    if (const int rc = check_env_run_args(a, nullptr)) return rc;
+    CGL_REQUIRE(!a.stop_when_fixed, CGL_E_BADARG, "cgl_env_run_cycle: stop_when_fixed must be 0 (max_period replaces it)");
+    CGL_REQUIRE(!a.actions_dev, CGL_E_BADARG,
+                "cgl_env_run_cycle: no action schedule (a cycle is not defined under actions)");
+    CGL_REQUIRE(max_period >= 1 && max_period <= CGL_RUN_MAX_PERIOD, CGL_E_BADARG,
+                "cgl_env_run_cycle: max_period must be in 1..%d", CGL_RUN_MAX_PERIOD);
+    const bool traced = a.reward_trace_dev || a.alive_trace_dev;
+    const RunTrace tr = {nullptr, a.reward_trace_dev, a.alive_trace_dev, a.err_flag_dev, a.masked_toggle};
+    cudaStream_t st = as_stream(stream);
+    if (cgl_env_step_is_fused(a.side)) {
+#define CGL_CASE(S) \
+    case S: return launch_env_run_cycle<S>(a, traced, tr, max_period, period_out, st)
+        switch (a.side) {
+            CGL_CASE(32); CGL_CASE(64); CGL_CASE(96); CGL_CASE(128);
+            CGL_CASE(160); CGL_CASE(192); CGL_CASE(224); CGL_CASE(256);
+        }
+#undef CGL_CASE
+    }
+    const uint64_t smem = generic_smem(a.side, max_period);
+    CGL_REQUIRE(smem <= 220 * 1024, CGL_E_BADARG,
+                "cgl_env_run_cycle: a side that is not fused needs 3*side^2 + max_period*4*ceil(side^2/32) bytes <= "
+                "220 KiB of shared memory (side <= 268 at max_period 1, <= 237 at 8); side %u at max_period %u needs %llu",
+                a.side, max_period, (unsigned long long)smem);
+    static PerDeviceOnce once;
+    if (once.first()) {
+        CGL_CUDA(cudaFuncSetAttribute(env_run_generic_kernel<false, false, true>,
+                                      cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024));
+        CGL_CUDA(cudaFuncSetAttribute(env_run_generic_kernel<true, false, true>,
+                                      cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024));
+    }
+#define CGL_RUN_GENERIC(TR)                                                                                            \
+    env_run_generic_kernel<TR, false, true><<<(unsigned)a.n_envs, 256, smem, st>>>(                                    \
+        a.world_in_dev, a.world_out_dev, a.stable_dev, a.side, cgl_words_per_row(a.side), a.max_steps, 0,             \
+        (int8_t)a.spawn, (int8_t)a.stable_max, a.steps_out_dev, a.reward_out_dev, a.alive_out_dev, a.dead_rule,        \
+        (int8_t)a.empty, (int8_t)a.empty_min, tr, nullptr, max_period, period_out)
+    if (traced) CGL_RUN_GENERIC(true);
+    else CGL_RUN_GENERIC(false);
 #undef CGL_RUN_GENERIC
     CGL_LAUNCH_CHECK();
     return 0;

@@ -249,6 +249,28 @@ typedef struct cgl_env_run_obs_args {
 } cgl_env_run_obs_args_t;
 int cgl_env_run_obs(const cgl_env_run_obs_args_t *args, cgl_stream_t stream);
 
+/* cgl_env_run_ex that stops each env when its world enters a cycle of period <= max_period, not only at a fixed
+ * point: an exact, world-only generalisation of stop_when_fixed.  Let world_0 be the world when the call starts and
+ * world_t the world after step t.  Env e stops after the first step t (1 <= t <= max_steps) such that
+ * world_t == world_{t-p} for some p with 1 <= p <= min(max_period, t):
+ *   steps_out_dev[e]  = that t, or max_steps if no step matches;
+ *   period_out_dev[e] = that p, or 0 if no step matches (a match at t == max_steps counts).  May be NULL.
+ * The p is unique and is the cycle's length: the env did not stop earlier, so world_0 .. world_{t-1} are pairwise
+ * distinct within any window of max_period steps, and two matching lags p < q would make world_{t-p} ==
+ * world_{t-q} a repeat at lag q - p found at step t - p.  The world, stability plane, reward, alive and trace rows
+ * are those after step steps_out_dev[e], exactly as stop_when_fixed leaves them; rows t >= steps_out_dev[e] are not
+ * written.  max_period == 1 equals stop_when_fixed == 1 in every output.  The stability plane keeps its own dead-cell
+ * rule and is not compared.  A spaceship's world repeats only after it has crossed the torus (a glider: 4*side
+ * steps), so it reports period 0.
+ * Fused sides run the bit-sliced kernel at every max_steps (CGL_RUN_IMPL does not apply); other sides need
+ * 3*side^2 (rounded up to 4) + max_period*4*ceil(side^2/32) bytes <= 220 KiB of shared memory (side <= 268 at
+ * max_period 1, <= 237 at 8).  Besides the errors of cgl_env_run_ex, these return CGL_E_BADARG before any device
+ * work: args->stop_when_fixed != 0 (max_period replaces it), an action schedule (a cycle is not defined under
+ * actions), max_period outside 1..CGL_RUN_MAX_PERIOD, and a non-fused side past that bound. */
+#define CGL_RUN_MAX_PERIOD 8
+int cgl_env_run_cycle(const cgl_env_run_args_t *args, uint32_t max_period, int32_t *period_out_dev,
+                      cgl_stream_t stream);
+
 /* Value counts of the stability plane, the device form of breakdown_stable (CGL/CGL_action+/CGL.py:
  * 294-297, np.unique(..., return_counts=True)): hist_out_dev uint32 [n_envs][256],
  * hist[e][v + 128] = number of cells of env e whose stability equals v. */
