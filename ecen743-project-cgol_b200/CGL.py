@@ -520,6 +520,15 @@ class sim:
         self._changed()
         return n, p
 
+    def action_rewards(self):
+        """np.int32[size + 1]: entry a is what `toggle_state(a); step(); reward()` would return from the current
+        state (CGL/main.py:66-71), entry `size` the no-op's.  Nothing is stepped or toggled; a deferred toggle and
+        deferred steps are applied first, as for any other observation of the state."""
+        self._flush()
+        b = self._b                                         # (stops a resident step server: the planes are current)
+        with self._torch.cuda.device(self._dev):
+            return b.action_rewards()[0].cpu().numpy()
+
     def breakdown_stable(self):
         """np.asarray((unique values, counts)) of the stability vector (CGL_action+/CGL.py:294-297)."""
         self._flush()

@@ -11,7 +11,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libcgl_b200.so")
-SOURCES = ["cgl_api.cu", "cgl_env.cu", "cgl_env_run.cu", "cgl_sim1.cu", "cgl_rollout.cu", "cgl_life.cu", "cgl_life_tb.cu"]
+SOURCES = ["cgl_api.cu", "cgl_env.cu", "cgl_env_run.cu", "cgl_env_lookahead.cu", "cgl_sim1.cu", "cgl_rollout.cu", "cgl_life.cu", "cgl_life_tb.cu"]
 HEADERS = ["cgl_bits.cuh", "cgl_internal.cuh", os.path.join("..", "..", "include", "cgl_b200.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "--use_fast_math", "-Xcompiler", "-fPIC", "-shared", "-cudart", "static"]

@@ -19,6 +19,7 @@ Beyond the single step (SURVEY.md section 8f):
   run(k, actions=, reward_trace=, alive_trace=)   k steps following an action schedule, every step's reward recorded
   run(k, ..., obs_trace=)       and every step's observation, written straight into a caller buffer (replay ring)
   run(k, max_period=P)          run until each world repeats one of its last P worlds (its cycle length -> period_out)
+  action_rewards() / greedy_actions()   every action's next-step reward, and the one-step greedy action, without stepping
   dead_rule=, empty=, empty_min=, masked_toggle=   the CGL_action+ fork's env
   breakdown_stable / breakdown_state, block_action, save_checkpoint / load_checkpoint, step_host(sync=False)
 """
@@ -354,6 +355,47 @@ class BatchedSim:
         self.count += max_steps
         self.launches += 1
         return self.stable, self._reward, steps
+
+    def _lookahead(self, rewards_out, best_action, best_reward) -> None:
+        a = native.EnvActionRewardsArgs()
+        a.world, a.stable, a.n_envs, a.side = self._wa.data_ptr(), self.stable.data_ptr(), self.n_envs, self.side
+        a.spawn, a.stable_max = self.spawn, self.stable_max
+        a.dead_rule, a.empty, a.empty_min = DEAD_RULES[self.dead_rule], self.empty, self.empty_min
+        a.masked_toggle = int(self.masked_toggle)
+        a.rewards_out = None if rewards_out is None else rewards_out.data_ptr()
+        a.best_action_out = None if best_action is None else best_action.data_ptr()
+        a.best_reward_out = None if best_reward is None else best_reward.data_ptr()
+        with torch.cuda.device(self.device):
+            native.check(self._lib.cgl_env_action_rewards(ctypes.byref(a), self._stream()), "cgl_env_action_rewards")
+        self.launches += 1 if self.fused else 3
+
+    def _int32_out(self, t, name, shape):
+        if t is None:
+            return torch.empty(shape, dtype=torch.int32, device=self.device)
+        if (not isinstance(t, torch.Tensor) or t.dtype != torch.int32 or t.device != self.device
+                or not t.is_contiguous() or tuple(t.shape) != shape):
+            raise TypeError(f"{name} must be a contiguous int32 tensor {list(shape)} on the env's device")
+        return t
+
+    def action_rewards(self, out: torch.Tensor | None = None) -> torch.Tensor:
+        """int32 [B, size + 1]: column a is the reward step(a) would return from the current state (toggle_state(a),
+        step(), reward(): CGL/main.py:66-71), column `size` the no-op's -- the exact gamma = 0 Q-values.  Nothing is
+        stepped: the planes, `count` and the cached step arguments are left as they are (`cgl_env_action_rewards`).
+        out: a caller-owned contiguous int32 [B, size + 1] tensor on the env's device to write into."""
+        out = self._int32_out(out, "out", (self.n_envs, self.size + 1))
+        self._lookahead(out, None, None)
+        return out
+
+    def greedy_actions(self, out: torch.Tensor | None = None, reward_out: torch.Tensor | None = None):
+        """The one-step greedy policy: (actions, rewards), int32 [B] each, actions[e] = the smallest action with the
+        largest next-step reward (action_rewards().argmax(1)) and rewards[e] that reward.  No map is written, so this
+        costs one read of the planes.  out / reward_out: caller-owned contiguous int32 [B] tensors on the env's device."""
+        out = self._int32_out(out, "out", (self.n_envs,))
+        reward_out = self._int32_out(reward_out, "reward_out", (self.n_envs,))
+        if out.data_ptr() == reward_out.data_ptr():
+            raise TypeError("out and reward_out must be separate tensors")
+        self._lookahead(None, out, reward_out)
+        return out, reward_out
 
     def breakdown_stable(self) -> torch.Tensor:
         """Value counts of every env's stability plane: int64 [B, 256], column v + 128 = number of cells

@@ -102,6 +102,17 @@ SIGNATURES["cgl_env_run_ex"] = (_i, [ctypes.POINTER(EnvRunArgs), _vp])
 SIGNATURES["cgl_env_run_obs"] = (_i, [ctypes.POINTER(EnvRunObsArgs), _vp])
 SIGNATURES["cgl_env_run_cycle"] = (_i, [ctypes.POINTER(EnvRunArgs), _u32, _vp, _vp])
 RUN_MAX_PERIOD = 8                      # CGL_RUN_MAX_PERIOD
+
+
+class EnvActionRewardsArgs(ctypes.Structure):
+    """cgl_env_action_rewards_args_t (include/cgl_b200.h)."""
+    _fields_ = [("world", _vp), ("stable", _vp), ("n_envs", _u64), ("side", _u32), ("spawn", ctypes.c_int32),
+                ("stable_max", ctypes.c_int32), ("dead_rule", ctypes.c_int32), ("empty", ctypes.c_int32),
+                ("empty_min", ctypes.c_int32), ("masked_toggle", ctypes.c_int32), ("rewards_out", _vp),
+                ("best_action_out", _vp), ("best_reward_out", _vp)]
+
+
+SIGNATURES["cgl_env_action_rewards"] = (_i, [ctypes.POINTER(EnvActionRewardsArgs), _vp])
 SIGNATURES["cgl_env_step_ex"] = (_i, [ctypes.POINTER(EnvStepArgs), _vp])
 SIGNATURES["cgl_env_step_seq"] = (_i, [ctypes.POINTER(EnvStepArgs), _u32, _u64, _u64, _vp])
 SIGNATURES["cgl_env_step_seq_timed"] = (_i, [ctypes.POINTER(EnvStepArgs), _u32, _u64, _u64, _vp, _vp, _vp])

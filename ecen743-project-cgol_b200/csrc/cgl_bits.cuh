@@ -200,6 +200,53 @@ CGL_HD int8_t stable_update1_rule(int rule, int8_t s, bool prev, bool next, int8
     return 0;
 }
 
+// ---- one-step lookahead: every action's next-step reward (cgl_env_lookahead.cu) -------------------------------------
+// A toggle at cell c changes only c's state and stability and, by the same +-1, the neighbour count of the 8 cells
+// around c (on a torus of side >= 3 those 9 cells are distinct).  So with the plain step's reward R_noop,
+//   R(c) = R_noop + h(c) + sum_{x in N8(c)} (c alive ? gm(x) : gp(x))        (mod 2^32)
+// where, for a cell with state `alive`, neighbour count n and stability s:
+//   plain  its stability after the plain step;
+//   gp/gm  how that changes if n becomes n + 1 / n - 1 (state and stability kept);
+//   h      its stability after the step if the cell itself is toggled first (state flipped, stability set by the
+//          toggle: SPAWN, or with the masked toggle 0 for a cell toggled to dead), minus plain.
+// Closed forms: with live = (alive ? s incremented unless MAX : SPAWN) the value a live-next cell gets and D the
+// dead-cell rule's value, the stability only moves where `next` changes, by +-(live - D):
+//   gp = +V at n == 2 - alive, -V at n == 3;   gm = +V at n == 4, -V at n == 3 - alive;   V = live - D.
+struct Look1 { int plain, gp, gm, h; };
+
+CGL_HD int8_t dead_value1(int rule, int8_t s, int8_t empty, int8_t empty_min)
+{
+    if (rule == CGL_DEAD_DECAY) return (s != empty_min) ? (int8_t)(s - 1) : s;
+    if (rule == CGL_DEAD_SAT) {
+        const int8_t t = (int8_t)(s + empty);
+        return t < empty_min ? t : empty_min;
+    }
+    return 0;
+}
+
+CGL_HD Look1 lookahead1_rule(int rule, int8_t s, bool alive, int n, int8_t spawn, int8_t stable_max, int8_t empty,
+                             int8_t empty_min, bool masked)
+{
+    const int8_t inc = (s != stable_max) ? (int8_t)(s + 1) : s;
+    const int d = dead_value1(rule, s, empty, empty_min);
+    const int live = alive ? (int)inc : (int)spawn;
+    const bool next = n == 3 || (n == 2 && alive);
+    const int v = live - d;
+    Look1 r;
+    r.plain = next ? live : d;
+    r.gp = n == 2 - (int)alive ? v : (n == 3 ? -v : 0);
+    r.gm = n == 4 ? v : (n == 3 - (int)alive ? -v : 0);
+    // the toggled cell: a dead cell becomes alive with SPAWN and survives at n = 2, 3; a live one becomes dead (SPAWN,
+    // or 0 with the masked toggle) and is born at n = 3
+    const int8_t put = (masked && alive) ? (int8_t)0 : spawn;
+    int t;
+    if (alive) t = n == 3 ? (int)spawn : (int)dead_value1(rule, put, empty, empty_min);
+    else t = (n == 2 || n == 3) ? (int)((put != stable_max) ? (int8_t)(put + 1) : put)
+                                : (int)dead_value1(rule, put, empty, empty_min);
+    r.h = t - r.plain;
+    return r;
+}
+
 // ---- bit-sliced int8 stability (32 cells per operation) -----------------------------------
 // For kernels that keep an env on chip for many steps the int8 plane is held as 8 bit planes per 32 cells
 // (plane b, bit j = bit b of cell j's byte): the rule then costs ~33 logic ops per 32 cells instead of ~100

@@ -10,6 +10,7 @@
 //   env_run_ex     the same with an action schedule and per-step reward / alive traces -> cgl_env_run_ex
 //                  and, with obs_trace, the observation after every step               -> cgl_env_run_obs
 //                  or, with max_period, until the world repeats one of its last P     -> cgl_env_run_cycle
+//   env_action_rewards  every action's next-step reward and the greedy action per env  -> cgl_env_action_rewards
 //   pack / unpack  uint8 cells <-> bit-packed world at the API boundary                -> cgl_pack / cgl_unpack
 //   reward / alive the reference's reductions (CGL/CGL.py:255-260)                     -> cgl_reward / cgl_alive
 //   life_run       world-only generations (life mode)                                  -> cgl_life_run
@@ -185,6 +186,43 @@ at::Tensor env_run_ex(const at::Tensor &world, const at::Tensor &stable, int64_t
     return steps;
 }
 
+// The reward every action would give (rewards_out int32 [n_envs, side*side + 1]) and / or the greedy action and its
+// reward (best_action_out, best_reward_out: int32 [n_envs]); at least one output.  world / stable are only read.
+void env_action_rewards(const at::Tensor &world, const at::Tensor &stable, int64_t side, int64_t spawn,
+                        int64_t stable_max, int64_t dead_rule, int64_t empty, int64_t empty_min, bool masked_toggle,
+                        const c10::optional<at::Tensor> &rewards_out, const c10::optional<at::Tensor> &best_action_out,
+                        const c10::optional<at::Tensor> &best_reward_out)
+{
+    check_cuda(world, at::kInt, "world");
+    check_cuda(stable, at::kChar, "stable");
+    const int64_t size = side * side, W = (side + 31) / 32;
+    TORCH_CHECK(side >= 1 && stable.numel() % size == 0 && stable.numel() > 0, "stable does not hold whole environments");
+    const int64_t n = stable.numel() / size;
+    TORCH_CHECK(world.numel() == n * side * W, "world does not match ", n, " environments of side ", side);
+    TORCH_CHECK(world.device() == stable.device(), "world and stable must be on the same device");
+    const std::pair<const c10::optional<at::Tensor> *, const char *> outs[3] = {
+        {&rewards_out, "rewards_out"}, {&best_action_out, "best_action_out"}, {&best_reward_out, "best_reward_out"}};
+    for (const auto &o : outs) {
+        if (!o.first->has_value()) continue;
+        check_cuda(**o.first, at::kInt, o.second);
+        TORCH_CHECK((*o.first)->device() == world.device(), o.second, " must be on the world's device");
+    }
+    if (rewards_out) TORCH_CHECK(rewards_out->numel() == n * (size + 1), "rewards_out must be [n_envs, side*side + 1]");
+    if (best_action_out) TORCH_CHECK(best_action_out->numel() == n, "one best action per env");
+    if (best_reward_out) TORCH_CHECK(best_reward_out->numel() == n, "one best reward per env");
+    c10::cuda::CUDAGuard guard(world.device());
+    cgl_env_action_rewards_args_t a = {};
+    a.world_dev = static_cast<const uint32_t *>(world.data_ptr());
+    a.stable_dev = static_cast<const int8_t *>(stable.data_ptr());
+    a.n_envs = (uint64_t)n; a.side = (uint32_t)side;
+    a.spawn = (int32_t)spawn; a.stable_max = (int32_t)stable_max; a.dead_rule = (int32_t)dead_rule;
+    a.empty = (int32_t)empty; a.empty_min = (int32_t)empty_min; a.masked_toggle = masked_toggle ? 1 : 0;
+    a.rewards_out_dev = ptr<int32_t>(rewards_out);
+    a.best_action_out_dev = ptr<int32_t>(best_action_out);
+    a.best_reward_out_dev = ptr<int32_t>(best_reward_out);
+    check_rc(cgl_env_action_rewards(&a, stream_of(world)), "cgl_env_action_rewards");
+}
+
 // uint8 cells [n_envs, rows*cols] (nonzero = alive) -> int32 [n_envs, rows, W] packed words.
 at::Tensor pack(const at::Tensor &cells, int64_t rows, int64_t cols)
 {
@@ -297,6 +335,10 @@ PYBIND11_MODULE(TORCH_EXTENSION_NAME, m)
           py::arg("actions") = py::none(), py::arg("reward_trace") = py::none(), py::arg("alive_trace") = py::none(),
           py::arg("reward_out") = py::none(), py::arg("alive_out") = py::none(), py::arg("err_flag") = py::none(),
           py::arg("obs_trace") = py::none(), py::arg("max_period") = 0, py::arg("period") = py::none());
+    m.def("env_action_rewards", &env_action_rewards, py::arg("world"), py::arg("stable"), py::arg("side"),
+          py::arg("spawn") = -1, py::arg("stable_max") = 1, py::arg("dead_rule") = 0, py::arg("empty") = 0,
+          py::arg("empty_min") = -128, py::arg("masked_toggle") = false, py::arg("rewards_out") = py::none(),
+          py::arg("best_action_out") = py::none(), py::arg("best_reward_out") = py::none());
     m.def("pack", &pack);
     m.def("unpack", &unpack);
     m.def("reward", &reward);

@@ -271,6 +271,33 @@ int cgl_env_run_obs(const cgl_env_run_obs_args_t *args, cgl_stream_t stream);
 int cgl_env_run_cycle(const cgl_env_run_args_t *args, uint32_t max_period, int32_t *period_out_dev,
                       cgl_stream_t stream);
 
+/* One-step lookahead: the reward of every action, and the greedy action per env, without stepping.
+ * For every env e and action a in 0 .. side*side, rewards_out_dev[e * (side*side + 1) + a] is the int32 reward that
+ * cgl_env_step_rule with actions[e] = a and the same constants would return from the current planes (toggle_state(a),
+ * step(), reward(): CGL/main.py:66-71); a = side*side is the no-op.  That covers the masked toggle, the three dead-cell
+ * rules, empty / empty_min, the int8 wrap of the counter and the int32 wrap of the sum.
+ *   best_action_out_dev[e]  the smallest a that attains the maximum (what torch.argmax of the row returns);
+ *   best_reward_out_dev[e]  that maximum.
+ * Each output may be NULL, but not all three; the map is not written unless it is asked for.  The planes are only read,
+ * and nothing else changes (no count, no token, no alarm word).  Every side up to 46340 (side*side + 1 must fit int32);
+ * map offsets are 64-bit.  A toggle at cell c changes only c and the neighbour count of its 8 neighbours, so on a torus
+ * of side >= 3 the map is the plain step's reward plus a 9-cell correction per action (DESIGN.md section 8 f5); sides 1
+ * and 2 are computed by definition.  Fused sides (multiples of 32 up to 256) run one kernel; other sides three small ones
+ * and a stream-ordered scratch allocation of 12 bytes per env.  CGL_E_BADARG before any device work for: a NULL struct
+ * or plane, all three outputs NULL, n_envs == 0 or >= 2^31, dead_rule / empty / empty_min / masked_toggle out of range
+ * (as cgl_env_run_ex checks them), and an output whose bytes overlap the world, the plane or another output. */
+typedef struct cgl_env_action_rewards_args {
+    const uint32_t *world_dev;        /* packed world [n_envs][side][W] */
+    const int8_t *stable_dev;         /* int8 [n_envs][side*side] */
+    uint64_t n_envs;
+    uint32_t side;
+    int32_t spawn, stable_max, dead_rule, empty, empty_min, masked_toggle;
+    int32_t *rewards_out_dev;         /* int32 [n_envs][side*side + 1] or NULL */
+    int32_t *best_action_out_dev;     /* int32 [n_envs] or NULL */
+    int32_t *best_reward_out_dev;     /* int32 [n_envs] or NULL */
+} cgl_env_action_rewards_args_t;
+int cgl_env_action_rewards(const cgl_env_action_rewards_args_t *args, cgl_stream_t stream);
+
 /* Value counts of the stability plane, the device form of breakdown_stable (CGL/CGL_action+/CGL.py:
  * 294-297, np.unique(..., return_counts=True)): hist_out_dev uint32 [n_envs][256],
  * hist[e][v + 128] = number of cells of env e whose stability equals v. */
