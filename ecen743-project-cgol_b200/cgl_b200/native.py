@@ -70,6 +70,10 @@ SIGNATURES = {
     "cgl_dev_alloc": (_i, [_u64, ctypes.POINTER(_vp)]),
     "cgl_dev_free": (_i, [_vp]),
     "cgl_dev_memset": (_i, [_vp, _i, _u64, _vp]),
+    "cgl_state_granularity": (ctypes.c_size_t, [_i]),
+    "cgl_state_alloc": (_vp, [ctypes.c_size_t, _i, _vp]),
+    "cgl_state_free": (None, [_vp, ctypes.c_size_t, _i, _vp]),
+    "cgl_state_compressed": (_i, [_vp]),
 }
 
 class EnvStepArgs(ctypes.Structure):
@@ -190,6 +194,28 @@ def ext():
             raise CglNativeError("_cgl_ext.so was built against another ABI version")
         _ext = mod
     return _ext
+
+
+_state_allocator = None
+_state_pools = {}
+
+
+def state_pool(device_index: int):
+    """The torch.cuda.MemPool of `device_index` over cgl_state_alloc / cgl_state_free (hardware-compressed device
+    memory, see include/cgl_b200.h), or None if the device offers no compression.  One pool per device, kept for the
+    life of the process."""
+    global _state_allocator
+    if device_index in _state_pools:
+        return _state_pools[device_index]
+    import torch
+    pool = None
+    if load().cgl_state_granularity(device_index):
+        if _state_allocator is None:
+            _state_allocator = torch.cuda.memory.CUDAPluggableAllocator(LIB_PATH, "cgl_state_alloc", "cgl_state_free")
+        with torch.cuda.device(device_index):
+            pool = torch.cuda.MemPool(_state_allocator.allocator())
+    _state_pools[device_index] = pool
+    return pool
 
 
 def check(rc: int, what: str = "") -> None:

@@ -1,6 +1,10 @@
 // cgl_api.cu -- error state, device queries, host-buffer entry points, IPC + halo helpers.
+#include <cuda.h>
 #include <stdarg.h>
 #include <string.h>
+
+#include <map>
+#include <mutex>
 
 #include "cgl_internal.cuh"
 
@@ -344,4 +348,191 @@ extern "C" int cgl_dev_free(void *dev_ptr)
 {
     CGL_CUDA(cudaFree(dev_ptr));
     return 0;
+}
+
+// ---- hardware-compressed device memory for the env state planes --------------------------------------------
+// cuMemCreate with CU_MEM_ALLOCATION_COMP_GENERIC: the L2 compresses lines on their way to DRAM and expands them on
+// the way back, so a stability plane that is mostly zero bytes moves fewer DRAM bytes per step while every kernel
+// sees ordinary memory.  The driver API is reached through cudaGetDriverEntryPoint: the library links cudart
+// statically and takes no libcuda dependency.
+namespace {
+struct DriverVmm {
+    decltype(&::cuDeviceGetAttribute) dev_attr = nullptr;
+    decltype(&::cuMemGetAllocationGranularity) granularity = nullptr;
+    decltype(&::cuMemCreate) create = nullptr;
+    decltype(&::cuMemGetAllocationPropertiesFromHandle) props = nullptr;
+    decltype(&::cuMemAddressReserve) reserve = nullptr;
+    decltype(&::cuMemMap) map = nullptr;
+    decltype(&::cuMemSetAccess) access = nullptr;
+    decltype(&::cuMemUnmap) unmap = nullptr;
+    decltype(&::cuMemRelease) release = nullptr;
+    decltype(&::cuMemAddressFree) address_free = nullptr;
+    bool ok = false;
+};
+
+template <class F> bool entry(const char *name, F &fn)
+{
+    void *p = nullptr;
+    cudaDriverEntryPointQueryResult q;
+    if (cudaGetDriverEntryPoint(name, &p, cudaEnableDefault, &q) != cudaSuccess || q != cudaDriverEntryPointSuccess ||
+        !p) {
+        cudaGetLastError();
+        return false;
+    }
+    fn = reinterpret_cast<F>(p);
+    return true;
+}
+
+const DriverVmm &vmm()
+{
+    static const DriverVmm d = [] {
+        DriverVmm v;
+        v.ok = entry("cuDeviceGetAttribute", v.dev_attr) && entry("cuMemGetAllocationGranularity", v.granularity) &&
+               entry("cuMemCreate", v.create) && entry("cuMemGetAllocationPropertiesFromHandle", v.props) &&
+               entry("cuMemAddressReserve", v.reserve) && entry("cuMemMap", v.map) &&
+               entry("cuMemSetAccess", v.access) && entry("cuMemUnmap", v.unmap) &&
+               entry("cuMemRelease", v.release) && entry("cuMemAddressFree", v.address_free);
+        return v;
+    }();
+    return d;
+}
+
+CUmemAllocationProp compressible_prop(int device)
+{
+    CUmemAllocationProp p = {};
+    p.type = CU_MEM_ALLOCATION_TYPE_PINNED;
+    p.location.type = CU_MEM_LOCATION_TYPE_DEVICE;
+    p.location.id = device;
+    p.allocFlags.compressionType = CU_MEM_ALLOCATION_COMP_GENERIC;
+    return p;
+}
+
+// Allocation granularity of compressible memory on `device`; 0 if the device (or driver) does not offer it.
+size_t compressible_granularity(int device)
+{
+    static size_t cached[64];
+    static bool known[64] = {};
+    if (device < 0 || device >= 64) return 0;
+    if (known[device]) return cached[device];
+    const DriverVmm &d = vmm();
+    int supported = 0;
+    size_t g = 0;
+    if (d.ok && d.dev_attr(&supported, CU_DEVICE_ATTRIBUTE_GENERIC_COMPRESSION_SUPPORTED, device) == CUDA_SUCCESS &&
+        supported) {
+        CUmemAllocationProp p = compressible_prop(device);
+        if (d.granularity(&g, &p, CU_MEM_ALLOC_GRANULARITY_RECOMMENDED) != CUDA_SUCCESS) g = 0;
+    }
+    cached[device] = g;
+    known[device] = true;
+    return g;
+}
+
+// Every live allocation of cgl_state_alloc by base address: its size, and the physical handle if it is compressed
+// (handle 0: the cudaMalloc fall-back).
+struct StateBlock {
+    size_t bytes;
+    CUmemGenericAllocationHandle handle;
+};
+std::mutex g_state_mu;
+std::map<uintptr_t, StateBlock> g_state_blocks;
+
+void *compressed_alloc(size_t bytes, int device, CUmemGenericAllocationHandle *handle_out)
+{
+    const DriverVmm &d = vmm();
+    const size_t g = compressible_granularity(device);
+    if (!g) return nullptr;
+    bytes = (bytes + g - 1) / g * g;
+    CUmemAllocationProp p = compressible_prop(device);
+    CUmemGenericAllocationHandle h = 0;
+    if (d.create(&h, bytes, &p, 0) != CUDA_SUCCESS) return nullptr;
+    CUmemAllocationProp got = {};
+    if (d.props(&got, h) != CUDA_SUCCESS || got.allocFlags.compressionType != CU_MEM_ALLOCATION_COMP_GENERIC) {
+        d.release(h);                              // not granted: the caller takes plain memory instead
+        return nullptr;
+    }
+    CUdeviceptr va = 0;
+    if (d.reserve(&va, bytes, g, 0, 0) != CUDA_SUCCESS) {
+        d.release(h);
+        return nullptr;
+    }
+    CUmemAccessDesc acc = {};
+    acc.location = p.location;
+    acc.flags = CU_MEM_ACCESS_FLAGS_PROT_READWRITE;
+    if (d.map(va, bytes, 0, h, 0) != CUDA_SUCCESS) {
+        d.address_free(va, bytes);
+        d.release(h);
+        return nullptr;
+    }
+    if (d.access(va, bytes, &acc, 1) != CUDA_SUCCESS) {
+        d.unmap(va, bytes);
+        d.address_free(va, bytes);
+        d.release(h);
+        return nullptr;
+    }
+    *handle_out = h;
+    return reinterpret_cast<void *>(va);
+}
+}  // namespace
+
+extern "C" size_t cgl_state_granularity(int device) { return compressible_granularity(device); }
+
+extern "C" void *cgl_state_alloc(size_t bytes, int device, cgl_stream_t)
+{
+    if (!bytes) return nullptr;
+    int cur = -1;
+    if (cudaGetDevice(&cur) != cudaSuccess) return nullptr;
+    if (cur != device && cudaSetDevice(device) != cudaSuccess) return nullptr;
+    CUmemGenericAllocationHandle h = 0;
+    void *p = compressed_alloc(bytes, device, &h);
+    if (p) {
+        const size_t g = compressible_granularity(device);
+        bytes = (bytes + g - 1) / g * g;
+    } else if (cudaMalloc(&p, bytes) != cudaSuccess) {
+        cudaGetLastError();
+        p = nullptr;
+    }
+    if (cur != device) cudaSetDevice(cur);
+    if (p) {
+        std::lock_guard<std::mutex> lock(g_state_mu);
+        g_state_blocks[reinterpret_cast<uintptr_t>(p)] = StateBlock{bytes, h};
+    }
+    return p;
+}
+
+extern "C" void cgl_state_free(void *ptr, size_t, int device, cgl_stream_t)
+{
+    if (!ptr) return;
+    StateBlock b;
+    {
+        std::lock_guard<std::mutex> lock(g_state_mu);
+        auto it = g_state_blocks.find(reinterpret_cast<uintptr_t>(ptr));
+        if (it == g_state_blocks.end()) return;
+        b = it->second;
+        g_state_blocks.erase(it);
+    }
+    int cur = -1;
+    cudaGetDevice(&cur);
+    if (cur != device) cudaSetDevice(device);
+    if (b.handle) {
+        // cudaFree waits for the device; an unmap does not promise to, so wait here before the range goes away
+        cudaDeviceSynchronize();
+        const DriverVmm &d = vmm();
+        const CUdeviceptr va = reinterpret_cast<CUdeviceptr>(ptr);
+        d.unmap(va, b.bytes);
+        d.release(b.handle);
+        d.address_free(va, b.bytes);
+    } else {
+        cudaFree(ptr);
+    }
+    if (cur != device && cur >= 0) cudaSetDevice(cur);
+}
+
+extern "C" int cgl_state_compressed(const void *ptr)
+{
+    const uintptr_t a = reinterpret_cast<uintptr_t>(ptr);
+    std::lock_guard<std::mutex> lock(g_state_mu);
+    auto it = g_state_blocks.upper_bound(a);
+    if (it == g_state_blocks.begin()) return 0;
+    --it;
+    return a < it->first + it->second.bytes && it->second.handle != 0;
 }

@@ -22,6 +22,7 @@
 #ifndef CGL_B200_H
 #define CGL_B200_H
 
+#include <stddef.h>
 #include <stdint.h>
 
 #ifdef __cplusplus
@@ -523,6 +524,18 @@ int cgl_halo_exchange(const uint32_t *top_src_dev, const uint32_t *bot_src_dev, 
 int cgl_dev_alloc(uint64_t bytes, void **dev_ptr_out);
 int cgl_dev_free(void *dev_ptr);
 int cgl_dev_memset(void *dev_ptr, int value, uint64_t bytes, cgl_stream_t stream);
+
+/* ---- hardware-compressed device memory for the env state planes ----------------------------------------------
+ * cgl_state_alloc / cgl_state_free have the signatures of torch.cuda.memory.CUDAPluggableAllocator.  An allocation
+ * is compressible device memory (cuMemCreate with CU_MEM_ALLOCATION_COMP_GENERIC, size rounded up to the granularity)
+ * when the device supports it and the driver grants it, plain cudaMalloc memory otherwise; either kind is freed by
+ * cgl_state_free, which waits for the device first.  Kernels see ordinary memory: only the DRAM traffic changes.
+ * cgl_state_granularity: the allocation granularity of compressible memory on `device`, 0 if there is none.
+ * cgl_state_compressed: 1 if `ptr` lies in a compressed allocation of cgl_state_alloc, else 0. */
+size_t cgl_state_granularity(int device);
+void *cgl_state_alloc(size_t bytes, int device, cgl_stream_t stream);
+void cgl_state_free(void *ptr, size_t bytes, int device, cgl_stream_t stream);
+int cgl_state_compressed(const void *ptr);
 
 #ifdef __cplusplus
 }
