@@ -520,6 +520,23 @@ class sim:
         self._changed()
         return n, p
 
+    def run_until_settled(self, iters):
+        """`run_until_cycle` without a bound on the period: stops after the first step t whose world equals any
+        earlier world, the world when the call starts counting as world_0.  Returns (steps executed, p): p is the
+        exact period of the cycle the world entered (a glider's is 4*side), 0 if no step in `iters` repeated a
+        world.  `count` advances by the steps."""
+        self._flush()
+        self._wait()
+        with self._torch.cuda.device(self._dev):
+            period = self._torch.zeros(1, dtype=self._torch.int32, device=self._dev)
+            _, rew, steps = self._b.run(int(iters), until_settled=True, period_out=period)
+            n, p = int(steps.item()), int(period.item())
+            self._res[0] = int(rew.item())
+        self.count += n
+        self._reward_valid, self._alive_valid = True, False
+        self._changed()
+        return n, p
+
     def action_rewards(self):
         """np.int32[size + 1]: entry a is what `toggle_state(a); step(); reward()` would return from the current
         state (CGL/main.py:66-71), entry `size` the no-op's.  Nothing is stepped or toggled; a deferred toggle and

@@ -19,6 +19,7 @@ Beyond the single step (SURVEY.md section 8f):
   run(k, actions=, reward_trace=, alive_trace=)   k steps following an action schedule, every step's reward recorded
   run(k, ..., obs_trace=)       and every step's observation, written straight into a caller buffer (replay ring)
   run(k, max_period=P)          run until each world repeats one of its last P worlds (its cycle length -> period_out)
+  run(k, until_settled=True)    run until each world repeats any earlier world (steps to settle, exact period)
   action_rewards() / greedy_actions()   every action's next-step reward, and the one-step greedy action, without stepping
   dead_rule=, empty=, empty_min=, masked_toggle=   the CGL_action+ fork's env
   breakdown_stable / breakdown_state, block_action, save_checkpoint / load_checkpoint, step_host(sync=False)
@@ -304,7 +305,7 @@ class BatchedSim:
     def run(self, max_steps: int, until_fixed: bool = False, want_alive: bool = False,
             actions: torch.Tensor | None = None, reward_trace: torch.Tensor | None = None,
             alive_trace: torch.Tensor | None = None, obs_trace: torch.Tensor | None = None,
-            max_period: int = 0, period_out: torch.Tensor | None = None):
+            max_period: int = 0, period_out: torch.Tensor | None = None, until_settled: bool = False):
         """`max_steps` steps for every env in ONE launch, the environments resident in shared memory between
         steps (`cgl_env_run_ex`): the loop of CGL/bench.py:39-40.  With until_fixed an env stops after the
         first step that leaves its world unchanged -- the convergence loop of CGL_action+/validate.py:133-139
@@ -324,6 +325,10 @@ class BatchedSim:
         p <= max_period steps earlier (the world when the call started counts as step 0); max_period=1 is
         until_fixed.  period_out (caller-owned contiguous int32 [B] on the env's device, optional) receives that p,
         or 0 for an env that ran all max_steps without a repeat.  It takes no until_fixed, actions or obs_trace.
+        until_settled (`cgl_env_run_settle`): max_period without a bound on p.  An env stops after the first step t
+        whose world equals any earlier one; p is then the exact period of the cycle it entered (a glider's is
+        4*side) and t = the steps to settle + p.  period_out receives p, or 0 for an env that did not repeat within
+        max_steps.  It takes no until_fixed, max_period, actions or obs_trace.
         Returns (obs, reward, steps): steps = int32 [B] steps executed per env.  `count` advances by
         max_steps, the number of steps the batch was asked for."""
         if not isinstance(max_steps, int) or max_steps < 0:
@@ -348,7 +353,9 @@ class BatchedSim:
                                        or period_out.device != self.device or not period_out.is_contiguous()
                                        or tuple(period_out.shape) != (self.n_envs,)):
             raise TypeError("period_out must be a contiguous int32 tensor [n_envs] on the env's device")
-        if period_out is not None and not max_period:
+        if until_settled and (until_fixed or max_period or actions is not None or obs_trace is not None):
+            raise ValueError("until_settled takes no until_fixed, max_period, actions or obs_trace")
+        if period_out is not None and not (max_period or until_settled):
             raise ValueError("period_out needs max_period")
         steps = torch.empty(self.n_envs, dtype=torch.int32, device=self.device)
         a = native.EnvRunArgs()
@@ -364,7 +371,11 @@ class BatchedSim:
         a.alive_out = self._alive.data_ptr() if want_alive else None
         a.err_flag = self._err.data_ptr()
         with torch.cuda.device(self.device):
-            if max_period:
+            if until_settled:
+                native.check(self._lib.cgl_env_run_settle(ctypes.byref(a),
+                                                          None if period_out is None else period_out.data_ptr(),
+                                                          self._stream()), "cgl_env_run_settle")
+            elif max_period:
                 native.check(self._lib.cgl_env_run_cycle(ctypes.byref(a), max_period,
                                                          None if period_out is None else period_out.data_ptr(),
                                                          self._stream()), "cgl_env_run_cycle")

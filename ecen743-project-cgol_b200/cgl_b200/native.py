@@ -106,6 +106,7 @@ SIGNATURES["cgl_env_run_ex"] = (_i, [ctypes.POINTER(EnvRunArgs), _vp])
 SIGNATURES["cgl_env_run_obs"] = (_i, [ctypes.POINTER(EnvRunObsArgs), _vp])
 SIGNATURES["cgl_env_run_cycle"] = (_i, [ctypes.POINTER(EnvRunArgs), _u32, _vp, _vp])
 RUN_MAX_PERIOD = 8                      # CGL_RUN_MAX_PERIOD
+SIGNATURES["cgl_env_run_settle"] = (_i, [ctypes.POINTER(EnvRunArgs), _vp, _vp])
 
 
 class EnvActionRewardsArgs(ctypes.Structure):

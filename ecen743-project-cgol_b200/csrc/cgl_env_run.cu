@@ -22,6 +22,8 @@
 // byte and generic kernels (DESIGN.md section 8 f3.2).
 // cgl_env_run_cycle stops an env when its world repeats one of its last max_period worlds, through the CYC
 // instantiations of the bit-sliced and generic kernels (DESIGN.md section 8 f3.3).
+// cgl_env_run_settle stops an env at its first repeated world of any period: world-only finder kernels give each env's
+// step count, which the SETTLE instantiations of the same two kernels then run (DESIGN.md section 8 f3.4).
 #include <stdlib.h>
 
 #include <utility>
@@ -373,7 +375,10 @@ struct SlicedCfg {
 // into a shared slot indexed by step & 3, read after the next step's barrier (the one that carries the vote) and
 // cleared two steps later, and the last step's slot is read after the final barrier.  Several envs per CTA: the warp
 // reduction is the whole env.
-template <int S, int RULE, bool TR, bool CYC = false>
+//
+// SETTLE (cgl_env_run_settle, phase C): env e runs steps_out[e] steps, as set by the settle finder, instead of max_steps.
+// One env per CTA: the bound is uniform over the CTA; several envs per CTA: each warp leaves at its own.
+template <int S, int RULE, bool TR, bool CYC = false, bool SETTLE = false>
 __global__ void __launch_bounds__(SlicedCfg<S>::THREADS)
 env_run_sliced_kernel(const uint32_t *world_in, uint32_t *world_out, int8_t *stable, uint32_t n_envs,
                       uint32_t max_steps, int stop_when_fixed, int spawn, int stable_max, int empty_min,
@@ -394,6 +399,8 @@ env_run_sliced_kernel(const uint32_t *world_in, uint32_t *world_out, int8_t *sta
     uint32_t *ring = reinterpret_cast<uint32_t *>(cyc + 4) + g * max_period * C::WPE + t;
     const uint32_t e = blockIdx.x * C::EPC + g;
     const bool active = e < n_envs;
+    if constexpr (SETTLE)
+        if (active) max_steps = (uint32_t)steps_out[e];
 
     uint32_t cw[C::RPB][C::W];                      // this thread's rows of the world
     uint32_t pl[C::RPB][C::W][8];                   // and their stability: 8 bit planes per word
@@ -644,7 +651,8 @@ env_run_sliced_kernel(const uint32_t *world_in, uint32_t *world_out, int8_t *sta
 // three planes.  The cell loop runs over whole warps; each warp packs its 32 new cells with one ballot (i is
 // warp-contiguous; the bit order does not matter for equality) and its lane 0 compares the word with every slot and
 // stores it.  Lane 0s atomicOr their "differs" bits into a shared slot indexed by step & 3, read after the vote.
-template <bool TR, bool OBS = false, bool CYC = false>
+// SETTLE (cgl_env_run_settle, phase C): the env runs steps_out[e] steps, as set by the settle finder, not max_steps.
+template <bool TR, bool OBS = false, bool CYC = false, bool SETTLE = false>
 __global__ void __launch_bounds__(256)
 env_run_generic_kernel(const uint32_t *world_in, uint32_t *world_out, int8_t *stable, uint32_t side, uint32_t W,
                        uint32_t max_steps, int stop_when_fixed, int8_t spawn, int8_t stable_max,
@@ -664,6 +672,7 @@ env_run_generic_kernel(const uint32_t *world_in, uint32_t *world_out, int8_t *st
     const uint32_t *wi = world_in + e * side * W;
     uint32_t *wo = world_out + e * side * W;
     int8_t *sg = stable + e * size;
+    if constexpr (SETTLE) max_steps = (uint32_t)steps_out[e];
     if (threadIdx.x == 0) { red[0] = 0; red[1] = 0; }
     if constexpr (TR)
         if (threadIdx.x == 0) { red[2] = 0; red[3] = 0; red[4] = 0; red[5] = 0; }
@@ -793,6 +802,244 @@ env_run_generic_kernel(const uint32_t *world_in, uint32_t *world_out, int8_t *st
     }
 }
 
+// =========================================================================================
+// cgl_env_run_settle, phases A and B: each env's first repeated world, of any period, from world-only generations.
+// A settle run takes no actions, so the world evolves without reference to the stability plane.  With M = max_steps:
+//   A: advance world_t and compare it with one checkpoint world_c, c the largest member of {0} u {2^k < M} u {M}
+//      below t.  The first match gives lambda = t - c: a match implies c >= mu, and the first match after c is at
+//      c + lambda.  No match by t = 2M means mu + lambda > M, since world_{M+lambda} == world_M would have matched.
+//   B: runners from world_0 and world_lambda in lockstep; the first equal pair is world_mu.  Given up once
+//      mu + lambda > M.
+// steps_out[e] = mu + lambda and period_out[e] = lambda, or (M, 0).  Phase C (the SETTLE instantiations above) then
+// runs exactly steps_out[e] full steps from the untouched inputs.  The counters are 64-bit: 2M passes 2^32.
+// =========================================================================================
+__device__ __forceinline__ bool settle_checkpoint(uint64_t t, uint64_t M)
+{
+    return t == M || (t < M && (t & (t - 1)) == 0);
+}
+
+// Fused sides: the bit-sliced kernel's layout and its one barrier per generation, without the stability planes.
+// Each thread holds its rows of the world and the checkpoint (phase A) or of both runners (phase B) in registers;
+// the barrier that publishes a generation's sums also carries the vote on the previous comparison.
+template <int S>
+__global__ void __launch_bounds__(SlicedCfg<S>::THREADS)
+env_settle_find_kernel(const uint32_t *world_in, uint32_t n_envs, uint32_t max_steps, int32_t *__restrict__ steps_out,
+                       int32_t *__restrict__ period_out)
+{
+    using C = SlicedCfg<S>;
+    extern __shared__ __align__(16) unsigned char smem_dyn[];
+    const int g = threadIdx.x / C::TPE;
+    const int t = threadIdx.x % C::TPE;
+    uint32_t *hbuf = reinterpret_cast<uint32_t *>(smem_dyn) + g * (4 * C::WPE);     // [buffer][plane][row][w]
+    const uint32_t e = blockIdx.x * C::EPC + g;
+    if (e >= n_envs) return;                        // a whole CTA (one env per CTA) or a whole warp (one per env)
+    const uint32_t *wp = world_in + (size_t)e * C::WPE;
+    const int r_first = t * C::RPB, r_last = t * C::RPB + C::RPB - 1;
+    const int r_up = r_first == 0 ? S - 1 : r_first - 1;
+    const int r_dn = r_last == S - 1 ? 0 : r_last + 1;
+    uint32_t buf = 0;
+
+    auto env_vote = [&](bool p) -> bool {
+        if constexpr (C::EPC == 1) return __syncthreads_or(p) != 0;
+        const bool r = __any_sync(0xffffffffu, p);
+        __syncwarp();
+        return r;
+    };
+    auto load = [&](uint32_t (&x)[C::RPB][C::W]) {
+#pragma unroll
+        for (int j = 0; j < C::RPB; ++j) lds_words<C::W>(wp + (t * C::RPB + j) * C::W, x[j]);
+    };
+    // One generation of x in two halves around the barrier: sums() publishes the edge rows' sums, next() reads the
+    // neighbours' sums and replaces x, calling visit(j, w, old word, new word) for every word.
+    auto sums = [&](const uint32_t (&x)[C::RPB][C::W], HSum (&hs)[C::RPB][C::W]) {
+        uint32_t *h0 = hbuf + buf * (2 * C::WPE), *h1 = h0 + C::WPE;
+#pragma unroll
+        for (int j = 0; j < C::RPB; ++j) {
+            uint32_t s0[C::W], s1[C::W];
+#pragma unroll
+            for (int w = 0; w < C::W; ++w) {
+                hs[j][w] = hsum(west_plane(x[j][(w + C::W - 1) % C::W], x[j][w]), x[j][w],
+                                east_plane(x[j][w], x[j][(w + 1) % C::W]));
+                s0[w] = hs[j][w].s0; s1[w] = hs[j][w].s1;
+            }
+            if (j == 0 || j == C::RPB - 1) {
+                sts_words<C::W>(h0 + (t * C::RPB + j) * C::W, s0);
+                sts_words<C::W>(h1 + (t * C::RPB + j) * C::W, s1);
+            }
+        }
+    };
+    auto next = [&](uint32_t (&x)[C::RPB][C::W], const HSum (&hs)[C::RPB][C::W], auto &&visit) {
+        const uint32_t *h0 = hbuf + buf * (2 * C::WPE), *h1 = h0 + C::WPE;
+        uint32_t up0[C::W], up1[C::W], dn0[C::W], dn1[C::W];
+        lds_words<C::W>(h0 + r_up * C::W, up0);
+        lds_words<C::W>(h1 + r_up * C::W, up1);
+        lds_words<C::W>(h0 + r_dn * C::W, dn0);
+        lds_words<C::W>(h1 + r_dn * C::W, dn1);
+#pragma unroll
+        for (int j = 0; j < C::RPB; ++j) {
+#pragma unroll
+            for (int w = 0; w < C::W; ++w) {
+                const HSum up = {j == 0 ? up0[w] : hs[j > 0 ? j - 1 : 0][w].s0,
+                                 j == 0 ? up1[w] : hs[j > 0 ? j - 1 : 0][w].s1, 0, 0};
+                const HSum dn = {j == C::RPB - 1 ? dn0[w] : hs[j < C::RPB - 1 ? j + 1 : 0][w].s0,
+                                 j == C::RPB - 1 ? dn1[w] : hs[j < C::RPB - 1 ? j + 1 : 0][w].s1, 0, 0};
+                const uint32_t n = life_rule(up, hs[j][w], dn, x[j][w]);
+                visit(j, w, x[j][w], n);
+                x[j][w] = n;
+            }
+        }
+        buf ^= 1u;                                  // the next generation writes the other buffer
+    };
+    auto nop = [](int, int, uint32_t, uint32_t) {};
+
+    // ---- phase A: lambda ------------------------------------------------------------------------------
+    const uint64_t M = max_steps;
+    uint32_t x[C::RPB][C::W], y[C::RPB][C::W];      // A: the world and the checkpoint; B: the two runners
+    load(x);
+    load(y);
+    uint64_t c = 0, lam = 0;
+    uint32_t diff = 0;                              // OR of world_i ^ world_c over my words
+    for (uint64_t i = 0;; ++i) {
+        HSum hs[C::RPB][C::W];
+        sums(x, hs);
+        const bool differs = env_vote(diff != 0);
+        if (i > 0 && !differs) { lam = i - c; break; }
+        if (i == 2 * M) break;
+        const bool keep = settle_checkpoint(i, M);  // world_i becomes the checkpoint
+        if (keep) c = i;
+        diff = 0;
+        next(x, hs, [&](int j, int w, uint32_t o, uint32_t n) {
+            if (keep) y[j][w] = o;
+            diff |= n ^ y[j][w];
+        });
+    }
+
+    // ---- phase B: mu ----------------------------------------------------------------------------------
+    uint64_t steps = M;
+    uint32_t period = 0;
+    if (lam != 0 && lam <= M) {
+        load(x);
+        load(y);
+        for (uint64_t i = 0; i < lam; ++i) {       // y = world_lambda
+            HSum hs[C::RPB][C::W];
+            sums(y, hs);
+            env_vote(false);
+            next(y, hs, nop);
+        }
+        diff = 0;
+#pragma unroll
+        for (int j = 0; j < C::RPB; ++j)
+#pragma unroll
+            for (int w = 0; w < C::W; ++w) diff |= x[j][w] ^ y[j][w];
+        for (uint64_t mu = 0;; ++mu) {             // x = world_mu, y = world_{mu + lambda}
+            HSum hs[C::RPB][C::W];
+            sums(x, hs);
+            if (!env_vote(diff != 0)) { steps = mu + lam; period = (uint32_t)lam; break; }
+            if (mu + lam == M) break;
+            next(x, hs, nop);
+            sums(y, hs);
+            env_vote(false);
+            diff = 0;
+            next(y, hs, [&](int j, int w, uint32_t, uint32_t n) { diff |= n ^ x[j][w]; });
+        }
+    }
+    if (t == 0) {
+        steps_out[e] = (int32_t)(uint32_t)steps;
+        if (period_out != nullptr) period_out[e] = (int32_t)period;
+    }
+}
+
+// Other sides: one CTA per env.  Worlds are flat bit vectors of ceil(side^2/32) words in shared memory (bit i = cell
+// i), four of them: phase A uses three (the world, the next one and the checkpoint, which is the world's own buffer
+// until the world moves on), phase B two per runner.  A generation packs each warp's 32 new cells with one ballot;
+// lane 0 stores the word and compares it with the reference world's, and one barrier carries the vote.
+__global__ void __launch_bounds__(256)
+env_settle_find_generic_kernel(const uint32_t *world_in, uint32_t side, uint32_t W, uint32_t max_steps,
+                               int32_t *__restrict__ steps_out, int32_t *__restrict__ period_out)
+{
+    extern __shared__ __align__(16) unsigned char smem_dyn[];
+    const uint32_t size = side * side, nw = (size + 31) / 32;
+    uint32_t *bits = reinterpret_cast<uint32_t *>(smem_dyn);
+    auto world = [&](int k) { return bits + k * nw; };
+    const uint32_t *wi = world_in + (uint64_t)blockIdx.x * side * W;
+    auto load = [&](uint32_t *dst) {
+        for (uint32_t w = threadIdx.x; w < nw; w += blockDim.x) {
+            uint32_t word = 0;
+            for (uint32_t j = 0; j < 32 && 32 * w + j < size; ++j) {
+                const uint32_t i = 32 * w + j, y = i / side, x = i - y * side;
+                word |= ((wi[y * W + (x >> 5)] >> (x & 31)) & 1u) << j;
+            }
+            dst[w] = word;
+        }
+    };
+    // src -> dst; returns whether any new word differs from ref's (ref may be NULL: no comparison)
+    auto gen = [&](const uint32_t *src, uint32_t *dst, const uint32_t *ref) -> bool {
+        auto cell = [&](uint32_t y, uint32_t x) { const uint32_t k = y * side + x; return (src[k >> 5] >> (k & 31)) & 1u; };
+        uint32_t d = 0;
+        for (uint32_t i = threadIdx.x; i < nw * 32; i += blockDim.x) {       // whole warps: nw * 32 cells
+            bool live = false;
+            if (i < size) {
+                const uint32_t y = i / side, x = i - y * side;
+                const uint32_t yu = (y == 0 ? side : y) - 1, yd = (y + 1 == side) ? 0 : y + 1;
+                const uint32_t xl = (x == 0 ? side : x) - 1, xr = (x + 1 == side) ? 0 : x + 1;
+                const uint32_t n = cell(yu, xl) + cell(yu, x) + cell(yu, xr) + cell(y, xl) + cell(y, xr) +
+                                   cell(yd, xl) + cell(yd, x) + cell(yd, xr);
+                live = n == 3u || (n == 2u && cell(y, x));
+            }
+            const uint32_t word = __ballot_sync(0xffffffffu, live);
+            if ((threadIdx.x & 31) == 0) {
+                dst[i >> 5] = word;
+                if (ref != nullptr) d |= word ^ ref[i >> 5];
+            }
+        }
+        return __syncthreads_or(d != 0) != 0;
+    };
+
+    // ---- phase A: lambda ------------------------------------------------------------------------------
+    const uint64_t M = max_steps;
+    load(world(0));
+    __syncthreads();
+    int cur = 0, ck = 0;
+    uint64_t c = 0, lam = 0;
+    for (uint64_t i = 0; i < 2 * M; ++i) {
+        if (settle_checkpoint(i, M)) { ck = cur; c = i; }
+        const int nxt = cur != ck ? 3 - cur - ck : (cur + 1) % 3;
+        const bool differs = gen(world(cur), world(nxt), world(ck));
+        cur = nxt;
+        if (!differs) { lam = i + 1 - c; break; }
+    }
+
+    // ---- phase B: mu ----------------------------------------------------------------------------------
+    uint64_t steps = M;
+    uint32_t period = 0;
+    if (lam != 0 && lam <= M) {
+        int x = 0, y = 2;                           // x in buffers 0 / 1, y in 2 / 3
+        load(world(x));
+        load(world(y));
+        __syncthreads();
+        for (uint64_t i = 0; i < lam; ++i) { gen(world(y), world(y ^ 1), nullptr); y ^= 1; }
+        uint32_t d = 0;
+        for (uint32_t w = threadIdx.x; w < nw; w += blockDim.x) d |= world(x)[w] ^ world(y)[w];
+        bool differs = __syncthreads_or(d != 0) != 0;
+        uint64_t mu = 0;
+        for (; differs && mu + lam < M; ++mu) {
+            gen(world(x), world(x ^ 1), nullptr); x ^= 1;
+            differs = gen(world(y), world(y ^ 1), world(x)); y ^= 1;
+        }
+        if (!differs) { steps = mu + lam; period = (uint32_t)lam; }
+    }
+    if (threadIdx.x == 0) {
+        steps_out[blockIdx.x] = (int32_t)(uint32_t)steps;
+        if (period_out != nullptr) period_out[blockIdx.x] = (int32_t)period;
+    }
+}
+
+// Shared memory of the generic settle finder: four bit-vector worlds.
+static uint64_t settle_find_smem(uint32_t side)
+{
+    return 4 * 4 * (((uint64_t)side * side + 31) / 32);
+}
+
 // CGL_RUN_IMPL=bytes | sliced forces one kernel (tests, tuning); default: sliced from 4 steps on
 // (measured on B200 at 4096 x 128^2: a launch costs ~50 us + 5.3 us per step sliced, ~25 us + 14 us per step bytes).
 static bool run_use_sliced(uint32_t max_steps)
@@ -894,6 +1141,64 @@ static uint64_t generic_smem(uint32_t side, uint32_t max_period)
 {
     const uint64_t size = (uint64_t)side * side;
     return max_period == 0 ? 3 * size : ((3 * size + 3) & ~3ull) + (uint64_t)max_period * 4 * ((size + 31) / 32);
+}
+
+// Settle runs on the fused sides: the finder, then phase C on the bit-sliced kernel at every step count (CGL_RUN_IMPL
+// does not apply).  Both kernels read the untouched inputs; only phase C writes.
+template <int S, bool TR>
+static void launch_env_run_settle_as(const cgl_env_run_args_t &a, const RunTrace &tr, cudaStream_t st)
+{
+    using D = SlicedCfg<S>;
+    const unsigned grid = (unsigned)((a.n_envs + D::EPC - 1) / D::EPC);
+    constexpr int smem = D::SMEM + (TR ? 16 : 0);                 // TR: the step sums' slots
+#define CGL_RUN_SLICED(RULE)                                                                                          \
+    env_run_sliced_kernel<S, RULE, TR, false, true><<<grid, D::THREADS, smem, st>>>(                                   \
+        a.world_in_dev, a.world_out_dev, a.stable_dev, (uint32_t)a.n_envs, a.max_steps, 0, a.spawn, a.stable_max,      \
+        a.empty_min, a.steps_out_dev, a.reward_out_dev, a.alive_out_dev, a.empty, tr, 0u, nullptr)
+    if (a.dead_rule == CGL_DEAD_DECAY) CGL_RUN_SLICED(CGL_DEAD_DECAY);
+    else if (a.dead_rule == CGL_DEAD_SAT) CGL_RUN_SLICED(CGL_DEAD_SAT);
+    else CGL_RUN_SLICED(CGL_DEAD_ZERO);
+#undef CGL_RUN_SLICED
+}
+
+template <int S>
+static int launch_env_run_settle(const cgl_env_run_args_t &a, bool traced, const RunTrace &tr, int32_t *period_out,
+                                 cudaStream_t st)
+{
+    using D = SlicedCfg<S>;
+    const unsigned grid = (unsigned)((a.n_envs + D::EPC - 1) / D::EPC);
+    env_settle_find_kernel<S><<<grid, D::THREADS, D::EPC * 4 * D::WPE * 4, st>>>(
+        a.world_in_dev, (uint32_t)a.n_envs, a.max_steps, a.steps_out_dev, period_out);
+    if (traced) launch_env_run_settle_as<S, true>(a, tr, st);
+    else launch_env_run_settle_as<S, false>(a, tr, st);
+    CGL_LAUNCH_CHECK();
+    return 0;
+}
+
+// Settle runs on the other sides: the generic finder, then phase C on the generic kernel.
+static int launch_env_run_settle_generic(const cgl_env_run_args_t &a, bool traced, const RunTrace &tr,
+                                         int32_t *period_out, cudaStream_t st)
+{
+    static PerDeviceOnce once;
+    if (once.first()) {
+        CGL_CUDA(cudaFuncSetAttribute(env_run_generic_kernel<false, false, false, true>,
+                                      cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024));
+        CGL_CUDA(cudaFuncSetAttribute(env_run_generic_kernel<true, false, false, true>,
+                                      cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024));
+    }
+    const uint32_t W = cgl_words_per_row(a.side);
+    env_settle_find_generic_kernel<<<(unsigned)a.n_envs, 256, settle_find_smem(a.side), st>>>(
+        a.world_in_dev, a.side, W, a.max_steps, a.steps_out_dev, period_out);
+#define CGL_RUN_GENERIC(TR)                                                                                            \
+    env_run_generic_kernel<TR, false, false, true><<<(unsigned)a.n_envs, 256, generic_smem(a.side, 0), st>>>(         \
+        a.world_in_dev, a.world_out_dev, a.stable_dev, a.side, W, a.max_steps, 0, (int8_t)a.spawn,                     \
+        (int8_t)a.stable_max, a.steps_out_dev, a.reward_out_dev, a.alive_out_dev, a.dead_rule, (int8_t)a.empty,        \
+        (int8_t)a.empty_min, tr, nullptr, 0u, nullptr)
+    if (traced) CGL_RUN_GENERIC(true);
+    else CGL_RUN_GENERIC(false);
+#undef CGL_RUN_GENERIC
+    CGL_LAUNCH_CHECK();
+    return 0;
 }
 
 // Value counts of int8 planes: hist[e][v + 128] = #{i : stable[e][i] == v}.  One CTA per env; equal
@@ -1055,6 +1360,41 @@ extern "C" int cgl_env_run_cycle(const cgl_env_run_args_t *args, uint32_t max_pe
 #undef CGL_RUN_GENERIC
     CGL_LAUNCH_CHECK();
     return 0;
+}
+
+extern "C" int cgl_env_run_settle(const cgl_env_run_args_t *args, int32_t *period_out, cgl_stream_t stream)
+{
+    CGL_REQUIRE(args, CGL_E_BADARG, "cgl_env_run_settle: null");
+    cgl_env_run_args_t a = *args;
+    // the side bound of check_env_run_args is the settle bound too: phase C needs 3*side^2 bytes of shared memory,
+    // the generic finder 16*ceil(side^2/32)
+    if (const int rc = check_env_run_args(a, nullptr)) return rc;
+    CGL_REQUIRE(!a.stop_when_fixed, CGL_E_BADARG,
+                "cgl_env_run_settle: stop_when_fixed must be 0 (the first repeat of any period replaces it)");
+    CGL_REQUIRE(!a.actions_dev, CGL_E_BADARG,
+                "cgl_env_run_settle: no action schedule (a cycle is not defined under actions)");
+    const bool traced = a.reward_trace_dev || a.alive_trace_dev;
+    const RunTrace tr = {nullptr, a.reward_trace_dev, a.alive_trace_dev, a.err_flag_dev, a.masked_toggle};
+    cudaStream_t st = as_stream(stream);
+    void *scratch = nullptr;                     // the per-env step counts hand phase C its bounds
+    if (a.steps_out_dev == nullptr) {
+        CGL_CUDA(cudaMallocAsync(&scratch, (size_t)a.n_envs * sizeof(int32_t), st));
+        a.steps_out_dev = static_cast<int32_t *>(scratch);
+    }
+    int rc = 0;
+    if (cgl_env_step_is_fused(a.side)) {
+#define CGL_CASE(S) \
+    case S: rc = launch_env_run_settle<S>(a, traced, tr, period_out, st); break
+        switch (a.side) {
+            CGL_CASE(32); CGL_CASE(64); CGL_CASE(96); CGL_CASE(128);
+            CGL_CASE(160); CGL_CASE(192); CGL_CASE(224); CGL_CASE(256);
+        }
+#undef CGL_CASE
+    } else {
+        rc = launch_env_run_settle_generic(a, traced, tr, period_out, st);
+    }
+    if (scratch != nullptr) CGL_CUDA(cudaFreeAsync(scratch, st));
+    return rc;
 }
 
 extern "C" int cgl_env_run_ex(const cgl_env_run_args_t *args, cgl_stream_t stream)

@@ -10,6 +10,7 @@
 //   env_run_ex     the same with an action schedule and per-step reward / alive traces -> cgl_env_run_ex
 //                  and, with obs_trace, the observation after every step               -> cgl_env_run_obs
 //                  or, with max_period, until the world repeats one of its last P     -> cgl_env_run_cycle
+//                  or, with until_settled, until the world repeats any earlier world   -> cgl_env_run_settle
 //   env_action_rewards  every action's next-step reward and the greedy action per env  -> cgl_env_action_rewards
 //   pack / unpack  uint8 cells <-> bit-packed world at the API boundary                -> cgl_pack / cgl_unpack
 //   reward / alive the reference's reductions (CGL/CGL.py:255-260)                     -> cgl_reward / cgl_alive
@@ -119,6 +120,8 @@ at::Tensor env_run(const at::Tensor &world, const at::Tensor &stable, int64_t si
 // [max_steps, n_envs, side*side]) receives the stability plane after every step; `stable` is then read only.
 // max_period (1..CGL_RUN_MAX_PERIOD) stops each env when its world repeats one of its last max_period worlds; period
 // (int32 [n_envs], optional) receives the cycle length or 0.  It takes no until_fixed, actions or obs_trace.
+// until_settled stops each env at its first repeated world of any period; period receives that period or 0.  It
+// takes no max_period, until_fixed, actions or obs_trace.
 // Returns steps per env.
 at::Tensor env_run_ex(const at::Tensor &world, const at::Tensor &stable, int64_t side, int64_t max_steps,
                       bool until_fixed, int64_t spawn, int64_t stable_max, int64_t dead_rule, int64_t empty,
@@ -126,7 +129,7 @@ at::Tensor env_run_ex(const at::Tensor &world, const at::Tensor &stable, int64_t
                       const c10::optional<at::Tensor> &reward_trace, const c10::optional<at::Tensor> &alive_trace,
                       const c10::optional<at::Tensor> &reward_out, const c10::optional<at::Tensor> &alive_out,
                       const c10::optional<at::Tensor> &err_flag, const c10::optional<at::Tensor> &obs_trace,
-                      int64_t max_period, const c10::optional<at::Tensor> &period)
+                      int64_t max_period, const c10::optional<at::Tensor> &period, bool until_settled)
 {
     check_cuda(world, at::kInt, "world");
     check_cuda(stable, at::kChar, "stable");
@@ -154,8 +157,10 @@ at::Tensor env_run_ex(const at::Tensor &world, const at::Tensor &stable, int64_t
     TORCH_CHECK(max_period >= 0 && max_period <= CGL_RUN_MAX_PERIOD, "max_period must be in 0..", CGL_RUN_MAX_PERIOD);
     TORCH_CHECK(max_period == 0 || (!until_fixed && !actions.has_value() && !obs_trace.has_value()),
                 "max_period replaces until_fixed and takes no actions or obs_trace");
+    TORCH_CHECK(!until_settled || (max_period == 0 && !until_fixed && !actions.has_value() && !obs_trace.has_value()),
+                "until_settled takes no max_period, until_fixed, actions or obs_trace");
     if (period.has_value()) {
-        TORCH_CHECK(max_period > 0, "period needs max_period");
+        TORCH_CHECK(max_period > 0 || until_settled, "period needs max_period or until_settled");
         check_cuda(*period, at::kInt, "period");
         TORCH_CHECK(period->numel() == n, "one period per env");
         TORCH_CHECK(period->device() == world.device(), "period must be on the world's device");
@@ -179,7 +184,9 @@ at::Tensor env_run_ex(const at::Tensor &world, const at::Tensor &stable, int64_t
     a.alive_out_dev = ptr<uint32_t>(alive_out);
     a.err_flag_dev = ptr<int>(err_flag);
     o.obs_trace_dev = ptr<int8_t>(obs_trace);
-    if (max_period > 0)
+    if (until_settled)
+        check_rc(cgl_env_run_settle(&a, ptr<int32_t>(period), stream_of(world)), "cgl_env_run_settle");
+    else if (max_period > 0)
         check_rc(cgl_env_run_cycle(&a, (uint32_t)max_period, ptr<int32_t>(period), stream_of(world)), "cgl_env_run_cycle");
     else if (obs_trace.has_value()) check_rc(cgl_env_run_obs(&o, stream_of(world)), "cgl_env_run_obs");
     else check_rc(cgl_env_run_ex(&a, stream_of(world)), "cgl_env_run_ex");
@@ -334,7 +341,8 @@ PYBIND11_MODULE(TORCH_EXTENSION_NAME, m)
           py::arg("empty") = 0, py::arg("empty_min") = -128, py::arg("masked_toggle") = false,
           py::arg("actions") = py::none(), py::arg("reward_trace") = py::none(), py::arg("alive_trace") = py::none(),
           py::arg("reward_out") = py::none(), py::arg("alive_out") = py::none(), py::arg("err_flag") = py::none(),
-          py::arg("obs_trace") = py::none(), py::arg("max_period") = 0, py::arg("period") = py::none());
+          py::arg("obs_trace") = py::none(), py::arg("max_period") = 0, py::arg("period") = py::none(),
+          py::arg("until_settled") = false);
     m.def("env_action_rewards", &env_action_rewards, py::arg("world"), py::arg("stable"), py::arg("side"),
           py::arg("spawn") = -1, py::arg("stable_max") = 1, py::arg("dead_rule") = 0, py::arg("empty") = 0,
           py::arg("empty_min") = -128, py::arg("masked_toggle") = false, py::arg("rewards_out") = py::none(),

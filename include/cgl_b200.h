@@ -272,6 +272,23 @@ int cgl_env_run_obs(const cgl_env_run_obs_args_t *args, cgl_stream_t stream);
 int cgl_env_run_cycle(const cgl_env_run_args_t *args, uint32_t max_period, int32_t *period_out_dev,
                       cgl_stream_t stream);
 
+/* cgl_env_run_cycle without a bound on the period: env e stops after the first step t (1 <= t <= max_steps) such
+ * that world_t == world_{t-p} for some p with 1 <= p <= t, with world_0 and world_t as there:
+ *   steps_out_dev[e]  = that t, or max_steps if no step matches (may be NULL);
+ *   period_out_dev[e] = that p, or 0 if no step matches (a match at t == max_steps counts).  May be NULL.
+ * The p is unique and is the minimal period lambda of the cycle the world enters, and t = mu + lambda, mu the first
+ * step whose world ever recurs.  So a glider reports 4*side once it has crossed the torus, a lightweight spaceship
+ * 2*side.  The world, stability plane, reward, alive and trace rows are those after step steps_out_dev[e], exactly as
+ * stop_when_fixed and cgl_env_run_cycle leave them; rows t >= steps_out_dev[e] are not written.  An env whose p is
+ * <= CGL_RUN_MAX_PERIOD gets the outputs of cgl_env_run_cycle(max_period = CGL_RUN_MAX_PERIOD) bit for bit.
+ * The run costs at most 2*max_steps world-only generations more than a plain run (DESIGN.md section 8 f3.4): world-
+ * only kernels find (t, p) per env from O(1) worlds, without hashing, and the run then executes exactly t full steps
+ * from the inputs.  Fused sides run the bit-sliced kernel at every max_steps (CGL_RUN_IMPL does not apply); other
+ * sides need 3*side^2 bytes <= 220 KiB of shared memory (side <= 274), as for cgl_env_run_ex.  Besides the errors of
+ * cgl_env_run_ex, these return CGL_E_BADARG before any device work: args->stop_when_fixed != 0 and an action schedule
+ * (a cycle is not defined under actions). */
+int cgl_env_run_settle(const cgl_env_run_args_t *args, int32_t *period_out_dev, cgl_stream_t stream);
+
 /* One-step lookahead: the reward of every action, and the greedy action per env, without stepping.
  * For every env e and action a in 0 .. side*side, rewards_out_dev[e * (side*side + 1) + a] is the int32 reward that
  * cgl_env_step_rule with actions[e] = a and the same constants would return from the current planes (toggle_state(a),
